@@ -1,6 +1,6 @@
 """Benchmark of the hot path (BASELINE.json: frames/sec end-to-end + uplift trajectories/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dtype tf32|bf16|fp32] [--legs ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dtype tf32|bf16|fp32] [--legs ...] [--dump-outputs DIR]
 
 A step = one pass of ball-detect + decode over one batch of 32 synthetic 1920x1080 three-frame stacks
 (BASELINE.json configs[1]): fused resize/normalise/stack -> WASB heatmap network -> argmax + sub-pixel decode.
@@ -48,6 +48,17 @@ CALIB_CLIPS = 64
 CLIP_FRAMES = 300          # BASELINE.json configs[2]: full hub pipeline on a synthetic 300-frame clip
 RALLY_FRAMES = 50          # ... processed as rallies of 50 frames (see the pipeline leg)
 WORKLOAD = 'configs[1]: WASB ball-detect (1280x704 input, 344 GFLOP/stack) + heatmap decode on synthetic 1920x1080 3-frame stacks, batch %d per GPU' % BATCH
+
+
+def dump_outputs(out_dir, pos, heat):
+    """Write what the last timed step returned, so that two builds can be compared output for output on identical seeded
+    inputs: the decoded (x, y, 1) of every stack (float64) and the heatmaps of every fourth stack (float32; all 32 would be
+    115 MB), with the indices of those stacks."""
+    os.makedirs(out_dir, exist_ok=True)
+    stacks = np.arange(0, heat.shape[0], 4)
+    np.save(os.path.join(out_dir, 'positions.npy'), pos.reshape(-1, 3).cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, 'heatmaps.npy'), heat[::4].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, 'heatmap_stacks.npy'), stacks.astype(np.float64))
 
 
 def peaks():
@@ -307,7 +318,13 @@ def main():
     ap.add_argument('--no-eager-baseline', action='store_true')
     ap.add_argument('--legs', default='all', help='comma list of the secondary legs to run: bf16,uplift,vitpose,pipeline,clips,calibration (default all)')
     ap.add_argument('--dump-profile', default='', help='write the per-kernel table of one profiled step to this JSON file')
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='write what the last timed step returned (positions, a fixed sample of the heatmaps) to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the CUDA path; the reference arm keeps none')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local = int(os.environ.get('LOCAL_RANK', 0))
@@ -413,12 +430,19 @@ def main():
             r['ms_copy'] = timed(lambda: det.predict(triples_copy, return_heatmaps=False), steps, warmup)
         return r
 
+    last_pos = [None]
+
+    def head_step():
+        last_pos[0] = step_device(args.dtype)
+
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    head = {'ms_dev': timed(lambda: step_device(args.dtype), args.steps, args.warmup)}
+    head = {'ms_dev': timed(head_step, args.steps, args.warmup)}
     head['launches'] = 1 + engine.last_launches() + 2
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:           # before anything else overwrites `heat`
+        dump_outputs(args.dump_outputs, gathered if world > 1 else last_pos[0], heat)
     head['ms_copy_hm'] = timed(lambda: det.predict(triples_copy), args.steps, args.warmup)
     head['ms_pinned'] = timed(lambda: det.predict(triples_pinned, return_heatmaps=False), args.steps, args.warmup)
     head['ms_view'] = timed(lambda: det.predict(triples_view, return_heatmaps=False), sub_steps, 2)
