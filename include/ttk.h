@@ -257,13 +257,30 @@ TTK_API int ttk_uplift_num_params(const ttk_uplift* h);
 TTK_API int ttk_uplift_param_info(const ttk_uplift* h, int i, char* name, int* numel);
 TTK_API int ttk_uplift_set_param(ttk_uplift* h, int i, const float* data_host, int numel);
 TTK_API size_t ttk_uplift_workspace_bytes(const ttk_uplift* h, int batch, int seq_len, int dtype);
-/* ball B x T x 2, table B x 13 x 3 (x, y, visibility), mask B x T in {0,1}, times B x T (s);
- * rot_out B x 3 (global axes), pos_out B x T x 3.  All float32 device pointers.
+/* ball B x T x 2, table B x 13 x 3 (x, y, visibility), mask B x T, times B x T (s);
+ * rot_out B x 3 (global axes), pos_out B x T x 3.  All float32 device pointers.  seq_len in [2, 63].
+ * mask_additive 0: mask in {0, 1} (0 = padding, never attended); 1: mask holds the additive values themselves ({-1e9, 0}), which
+ * the reference keeps as they are (model.py:541-546): a padded query row then attends uniformly over the valid keys.
  * The caller validates the mask (the reference raises ValueError on an all-ones mask). */
 TTK_API int ttk_uplift_forward(ttk_uplift* h, const float* ball_dev, const float* table_dev, const float* mask_dev,
-                       const float* times_dev, int batch, int seq_len, int dtype, float* rot_out_dev,
+                       const float* times_dev, int batch, int seq_len, int mask_additive, int dtype, float* rot_out_dev,
                        float* pos_out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+/* kernels launched by the last ttk_uplift_forward on this handle (0 when it failed its argument checks) */
 TTK_API int ttk_uplift_last_launches(const ttk_uplift* h);
+/* Test hooks: the two kernels of the tf32x3 path on caller buffers.
+ * GEMM (one-to-one with the library's Gemm3Args): c[m][n] = act(A' W^T + bias) (+ res), K = 128, n a multiple of 128, W = w_hi + w_lo
+ * with w_hi = tf32(W) rounded to nearest, ties away; A' = LayerNorm(a) with the given float32 (mean, rstd) rows, gamma and beta when
+ * ln_stats is not NULL; res may alias c; out_stats [m][2] receives mean / rstd (eps 1e-5) of c's rows (n = 128 only, else
+ * TTK_ERR_UNSUPPORTED).
+ * Attention: mode 0 table-token stage (batch * seq_len sequences of 14 rows; first_only: only token 0 is a query and o has one row per
+ * sequence), 1 temporal stage (batch sequences of seq_len rows), 2 second stage (batch sequences of seq_len + 1 rows, token 0 the cls
+ * token); qkv [rows][384] with bias, o [rows][128]; table, mask, times, mask_additive as for ttk_uplift_forward; inv_freq [16]. */
+TTK_API int ttk_uplift_debug_gemm3(const float* a_dev, const float* w_hi_dev, const float* w_lo_dev, const float* bias_dev,
+                           const float* res_dev, float* c_dev, int m, int n, int relu, const float* ln_stats_dev,
+                           const float* ln_gamma_dev, const float* ln_beta_dev, float* out_stats_dev, void* stream);
+TTK_API int ttk_uplift_debug_attention3(int mode, int first_only, const float* qkv_dev, float* o_dev, const float* table_dev,
+                                const float* mask_dev, const float* times_dev, const float* inv_freq_dev, int batch, int seq_len,
+                                int mask_additive, void* stream);
 
 /* Spin global -> local axes.  Replaces transform_rotationaxes (uplifting/helper.py:394-420).
  * rot B x 3, pos B x T x 3 -> out B x 3, float32. */

@@ -74,8 +74,10 @@ def _load():
         'ttk_uplift_param_info': (i32, [vp, i32, C.c_char_p, C.POINTER(i32)]),
         'ttk_uplift_set_param': (i32, [vp, i32, vp, i32]),
         'ttk_uplift_workspace_bytes': (sz, [vp, i32, i32, i32]),
-        'ttk_uplift_forward': (i32, [vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, sz, vp]),
+        'ttk_uplift_forward': (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, sz, vp]),
         'ttk_uplift_last_launches': (i32, [vp]),
+        'ttk_uplift_debug_gemm3': (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp]),
+        'ttk_uplift_debug_attention3': (i32, [i32, i32, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]),
         'ttk_rotation_local': (i32, [vp, vp, i32, i32, vp, vp]),
         'ttk_project': (i32, [vp, vp, vp, i32, i32, vp, vp]),
     }

@@ -220,7 +220,10 @@ __global__ void __launch_bounds__(THREADS, 1) gemm3_umma_kernel(const __grid_con
       fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);  // the accumulator is in registers: the MMA warp may overwrite it
-      float mean = 0.f, m2 = 0.f;                        // mean / sum of squared deviations of this thread's 64 columns (Chan merge of two 32-wide chunks)
+      // mean / sum of squared deviations of this thread's 64 columns (Chan merge of two 32-wide chunks), taken about `shift` (the first
+      // value): chunk means of rows with a large mean and a small spread would otherwise carry the rounding of a sum of large values
+      // (1e-5 of a mean of 50 against a spread of 0.05), and the merge term delta^2 inherits it
+      float shift = 0.f, mean = 0.f, m2 = 0.f;
 #pragma unroll
       for (int c = 0; c < 2; ++c) {
         float f[32];
@@ -235,13 +238,15 @@ __global__ void __launch_bounds__(THREADS, 1) gemm3_umma_kernel(const __grid_con
           for (int j = 0; j < 32; ++j) f[j] += __uint_as_float(r[c][j]);
         }
         if (gStats) {
+          if (c == 0) shift = f[0];
           float s = 0.f;
 #pragma unroll
-          for (int j = 0; j < 32; ++j) s += f[j];
+          for (int j = 0; j < 32; ++j) s += f[j] - shift;
           const float cm = s * (1.f / 32.f);
+          const float center = shift + cm;               // any centre near the mean gives the squared deviations to second order
           float cq = 0.f;
 #pragma unroll
-          for (int j = 0; j < 32; ++j) cq = fmaf(f[j] - cm, f[j] - cm, cq);
+          for (int j = 0; j < 32; ++j) cq = fmaf(f[j] - center, f[j] - center, cq);
           if (c == 0) {
             mean = cm;
             m2 = cq;
@@ -261,12 +266,12 @@ __global__ void __launch_bounds__(THREADS, 1) gemm3_umma_kernel(const __grid_con
       }
       if (gStats) {
         // the two column halves of a row meet in shared memory (N = 128: the tile holds whole rows)
-        if (half == 1) sHalf[rt] = make_float2(mean, m2);
+        if (half == 1) sHalf[rt] = make_float2(shift + mean, m2);
         asm volatile("bar.sync 3, 256;" ::: "memory");
         if (half == 0 && live) {
           const float2 h1 = sHalf[rt];
-          const float delta = h1.x - mean;
-          const float mu = mean + 0.5f * delta;
+          const float delta = (h1.x - shift) - mean;
+          const float mu = shift + (mean + 0.5f * delta);
           const float q2 = m2 + h1.y + delta * delta * 32.f;
           *reinterpret_cast<float2*>(gStats + 2 * (size_t)m) = make_float2(mu, rsqrtf(q2 * (1.f / KD) + 1e-5f));
         }
@@ -297,6 +302,12 @@ int ttk_gemm3(const Gemm3Args& g, cudaStream_t st) {
     ttk_set_error("ttk_gemm3: unsupported shape M %d N %d (K is 128, N a multiple of 128; row statistics need N = 128)", g.M, g.N);
     return TTK_ERR_UNSUPPORTED;
   }
+  // TMA reads A and W from 16-byte aligned rows; the epilogue reads R and writes C with 256-bit accesses
+  const auto misaligned = [](const void* p, uintptr_t a) { return ((uintptr_t)p & (a - 1)) != 0; };
+  if (misaligned(g.A, 16) || misaligned(g.W_hi, 16) || misaligned(g.W_lo, 16) || misaligned(g.C, 32) || misaligned(g.R, 32)) {
+    ttk_set_error("ttk_gemm3: A and W must be 16-byte aligned, C and R 32-byte aligned");
+    return TTK_ERR_ARG;
+  }
   static TtkPerDevice attr;
   if (attr.first()) {
     TTK_CUDA(cudaFuncSetAttribute(gemm3_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
@@ -312,4 +323,13 @@ int ttk_gemm3(const Gemm3Args& g, cudaStream_t st) {
   gemm3_umma_kernel<<<grid, THREADS, SMEM_BYTES, st>>>(maps, g, tiles_m, tiles_n);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
+}
+
+extern "C" int ttk_uplift_debug_gemm3(const float* a_dev, const float* w_hi_dev, const float* w_lo_dev, const float* bias_dev, const float* res_dev,
+                                      float* c_dev, int m, int n, int relu, const float* ln_stats_dev, const float* ln_gamma_dev,
+                                      const float* ln_beta_dev, float* out_stats_dev, void* stream) {
+  TTK_CHECK_ARG(a_dev && w_hi_dev && w_lo_dev && c_dev, "ttk_uplift_debug_gemm3: null pointer");
+  TTK_CHECK_ARG(!ln_stats_dev || (ln_gamma_dev && ln_beta_dev), "ttk_uplift_debug_gemm3: LayerNorm statistics need gamma and beta");
+  const Gemm3Args g{a_dev, w_hi_dev, w_lo_dev, bias_dev, res_dev, c_dev, m, n, relu, ln_stats_dev, ln_gamma_dev, ln_beta_dev, out_stats_dev};
+  return ttk_gemm3(g, (cudaStream_t)stream);
 }

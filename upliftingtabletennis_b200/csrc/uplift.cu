@@ -38,7 +38,8 @@ struct StackParams {
   float* X;               // [batch*T][128] residual stream between stages (in/out)
   const float* table_emb; // [batch][13][128]           (POS)
   const float* table;     // [batch][13][3] raw input    (POS: visibility)
-  const float* mask;      // [batch][T] {0,1}            (TEMPORAL, SECOND)
+  const float* mask;      // [batch][T] {0,1}, or additive {-1e9, 0} values when mask_additive (TEMPORAL, SECOND)
+  int mask_additive;
   const float* times;     // [batch][T] seconds          (TEMPORAL, SECOND)
   const float* cls;       // [128]                       (SECOND)
   const float* second_in; // [batch*T][128]              (SECOND: X (skip connection) or embed(pos))
@@ -156,7 +157,7 @@ __global__ void __launch_bounds__(THREADS, 1) uplift_stack_kernel(StackParams p)
   float* sW = sQ + MT * LDQ;
   float* sCos = sW + MT * LDW;      // [MT][NF]
   float* sSin = sCos + MT * NF;
-  float* sMask = sSin + MT * NF;    // additive mask per row (0 / -inf)
+  float* sMask = sSin + MT * NF;    // additive mask per row (0 / -inf, or the caller's additive values)
   float* sTime = sMask + MT;        // time per row; NaN = no rotation (cls token)
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -201,12 +202,10 @@ __global__ void __launch_bounds__(THREADS, 1) uplift_stack_kernel(StackParams p)
           m = p.table[(b * NTAB + (s - 1)) * 3 + 2] == 1.f ? 0.f : NEG_INF;    // model.py:363
           t = (float)(s - 1) / 100.f;                                           // model.py:367, arange / (MAX_FPS / 5)
         }
-      } else if (MODE == MODE_TEMPORAL) {
-        m = p.mask[seq * T + s] == 0.f ? NEG_INF : 0.f;                         // model.py:541-542
-        t = p.times[seq * T + s];
-      } else if (s > 0) {
-        m = p.mask[seq * T + (s - 1)] == 0.f ? NEG_INF : 0.f;
-        t = p.times[seq * T + (s - 1)];
+      } else if (MODE == MODE_TEMPORAL || s > 0) {
+        const float mv = p.mask[seq * T + s - (MODE == MODE_SECOND)];
+        m = p.mask_additive ? mv : (mv == 0.f ? NEG_INF : 0.f);                 // model.py:541-546
+        t = p.times[seq * T + s - (MODE == MODE_SECOND)];
       }
     }
     sMask[r] = m;
@@ -552,9 +551,10 @@ extern "C" size_t ttk_uplift_workspace_bytes(const ttk_uplift* h, int batch, int
 }
 
 extern "C" int ttk_uplift_forward(ttk_uplift* h, const float* ball_dev, const float* table_dev, const float* mask_dev,
-                                  const float* times_dev, int batch, int seq_len, int dtype, float* rot_out_dev,
+                                  const float* times_dev, int batch, int seq_len, int mask_additive, int dtype, float* rot_out_dev,
                                   float* pos_out_dev, void* workspace_dev, size_t workspace_bytes, void* stream) {
   TTK_CHECK_ARG(h, "ttk_uplift_forward: null handle");
+  h->launches = 0;
   if (int rc = ttk_bind_device(&h->device, "ttk_uplift_forward")) return rc;
   TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_TF32X3, "ttk_uplift_forward: bad dtype %d", dtype);
   TTK_CHECK_ARG(batch >= 0 && seq_len >= 2 && seq_len + 1 <= MT, "ttk_uplift_forward: seq_len must be in [2, %d] (got %d)", MT - 1, seq_len);
@@ -563,7 +563,6 @@ extern "C" int ttk_uplift_forward(ttk_uplift* h, const float* ball_dev, const fl
       ttk_set_error("ttk_uplift_forward: parameter %s was never set", p.name.c_str());
       return TTK_ERR_STATE;
     }
-  h->launches = 0;
   if (batch == 0) return TTK_OK;
   TTK_CHECK_ARG(ball_dev && table_dev && mask_dev && times_dev && rot_out_dev && pos_out_dev && workspace_dev,
                 "ttk_uplift_forward: null pointer");
@@ -609,6 +608,7 @@ extern "C" int ttk_uplift_forward(ttk_uplift* h, const float* ball_dev, const fl
     io.ball = ball_dev;
     io.table = table_dev;
     io.mask = mask_dev;
+    io.mask_additive = mask_additive;
     io.times = times_dev;
     io.batch = batch;
     io.T = T;
@@ -651,6 +651,7 @@ extern "C" int ttk_uplift_forward(ttk_uplift* h, const float* ball_dev, const fl
     io.ball = ball_dev;
     io.table = table_dev;
     io.mask = mask_dev;
+    io.mask_additive = mask_additive;
     io.times = times_dev;
     io.batch = batch;
     io.T = T;
@@ -689,6 +690,7 @@ extern "C" int ttk_uplift_forward(ttk_uplift* h, const float* ball_dev, const fl
   p.table_emb = table_emb;
   p.table = table_dev;
   p.mask = mask_dev;
+  p.mask_additive = mask_additive;
   p.times = times_dev;
   p.cls = h->dev("cls_token");
   p.second_in = X;

@@ -47,6 +47,7 @@ struct UpliftIO {
   float *rot_out, *pos_out;
   float *X, *table_emb, *second_emb;     // workspace slices
   void* attn_rows;                       // bf16 [batch*T][128]: attention output of the ball tokens in the last table-token layer
+  int mask_additive;                     // mask holds additive values ({-1e9, 0}) instead of {0, 1}
 };
 
 // gemm3_umma.cu: C = act(A' W^T + bias) (+ R) with K = 128, fp32 in / out, three TF32 tensor-core products per term (fp32-level results).

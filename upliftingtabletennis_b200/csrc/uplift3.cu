@@ -91,16 +91,17 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const float* __restric
 // FMAs and shuffles with 14 of 32 lanes busy: 4.9 ms per table-token layer against 1 ms of HBM time.)
 // SMAX: compile-time bound of the sequence length (score registers); G: sequences per CTA; SLOTS: thread slots per head (>= G S rows).
 // FIRST_ONLY: only token 0 of every sequence is a query and o has one row per SEQUENCE (last table-token layer: only the ball token is
-// used afterwards, model.py:375-378).
+// used afterwards, model.py:375-378).  mask_additive: `mask` holds the additive values themselves ({-1e9, 0}, model.py:543-544) instead of
+// {0, 1}.
 template <int MODE, int SMAX, int G, int SLOTS, bool FIRST_ONLY = false>
 __global__ void __launch_bounds__(4 * SLOTS, SLOTS == 32 ? 4 : 2) attention3_kernel(const float* __restrict__ qkv, float* __restrict__ o, const float* __restrict__ table,
                                                                      const float* __restrict__ mask, const float* __restrict__ times,
-                                                                     const float* __restrict__ invf, int batch, int T) {
+                                                                     const float* __restrict__ invf, int batch, int T, int mask_additive) {
   extern __shared__ __align__(16) float smem[];
   float* sQ = smem;                        // [rows][LDQ]: q (0..127) | k (128..255) | v (256..383)
   float* sCos = sQ + SLOTS * LDQ;          // [rows][NF]
   float* sSin = sCos + SLOTS * NF;
-  float* sMask = sSin + SLOTS * NF;        // additive key / query mask per row (0 / -inf)
+  float* sMask = sSin + SLOTS * NF;        // additive key / query mask per row (0 / -inf, or the caller's additive values)
   float* sTime = sMask + SLOTS;
   constexpr int ATT_THREADS = 4 * SLOTS;
   const int tid = threadIdx.x;
@@ -126,12 +127,10 @@ __global__ void __launch_bounds__(4 * SLOTS, SLOTS == 32 ? 4 : 2) attention3_ker
         m = table[(b * NTAB + (s - 1)) * 3 + 2] == 1.f ? 0.f : NEG_INF;        // model.py:363
         t = (float)(s - 1) / 100.f;                                               // model.py:367
       }
-    } else if (MODE == MODE_TEMPORAL) {
-      m = mask[seq * T + s] == 0.f ? NEG_INF : 0.f;                               // model.py:541-542
-      t = times[seq * T + s];
-    } else if (s > 0) {
-      m = mask[seq * T + (s - 1)] == 0.f ? NEG_INF : 0.f;
-      t = times[seq * T + (s - 1)];
+    } else if (MODE == MODE_TEMPORAL || s > 0) {
+      const float mv = mask[seq * T + s - (MODE == MODE_SECOND)];
+      m = mask_additive ? mv : (mv == 0.f ? NEG_INF : 0.f);                      // model.py:541-546
+      t = times[seq * T + s - (MODE == MODE_SECOND)];
     }
     sMask[r] = m;
     sTime[r] = t;
@@ -225,6 +224,37 @@ __global__ void __launch_bounds__(4 * SLOTS, SLOTS == 32 ? 4 : 2) attention3_ker
   for (int d = 0; d < HD; d += 4) op[d / 4] = make_float4(acc[d], acc[d + 1], acc[d + 2], acc[d + 3]);
 }
 
+// The attention instantiation of a stage: SMAX (score registers) is the smallest bound that holds S keys, the table-token stage packs two
+// sequences per CTA.  The stage and ttk_uplift_debug_attention3 both launch through here, so a test exercises the dispatch the model uses.
+int launch_attention3(int mode, bool first_only, const float* qkv, float* o, const float* table, const float* mask, const float* times,
+                      const float* invf, int batch, int T, int mask_additive, cudaStream_t st) {
+  static TtkPerDevice attr;
+  if (attr.first()) {
+    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_POS, NTAB + 1, 2, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(32)));
+    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_POS, NTAB + 1, 2, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(32)));
+    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_TEMPORAL, 52, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
+    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_TEMPORAL, 64, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
+    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_SECOND, 52, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
+    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_SECOND, 64, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
+  }
+  const int S = mode == MODE_POS ? NTAB + 1 : (mode == MODE_TEMPORAL ? T : T + 1);
+  const long long n_seq = mode == MODE_POS ? (long long)batch * T : batch;
+  if (mode == MODE_POS && first_only)
+    attention3_kernel<MODE_POS, NTAB + 1, 2, 32, true><<<ttk_cdiv(n_seq, 2), 128, att_smem(32), st>>>(qkv, o, table, mask, times, invf, batch, T, mask_additive);
+  else if (mode == MODE_POS)
+    attention3_kernel<MODE_POS, NTAB + 1, 2, 32><<<ttk_cdiv(n_seq, 2), 128, att_smem(32), st>>>(qkv, o, table, mask, times, invf, batch, T, mask_additive);
+  else if (mode == MODE_TEMPORAL && S <= 52)
+    attention3_kernel<MODE_TEMPORAL, 52, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, o, table, mask, times, invf, batch, T, mask_additive);
+  else if (mode == MODE_TEMPORAL)
+    attention3_kernel<MODE_TEMPORAL, 64, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, o, table, mask, times, invf, batch, T, mask_additive);
+  else if (S <= 52)
+    attention3_kernel<MODE_SECOND, 52, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, o, table, mask, times, invf, batch, T, mask_additive);
+  else
+    attention3_kernel<MODE_SECOND, 64, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, o, table, mask, times, invf, batch, T, mask_additive);
+  TTK_LAUNCH_CHECK();
+  return TTK_OK;
+}
+
 const char* kLayerPrefix[3] = {"firststage.pos_layers.%d.", "firststage.layers.%d.", "secondstage.%d."};
 
 std::string lname(int stage, int i, const char* suffix) {
@@ -232,6 +262,10 @@ std::string lname(int stage, int i, const char* suffix) {
   snprintf(b, sizeof(b), kLayerPrefix[stage], i);
   return std::string(b) + suffix;
 }
+
+// stats [rows][2] rounded up to whole 256-byte blocks: qkv and o / a behind it are C operands of ttk_gemm3, whose 256-bit stores need
+// 32-byte aligned rows (with an odd batch T the unpadded qkv started 16 bytes off)
+size_t stats_floats(size_t rows) { return (rows * 2 + 63) & ~(size_t)63; }
 
 }  // namespace
 
@@ -262,25 +296,16 @@ int ttk_uplift3_prepare(ttk_uplift* h) {
   return TTK_OK;
 }
 
-// x [rows][128] + stats [rows][2] + qkv [rows][384] + o / a [rows][128] for the largest stage (table tokens: batch T 14 rows)
+// x [rows][128] + stats + qkv [rows][384] + o / a [rows][128] for the largest stage (table tokens: batch T 14 rows)
 size_t ttk_uplift3_workspace_bytes(const ttk_uplift* h, int batch, int T) {
   (void)h;
   const size_t rows = (size_t)batch * T * (NTAB + 1);
-  return rows * (D + 3 * D + D + 2) * sizeof(float) + 4096;
+  return (rows * (D + 3 * D + D) + stats_floats(rows)) * sizeof(float) + 4096;
 }
 
 // One stage.  POS: io.X (ball embeddings [batch T][128]) and io.table_emb -> io.X (ball tokens after the table-token layers);
 // TEMPORAL: io.X in place; SECOND: cls + (io.X or io.second_emb) -> io.table_emb[0 .. batch) (the cls rows, input of the rotation head).
 int ttk_uplift3_stage(ttk_uplift* h, int mode, const UpliftIO& io, void* ws, cudaStream_t st) {
-  static TtkPerDevice attr;
-  if (attr.first()) {
-    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_POS, NTAB + 1, 2, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(32)));
-    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_POS, NTAB + 1, 2, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(32)));
-    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_TEMPORAL, 52, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
-    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_TEMPORAL, 64, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
-    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_SECOND, 52, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
-    TTK_CUDA(cudaFuncSetAttribute(attention3_kernel<MODE_SECOND, 64, 1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem(64)));
-  }
   const int T = io.T, batch = io.batch;
   const long long ntok = (long long)batch * T;
   const int S = mode == MODE_POS ? NTAB + 1 : (mode == MODE_TEMPORAL ? T : T + 1);
@@ -290,7 +315,7 @@ int ttk_uplift3_stage(ttk_uplift* h, int mode, const UpliftIO& io, void* ws, cud
   float* wsf = (float*)ws;
   float* x = mode == MODE_TEMPORAL ? io.X : wsf;                     // the temporal stage updates X in place
   float* stats = wsf + (size_t)batch * T * (NTAB + 1) * D;
-  float* qkv = stats + (size_t)batch * T * (NTAB + 1) * 2;
+  float* qkv = stats + stats_floats((size_t)batch * T * (NTAB + 1));
   float* oa = qkv + (size_t)batch * T * (NTAB + 1) * 3 * D;
   const float* second_in = h->skip ? io.X : io.second_emb;
   const int blocks = ttk_cdiv(rows, 8);
@@ -318,8 +343,8 @@ int ttk_uplift3_stage(ttk_uplift* h, int mode, const UpliftIO& io, void* ws, cud
     // sequence and projection + MLP run on those rows alone (1/14 of the rows), straight on io.X.
     const bool ball_only = mode == MODE_POS && i + 1 == n_layers;
     if (ball_only) {
-      attention3_kernel<MODE_POS, NTAB + 1, 2, 32, true><<<ttk_cdiv(n_seq, 2), 128, att_smem(32), st>>>(qkv, oa, io.table, io.mask, io.times, invf, batch, T);
-      TTK_LAUNCH_CHECK();
+      rc = launch_attention3(mode, true, qkv, oa, io.table, io.mask, io.times, invf, batch, T, io.mask_additive, st);
+      if (rc) return rc;
       gather_rows_kernel<<<ttk_cdiv(ntok, 8), 256, 0, st>>>(x, io.X, ntok, NTAB + 1);
       TTK_LAUNCH_CHECK();
       float* bstats = qkv;                              // q | k | v are dead once the attention has run
@@ -337,17 +362,8 @@ int ttk_uplift3_stage(ttk_uplift* h, int mode, const UpliftIO& io, void* ws, cud
       h->launches += 6;
       return TTK_OK;
     }
-    if (mode == MODE_POS)
-      attention3_kernel<MODE_POS, NTAB + 1, 2, 32><<<ttk_cdiv(n_seq, 2), 128, att_smem(32), st>>>(qkv, oa, io.table, io.mask, io.times, invf, batch, T);
-    else if (mode == MODE_TEMPORAL && S <= 52)
-      attention3_kernel<MODE_TEMPORAL, 52, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, oa, io.table, io.mask, io.times, invf, batch, T);
-    else if (mode == MODE_TEMPORAL)
-      attention3_kernel<MODE_TEMPORAL, 64, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, oa, io.table, io.mask, io.times, invf, batch, T);
-    else if (S <= 52)
-      attention3_kernel<MODE_SECOND, 52, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, oa, io.table, io.mask, io.times, invf, batch, T);
-    else
-      attention3_kernel<MODE_SECOND, 64, 1, 64><<<(int)n_seq, 256, att_smem(64), st>>>(qkv, oa, io.table, io.mask, io.times, invf, batch, T);
-    TTK_LAUNCH_CHECK();
+    rc = launch_attention3(mode, false, qkv, oa, io.table, io.mask, io.times, invf, batch, T, io.mask_additive, st);
+    if (rc) return rc;
     // x += o Wproj^T (no bias: model.py:268 passes attn_drop_rate into the proj_bias slot); statistics for LN2
     g = Gemm3Args{oa, whi + 384 * D, wlo + 384 * D, nullptr, x, x, (int)rows, D, 0, nullptr, nullptr, nullptr, stats};
     rc = ttk_gemm3(g, st);
@@ -373,4 +389,16 @@ int ttk_uplift3_stage(ttk_uplift* h, int mode, const UpliftIO& io, void* ws, cud
     h->launches++;
   }
   return TTK_OK;
+}
+
+extern "C" int ttk_uplift_debug_attention3(int mode, int first_only, const float* qkv_dev, float* o_dev, const float* table_dev,
+                                           const float* mask_dev, const float* times_dev, const float* inv_freq_dev, int batch, int seq_len,
+                                           int mask_additive, void* stream) {
+  TTK_CHECK_ARG(mode >= MODE_POS && mode <= MODE_SECOND && (!first_only || mode == MODE_POS), "ttk_uplift_debug_attention3: bad mode %d / first_only %d",
+                mode, first_only);
+  TTK_CHECK_ARG(batch > 0 && seq_len >= 2 && seq_len + 1 <= ATT_ROWS, "ttk_uplift_debug_attention3: seq_len must be in [2, %d] (got %d)",
+                ATT_ROWS - 1, seq_len);
+  TTK_CHECK_ARG(qkv_dev && o_dev && table_dev && mask_dev && times_dev && inv_freq_dev, "ttk_uplift_debug_attention3: null pointer");
+  return launch_attention3(mode, first_only != 0, qkv_dev, o_dev, table_dev, mask_dev, times_dev, inv_freq_dev, batch, seq_len, mask_additive,
+                           (cudaStream_t)stream);
 }

@@ -117,7 +117,9 @@ struct TcParams {
   __nv_bfloat16* attn_rows;
 };
 
-template <int MODE>
+// ADD_MASK: p.mask holds the additive values themselves ({-1e9, 0}) instead of {0, 1} (TEMPORAL / SECOND only).  A template argument
+// rather than a run-time flag so that the {0, 1} instantiation keeps its registers (the additive softmax holds more of them).
+template <int MODE, bool ADD_MASK = false>
 __global__ void __launch_bounds__(TC_THREADS, 1) uplift_tc_kernel(const __grid_constant__ CUtensorMap wmap, const TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();  // the swizzled operand tiles need 1024-byte alignment
@@ -132,7 +134,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) uplift_tc_kernel(const __grid_c
   float(*sMax)[ROWS] = reinterpret_cast<float(*)[ROWS]>(sW + 2 * CHUNK_BYTES);                        // [NG][ROWS] partial row maxima
   float(*sSum)[NG][ROWS] = reinterpret_cast<float(*)[NG][ROWS]>(sW + 2 * CHUNK_BYTES + NG * ROWS * 4);  // [HEADS][NG][ROWS] partial row sums
   float2(*sRed)[ROWS] = reinterpret_cast<float2(*)[ROWS]>(sKh);                                        // [NG][ROWS] LayerNorm partial sums
-  __shared__ float sMask[ROWS];                 // set-up only: additive key masks and times of the rows
+  __shared__ float sMask[ROWS];                 // additive key masks and times of the rows (-inf: never attended)
   __shared__ float sTime[ROWS];
   __shared__ uint64_t bars[4];                  // full[3], mma
   __shared__ uint32_t tmem_slot;
@@ -172,12 +174,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) uplift_tc_kernel(const __grid_c
           m = p.table[(b * NTAB + (s_row - 1)) * 3 + 2] == 1.f ? 0.f : NEG_INF;
           t_row = (float)(s_row - 1) / 100.f;
         }
-      } else if (MODE == MODE_TEMPORAL) {
-        m = p.mask[seq_row * T + s_row] == 0.f ? NEG_INF : 0.f;
-        t_row = p.times[seq_row * T + s_row];
-      } else if (s_row > 0) {
-        m = p.mask[seq_row * T + (s_row - 1)] == 0.f ? NEG_INF : 0.f;
-        t_row = p.times[seq_row * T + (s_row - 1)];
+      } else if (MODE == MODE_TEMPORAL || s_row > 0) {
+        const float mv = p.mask[seq_row * T + s_row - (MODE == MODE_SECOND)];
+        m = ADD_MASK ? mv : (mv == 0.f ? NEG_INF : 0.f);
+        t_row = p.times[seq_row * T + s_row - (MODE == MODE_SECOND)];
       }
     }
     sMask[row] = m;
@@ -198,7 +198,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) uplift_tc_kernel(const __grid_c
   const uint32_t lane_base = tmem + ((uint32_t)(quarter * 32) << 16);
   constexpr uint32_t COL_X = 384, COL_S = 0, COL_O = 128, COL_PROJ = 256, COL_FC1 = 0, COL_FC2 = 128;
   const int k_lo = g_row * SSTRIDE, k_hi = k_lo + S;        // this row's key block
-  const bool q_live = sMask[row] == 0.f;
+  const bool q_live = sMask[row] != NEG_INF;
 
   // rotary table of this thread's row (every warp group keeps a copy): angle = rint(t / 0.002) * inv_freq
   float rc[NF], rs[NF];
@@ -334,7 +334,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) uplift_tc_kernel(const __grid_c
   uint32_t key_bits = 0u;
   for (int j = 0; j < NC; ++j) {
     const int key = col0 + j;
-    if (q_live && key < k_hi && sMask[key] == 0.f) key_bits |= 1u << j;
+    if (q_live && key < k_hi && sMask[key] != NEG_INF) key_bits |= 1u << j;
   }
 
   if (warp == 0) {
@@ -505,10 +505,21 @@ __global__ void __launch_bounds__(TC_THREADS, 1) uplift_tc_kernel(const __grid_c
           tmem_ld_wait();
         }
         float mx = NEG_INF;
+        if constexpr (ADD_MASK) {
+          // finite additive masks: score * scale + (m_k + m_q) like model.py:218-224; a padded query row then attends uniformly
+          // over the valid keys (-1e9 absorbs the score)
+          const float mq = sMask[row];
 #pragma unroll
-        for (int j = 0; j < NC; ++j) {
-          e[j] = ((key_bits >> j) & 1u) ? e[j] * scale : NEG_INF;
-          mx = fmaxf(mx, e[j]);
+          for (int j = 0; j < NC; ++j) {
+            e[j] = ((key_bits >> j) & 1u) ? e[j] * scale + (sMask[col0 + j] + mq) : NEG_INF;
+            mx = fmaxf(mx, e[j]);
+          }
+        } else {
+#pragma unroll
+          for (int j = 0; j < NC; ++j) {
+            e[j] = ((key_bits >> j) & 1u) ? e[j] * scale : NEG_INF;
+            mx = fmaxf(mx, e[j]);
+          }
         }
         sMax[grp][row] = mx;
         quad_barrier(quarter);
@@ -710,6 +721,8 @@ int ttk_uplift_tc_stage(ttk_uplift* h, int mode, const UpliftIO& io, cudaStream_
     TTK_CUDA(cudaFuncSetAttribute(uplift_tc_kernel<MODE_POS>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
     TTK_CUDA(cudaFuncSetAttribute(uplift_tc_kernel<MODE_TEMPORAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
     TTK_CUDA(cudaFuncSetAttribute(uplift_tc_kernel<MODE_SECOND>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
+    TTK_CUDA(cudaFuncSetAttribute(uplift_tc_kernel<MODE_TEMPORAL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
+    TTK_CUDA(cudaFuncSetAttribute(uplift_tc_kernel<MODE_SECOND, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM));
   }
   const int n_layers_total = h->depth + 4;
   CUtensorMap wmap;
@@ -746,13 +759,19 @@ int ttk_uplift_tc_stage(ttk_uplift* h, int mode, const UpliftIO& io, cudaStream_
     p.n_layers = h->depth - 4;
     p.layer_first = 4;
     p.out_rows = io.X;
-    uplift_tc_kernel<MODE_TEMPORAL><<<ttk_cdiv(io.batch, 2), TC_THREADS, TC_SMEM, st>>>(wmap, p);
+    if (io.mask_additive)
+      uplift_tc_kernel<MODE_TEMPORAL, true><<<ttk_cdiv(io.batch, 2), TC_THREADS, TC_SMEM, st>>>(wmap, p);
+    else
+      uplift_tc_kernel<MODE_TEMPORAL><<<ttk_cdiv(io.batch, 2), TC_THREADS, TC_SMEM, st>>>(wmap, p);
   } else {
     p.layers = h->layers_dev + h->depth;
     p.n_layers = 4;
     p.layer_first = h->depth;
     p.out_rows = io.table_emb;        // dead by now: receives the [batch][128] cls rows
-    uplift_tc_kernel<MODE_SECOND><<<ttk_cdiv(io.batch, 2), TC_THREADS, TC_SMEM, st>>>(wmap, p);
+    if (io.mask_additive)
+      uplift_tc_kernel<MODE_SECOND, true><<<ttk_cdiv(io.batch, 2), TC_THREADS, TC_SMEM, st>>>(wmap, p);
+    else
+      uplift_tc_kernel<MODE_SECOND><<<ttk_cdiv(io.batch, 2), TC_THREADS, TC_SMEM, st>>>(wmap, p);
   }
   TTK_LAUNCH_CHECK();
   return TTK_OK;

@@ -46,14 +46,16 @@ class UpliftEngine:
 
     TF32X3_CHUNK = 4096          # trajectories per library call on the tf32x3 path: its activations live in HBM (7.3 GB per 4096)
 
-    def forward(self, ball, table, mask, times, dtype=torch.float32):
+    def forward(self, ball, table, mask, times, dtype=torch.float32, mask_additive=False):
+        """mask_additive False: mask in {0, 1}; True: mask holds the reference's additive {-1e9, 0} values, which it keeps as they are
+        (uplifting/model.py:541-546), so padded rows attend to the valid frames instead of to nothing."""
         assert self.loaded
         B, T, _ = ball.shape
         dev = ball.device
         dt = lib_enum(dtype)
         if dt == _lib.TF32X3 and B > self.TF32X3_CHUNK:
             parts = [self.forward(ball[i:i + self.TF32X3_CHUNK], table[i:i + self.TF32X3_CHUNK], mask[i:i + self.TF32X3_CHUNK],
-                                  times[i:i + self.TF32X3_CHUNK], dtype) for i in range(0, B, self.TF32X3_CHUNK)]
+                                  times[i:i + self.TF32X3_CHUNK], dtype, mask_additive) for i in range(0, B, self.TF32X3_CHUNK)]
             return torch.cat([p[0] for p in parts]), torch.cat([p[1] for p in parts])
         args = [a.to(torch.float32).contiguous() for a in (ball, table, mask, times)]
         need = lib.ttk_uplift_workspace_bytes(self.h, B, T, dt)
@@ -61,8 +63,8 @@ class UpliftEngine:
             self._ws = torch.empty((need,), dtype=torch.uint8, device=dev)
         rot = torch.empty((B, 3), dtype=torch.float32, device=dev)
         pos = torch.empty((B, T, 3), dtype=torch.float32, device=dev)
-        check(lib.ttk_uplift_forward(self.h, ptr(args[0]), ptr(args[1]), ptr(args[2]), ptr(args[3]), B, T, dt, ptr(rot), ptr(pos),
-                                     ptr(self._ws), self._ws.numel(), stream_ptr()))
+        check(lib.ttk_uplift_forward(self.h, ptr(args[0]), ptr(args[1]), ptr(args[2]), ptr(args[3]), B, T, int(bool(mask_additive)), dt,
+                                     ptr(rot), ptr(pos), ptr(self._ws), self._ws.numel(), stream_ptr()))
         return rot, pos
 
     def last_launches(self):
@@ -116,16 +118,17 @@ class MultiStageModel(PrecisionMixin, nn.Module):
     def forward(self, ball_pos, table_pos, mask, times):
         if not ball_pos.is_cuda:
             raise RuntimeError('upliftingtabletennis_b200 runs on a B200 GPU only; move the inputs to CUDA (there is no CPU fallback)')
-        # uplifting/model.py:541-546 -- same host-side check (and the same ValueError on an all-ones mask)
+        # uplifting/model.py:541-546 -- same host-side check (and the same ValueError on an all-ones mask); like the reference, an
+        # additive {-1e9, 0} mask is used as it is
         mn, mx = float(mask.min()), float(mask.max())
         if mn == 0 and mx == 1:
-            pass
+            additive = False
         elif mx == 0 and mn < -1e8:
-            mask = (mask == 0).to(torch.float32)
+            additive = True
         else:
             raise ValueError('wrong format for masks. Should be 0, 1 or -1e9, 0.')
         self._sync()
-        return self.engine.forward(ball_pos, table_pos, mask, times, self.compute_dtype)
+        return self.engine.forward(ball_pos, table_pos, mask, times, self.compute_dtype, mask_additive=additive)
 
 
 def get_model(name='singlestage', size='small', mode='stacked', time_rotation='new', dtype=None):
