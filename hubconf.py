@@ -18,12 +18,12 @@ def ball_detection(model_name='segformerpp_b2', dtype=None, **kwargs):
     """Loads the Ball Detection Model.  B200 kernels exist for 'wasb' and 'vitpose'; the reference's default name is kept, but
     segformer++ is not part of the reference repository and raises NotImplementedError before anything is downloaded.
     dtype: 'tf32' (WASB default: tensor cores at the precision class of the reference's cuDNN convolutions), 'tf32x3' (ViTPose
-    default: float32-class results on the tensor cores), 'fp32' (SIMT), 'bf16'."""
+    default, WASB on request: float32-class results on the tensor cores), 'fp32' (SIMT), 'bf16'."""
     return BallDetector(model_name=model_name, dtype=dtype)
 
 
 def table_detection(model_name='segformerpp_b2', dtype=None, **kwargs):
-    """Loads the Table Detection Model.  B200 kernels exist for 'hrnet' and 'vitpose'."""
+    """Loads the Table Detection Model.  B200 kernels exist for 'hrnet' and 'vitpose'.  dtype: as for ball_detection."""
     return TableDetector(model_name=model_name, dtype=dtype)
 
 

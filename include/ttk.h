@@ -29,7 +29,7 @@ extern "C" {
 enum { TTK_OK = 0, TTK_ERR_ARG = -1, TTK_ERR_CUDA = -2, TTK_ERR_STATE = -3, TTK_ERR_UNSUPPORTED = -4 };
 /* Arithmetic / storage type of a path.  TTK_TF32: fp32 storage, tensor-core products with TF32 operands (inputs rounded to
  * nearest-even TF32 by TMA, fp32 accumulate) -- the class cuDNN uses for the reference's convolutions on a GPU.
- * TTK_TF32X3 (uplifting transformer): fp32 storage, every product as three TF32 tensor-core products of split operands
+ * TTK_TF32X3 (uplifting transformer, ViTPose, HRNet): fp32 storage, every product as three TF32 tensor-core products of split operands
  * (a_hi b_hi + a_lo b_hi + a_hi b_lo) -- fp32-level results, the class of the reference's fp32 Linear layers. */
 enum { TTK_F32 = 0, TTK_BF16 = 1, TTK_TF32 = 2, TTK_TF32X3 = 3 };
 enum { TTK_DECODE_TABLE = 0, TTK_DECODE_BALL = 1 }; /* the two live sub-pixel variants */
@@ -89,7 +89,10 @@ TTK_API size_t ttk_hrnet_workspace_bytes(const ttk_hrnet* h, int batch, int heig
  * H and W must be multiples of 8.  dtype TTK_F32: fp32 SIMT path (parity with the CPU
  * reference at 1e-4); TTK_TF32: x and the activations are float32, the convolutions run on the
  * tcgen05 tensor cores with TF32 operands (the reference-on-GPU class, balldetection/models/wasb.py:29-105
- * through cuDNN's default TF32); TTK_BF16: tcgen05 path with bf16 storage, fp32 accumulate. */
+ * through cuDNN's default TF32); TTK_TF32X3: float32 tensors as for TTK_TF32, every product as three TF32 tensor-core products of
+ * split operands (fp32-level results: the reference on a CPU, or on a GPU with cudnn.allow_tf32 off; no fused BasicBlock or bottleneck
+ * kernels); TTK_BF16: tcgen05 path with bf16 storage, fp32 accumulate.  A convolution without a tensor-core kernel for its shape runs
+ * on the SIMT kernel of the same storage type. */
 TTK_API int ttk_hrnet_forward(ttk_hrnet* h, const void* x_dev, int batch, int height, int width, int dtype,
                       float* heatmaps_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 /* kernels launched by the last ttk_hrnet_forward on this handle (for bench accounting) */
@@ -99,13 +102,14 @@ TTK_API int ttk_hrnet_last_launches(const ttk_hrnet* h);
 TTK_API int ttk_hrnet_set_subbatch(ttk_hrnet* h, int images);
 /* Measurement aid (bench.py): when enabled, ttk_hrnet_forward brackets every kernel launch with CUDA
  * events on `stream`.  After the caller synchronised the stream, ttk_hrnet_profile_read returns, per
- * launch: op type (0 conv, 1 fuse-sum, 2 final conv), conv index (-1 if none), duration in ms,
+ * launch: op type (0 conv, 1 fuse-sum, 2 final conv, 3 conv of a tensor-core path that ran on the SIMT kernel because its shape has
+ * no tensor-core kernel), conv index (-1 if none), duration in ms,
  * algorithmic flops (2*MAC on the reference's logical channel counts) and compulsory bytes
  * (inputs + outputs + weights once). */
 TTK_API int ttk_hrnet_set_force_simt(ttk_hrnet* h, int enable);   /* bf16 path through the SIMT kernels (cross-check of the tcgen05 path) */
 /* Test hook: run one convolution of the plan on caller buffers (NHWC, channels padded to 16): out = act(conv(in) + bias [+ res]).
- * path 0: fp32 SIMT (float32 tensors), 1: bf16 SIMT, 2: bf16 tcgen05, 3: TF32 tcgen05 on float32 tensors (2 / 3 return
- * TTK_ERR_UNSUPPORTED when the shape has no tensor-core kernel). */
+ * path 0: fp32 SIMT (float32 tensors), 1: bf16 SIMT, 2: bf16 tcgen05, 3: TF32 tcgen05 on float32 tensors, 4: 3xTF32 tcgen05 on
+ * float32 tensors (2 to 4 return TTK_ERR_UNSUPPORTED when the shape has no tensor-core kernel; any other path is TTK_ERR_ARG). */
 TTK_API int ttk_hrnet_debug_conv(ttk_hrnet* h, int conv_index, const void* in_dev, int n, int hin, int win, const void* res_dev,
                          int relu, int path, void* out_dev, void* stream);
 /* Test hook: one BasicBlock (convs conv_index and conv_index + 1, 16 or 32 padded channels) through the fused tcgen05 kernel:

@@ -1,4 +1,4 @@
-"""Per-launch table of one detector pass (ttk_hrnet_set_profile): python tools/layer_profile.py [tf32|bf16|fp32] [batch] [out.json]."""
+"""Per-launch table of one detector pass (ttk_hrnet_set_profile): python tools/layer_profile.py [tf32|tf32x3|bf16|fp32] [batch] [out.json]."""
 import ctypes as C
 import json
 import os
@@ -44,10 +44,11 @@ check(lib.ttk_hrnet_set_profile(eng.h, 0))
 rows = []
 for (t_, c_), v in sorted(per.items(), key=lambda kv: -kv[1][0]):
     nm = eng.specs[c_][0] if c_ >= 0 else ('fuse_sum' if t_ == 1 else 'final_conv')
-    rows.append({'kernel': nm, 'spec_cin_cout_k_stride': eng.specs[c_][2:] if c_ >= 0 else None, 'launches': v[3], 'ms': v[0], 'share': v[0] / tot,
+    rows.append({'kernel': nm, 'spec_cin_cout_k_stride': eng.specs[c_][2:] if c_ >= 0 else None, 'simt_fallback': t_ == 3, 'launches': v[3], 'ms': v[0], 'share': v[0] / tot,
                  'tflops': v[1] / (v[0] * 1e-3) / 1e12, 'gbs': v[2] / (v[0] * 1e-3) / 1e9})
 print('profiled total %.2f ms' % tot)
 for r in rows[:45]:
-    print('%-42s %-18s n=%2d ms=%6.3f share=%5.1f%% tf=%6.0f gbs=%5.0f' % (r['kernel'], r['spec_cin_cout_k_stride'], r['launches'], r['ms'], 100 * r['share'], r['tflops'], r['gbs']))
+    print('%-42s %-18s n=%2d ms=%6.3f share=%5.1f%% tf=%6.0f gbs=%5.0f%s' % (r['kernel'], r['spec_cin_cout_k_stride'], r['launches'], r['ms'], 100 * r['share'], r['tflops'], r['gbs'],
+                                                                        ' (SIMT fallback)' if r['simt_fallback'] else ''))
 if len(sys.argv) > 3:
     json.dump({'precision': prec, 'batch': n, 'total_ms': tot, 'ms_per_pass': ms, 'rows': rows}, open(sys.argv[3], 'w'), indent=1)

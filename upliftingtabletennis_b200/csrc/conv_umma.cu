@@ -30,6 +30,14 @@
 // Roles (persistent CTA, static tile round-robin): warp 0 = TMA producer, warp 1 = MMA issuer
 // (one elected thread), warps 2-5 = epilogue (TMEM -> registers -> bias/residual/ReLU -> bf16 -> global).
 // Pipelines: smem full/empty ring over load units, double-buffered TMEM accumulators (tmem full/empty).
+//
+// 3xTF32 (template flag X3, fp32 elements): fp32-level products on the same tensor cores.  Every operand is split into two TF32
+// numbers, x = x_hi + x_lo with x_hi = tf32(x) and x_lo = x - x_hi, and each MMA of the TF32 kernel becomes three into the same
+// accumulator: A_hi W_hi + A_lo W_hi + A_hi W_lo (the dropped A_lo W_lo and kind::tf32 truncating the lo terms are 2^-22 of a product
+// each, as in gemm3_umma.cu).  The input map has type FLOAT32, so TMA stages the raw values; four transform warps (6-9) split a
+// staged unit element by element -- hi in place, lo into a second plane behind it with the same swizzle -- before the MMA warp may
+// read it, so HBM traffic is that of the TF32 kernel.  W_hi and W_lo are split once by the host and both stay resident.  Both
+// planes double the shared memory of the weights and of a stage, so the x3 tiles are sized separately (see kc_of / cout_tile).
 #include <cuda.h>
 
 #include <string.h>
@@ -47,6 +55,7 @@ using namespace umma;
 constexpr int BW = 128;          // output pixels per tile row = MMA M
 constexpr int THREADS = 192;         // TMA warp, MMA warp, 4 epilogue warps
 constexpr int THREADS_HF = 320;      // horizontal tap fusion: 8 epilogue warps (two per TMEM lane quarter, alternating output rows)
+constexpr int THREADS_X3 = 320;      // 3xTF32: TMA warp, MMA warp, 4 epilogue warps, 4 transform warps
 
 constexpr int pow2_cols(int c) { return c <= 32 ? 32 : c <= 64 ? 64 : c <= 128 ? 128 : c <= 256 ? 256 : 512; }
 constexpr int al1024(int b) { return (b + 1023) & ~1023; }
@@ -54,8 +63,9 @@ constexpr int al1024(int b) { return (b + 1023) & ~1023; }
 // KS: 1 or 3; S: stride 1 or 2 (3x3 only); CIN: padded input channels; COUT: output channels handled by one CTA
 // (blockIdx.y selects the slice when the layer has more); R: output rows per tile; STAGES: smem ring depth;
 // RB: reserve shared memory for TMA-staged residual tiles (double buffered with the accumulators);
-// KCO: channels per K-chunk when not the default (a narrower chunk buys a taller tile for the same shared memory).
-template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0>
+// KCO: channels per K-chunk when not the default (a narrower chunk buys a taller tile for the same shared memory);
+// X3: 3xTF32 (hi and lo planes of every staged unit and of the weights).
+template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0, int X3 = 0>
 struct Cfg {
   static constexpr int KCMAX = 128 / ESZ;                           // a swizzled smem row holds at most 128 bytes
   static constexpr int KC = KCO ? KCO : (CIN < KCMAX ? CIN : KCMAX);      // channels per K-chunk = one swizzled smem row
@@ -71,11 +81,13 @@ struct Cfg {
   static constexpr int TR = S == 2 ? R + 1 : R + 2 * PAD;
   static constexpr int BOX_BYTES = TR * TW * ROWB;
   static constexpr int BOX_AL = al1024(BOX_BYTES);
-  static constexpr int STAGE_BYTES = NBOX * BOX_AL;
+  static constexpr int NPLANE = X3 ? 2 : 1;
+  static constexpr int A_BYTES = NBOX * BOX_AL;         // one plane of a stage (X3: hi; lo follows)
+  static constexpr int STAGE_BYTES = NPLANE * A_BYTES;
   static constexpr int UNITS = NKC * NPY;               // load units per tile
   static constexpr int TAPS = KS * KS;
   static constexpr int W_BYTES = TAPS * NKC * COUT * ROWB;
-  static constexpr int W_BYTES_AL = al1024(W_BYTES);
+  static constexpr int W_BYTES_AL = al1024(W_BYTES);      // one plane of the weights (X3: W_hi; W_lo follows)
   static constexpr int ACC_COLS = (HF ? 3 : 1) * R * COUT;      // HF: three accumulator sets (one per horizontal tap) per output row
   static constexpr int TMEM_COLS = pow2_cols(2 * ACC_COLS);
   // residual staging: boxes of CB channels (<= 128 swizzled bytes per pixel) x 128 px x R rows
@@ -86,7 +98,7 @@ struct Cfg {
   static constexpr int RES_BYTES = RB ? 2 * NRB * RBOX_BYTES : 0;
   static constexpr uint32_t RSWZ = RROWB == 32 ? 1u : RROWB == 64 ? 3u : 7u;
   static constexpr int XCH_BYTES = HF ? 4 * 2 * R * COUT * 4 : 0;      // HF: edge-lane exchange between the four epilogue warps
-  static constexpr int SMEM_BASE = 1024 + W_BYTES_AL + STAGES * STAGE_BYTES + RES_BYTES + COUT * 4 + XCH_BYTES + 256;
+  static constexpr int SMEM_BASE = 1024 + NPLANE * W_BYTES_AL + STAGES * STAGE_BYTES + RES_BYTES + COUT * 4 + XCH_BYTES + 256;
   // STG (fp32 layers with >= 32 output channels per CTA, where shared memory allows): a column group (32 channels = 128 contiguous
   // bytes of a pixel) is staged per warp in shared memory and written out row-contiguous -- 8 pixels x 128 bytes per store
   // instruction instead of 32 pixels x 32 bytes, a quarter of the L1 wavefronts.  The wide layers' epilogues are bound by exactly
@@ -107,6 +119,8 @@ struct Cfg {
   static constexpr int GMAX = (ESZ == 2 && !PIPE) ? 64 : 32;
   static constexpr int GCOLS = ACC_COLS < GMAX ? ACC_COLS : GMAX;     // accumulator columns fetched per TMEM wait
   static_assert(ESZ == 2 || ESZ == 4, "bf16 or tf32-in-fp32 elements");
+  static_assert(!X3 || (ESZ == 4 && !HF), "3xTF32: fp32 elements, no horizontal tap fusion");
+  static_assert(3 * STAGES + 6 <= 31, "barriers and the TMEM slot share 256 bytes");
   static_assert(ACC_COLS % GCOLS == 0, "the epilogue drains whole groups of accumulator columns");
   static_assert(ROWB == 32 || ROWB == 64 || ROWB == 128, "a K-chunk is one 32/64/128-byte swizzled row");
   static_assert(COUT % 16 == 0 && COUT <= 256 && CIN % 16 == 0, "bad channel counts");
@@ -120,6 +134,7 @@ struct KMaps {
 
 struct KArgs {
   const void* w;               // packed weights, see ttk_conv_umma_pack
+  const void* w_lo;            // X3: the W_lo image (same layout)
   const float* bias;
   void* out;
   const void* res[3];
@@ -132,36 +147,38 @@ struct KArgs {
   int tiles_x, tiles_y, total;
 };
 
-template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0>
-__global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel(const __grid_constant__ KMaps maps, const KArgs a) {
-  constexpr int NTHR = HF ? THREADS_HF : THREADS;
-  using C = Cfg<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF>;
+template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0, int X3 = 0>
+__global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1) conv_umma_kernel(const __grid_constant__ KMaps maps, const KArgs a) {
+  constexpr int NTHR = HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS;
+  using C = Cfg<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* sW = smem;
-  uint8_t* sA = smem + C::W_BYTES_AL;
+  uint8_t* sA = smem + C::NPLANE * C::W_BYTES_AL;
   uint8_t* sR = sA + STAGES * C::STAGE_BYTES;           // [acc][box][row][px][CB] swizzled (1024-aligned)
   float* sBias = reinterpret_cast<float*>(sR + C::RES_BYTES);
   float* sXch = sBias + COUT;                           // HF: [warp][set 0 of lane 31 | set 2 of lane 0][R][COUT]
   uint64_t* bars = reinterpret_cast<uint64_t*>(sXch + C::XCH_BYTES / 4);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 6);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * STAGES + 6);
   // STG: per-warp staging rows of 128 bytes, 128-byte aligned (behind the barriers' 256 bytes)
   uint8_t* sStage = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(bars) + 256 + 127) & ~(uintptr_t)127);
   const uint32_t bar_full = smem_u32(bars), bar_empty = bar_full + 8 * STAGES, bar_tfull = bar_empty + 8 * STAGES,
-                 bar_tempty = bar_tfull + 16, bar_rfull = bar_tempty + 16;
+                 bar_tempty = bar_tfull + 16, bar_rfull = bar_tempty + 16,
+                 bar_ready = bar_rfull + 16;      // X3: unit split into hi / lo by the transform warps
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int n_off = blockIdx.y * COUT;                  // output-channel slice of this CTA
   const bool res_tma = RB && a.res_tma;
 
   // ---- one-time setup: weights (software swizzle on absolute address bits, as TMA does), bias, barriers, TMEM ----
   {
-    const uint4* wsrc = reinterpret_cast<const uint4*>(a.w) + (size_t)blockIdx.y * (C::W_BYTES / 16);
+    constexpr int WV = C::W_BYTES / 16, CPR = C::ROWB / 16;
     const uint32_t wbase = smem_u32(sW);
-    constexpr int CPR = C::ROWB / 16;
-    for (int i = tid; i < C::W_BYTES / 16; i += NTHR) {
-      uint32_t addr = wbase + (i / CPR) * C::ROWB + (i % CPR) * 16;
+    for (int i = tid; i < C::NPLANE * WV; i += NTHR) {
+      const int p = i / WV, j = i - p * WV;             // plane (X3: 0 = W_hi, 1 = W_lo), 16-byte piece within it
+      const uint4* wsrc = reinterpret_cast<const uint4*>(p ? a.w_lo : a.w) + (size_t)blockIdx.y * WV;
+      uint32_t addr = wbase + p * C::W_BYTES_AL + (j / CPR) * C::ROWB + (j % CPR) * 16;
       addr ^= ((addr >> 7) & C::SWZ) << 4;
-      *reinterpret_cast<uint4*>(sW + (addr - wbase)) = __ldg(wsrc + i);
+      *reinterpret_cast<uint4*>(sW + (addr - wbase)) = __ldg(wsrc + j);
     }
     for (int i = tid; i < COUT; i += NTHR) sBias[i] = a.bias[n_off + i];
   }
@@ -169,6 +186,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(bar_full + 8 * s, 1);
       mbar_init(bar_empty + 8 * s, 1);
+      if (X3) mbar_init(bar_ready + 8 * s, 4);
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(bar_tfull + 8 * i, 1);
@@ -229,7 +247,17 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem, 0);
       const bool leader = elect_one();
       const uint32_t wbase = smem_u32(sW) >> 4;
-      auto issue = [leader](uint32_t d, uint64_t da, uint64_t db, uint32_t idesc) {      // every MMA accumulates (the epilogue zeroes what it drains)
+      // operands as 16-byte shared-memory addresses of A and B; every MMA accumulates (the epilogue zeroes what it drains)
+      auto issue = [leader](uint32_t d, uint32_t a16, uint32_t b16, uint32_t idesc) {
+        const uint64_t da = make_desc16<8 * C::ROWB, C::LAYOUT>(a16), db = make_desc16<8 * C::ROWB, C::LAYOUT>(b16);
+        if (X3) {      // the lo planes sit one plane behind the hi planes
+          const uint64_t da_lo = make_desc16<8 * C::ROWB, C::LAYOUT>(a16 + C::A_BYTES / 16);
+          const uint64_t db_lo = make_desc16<8 * C::ROWB, C::LAYOUT>(b16 + C::W_BYTES_AL / 16);
+          if (leader) {
+            mma_tf32(d, da_lo, db, idesc, 1u);
+            mma_tf32(d, da, db_lo, idesc, 1u);
+          }
+        }
         if (leader) {
           if (ESZ == 2) mma(d, da, db, idesc, 1u);
           else mma_tf32(d, da, db, idesc, 1u);
@@ -244,7 +272,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
         for (int u = 0; u < C::UNITS; ++u, ++it) {
           const int kc = u / C::NPY, py = u % C::NPY;
           const uint32_t s = it % STAGES, ph = (it / STAGES) & 1;
-          mbar_wait(bar_full + 8 * s, ph);
+          mbar_wait((X3 ? bar_ready : bar_full) + 8 * s, ph);
           fence_after();
           const uint32_t abase = smem_u32(sA + s * C::STAGE_BYTES) >> 4;      // 16-byte units from here on (make_desc16)
           constexpr uint32_t RB16 = C::ROWB / 16;
@@ -263,7 +291,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
               const uint32_t brow = wbase + ((kc * 3 + k0) * 3 * COUT) * RB16;
 #pragma unroll
               for (int ks = 0; ks < C::KSTEPS; ++ks)
-                issue(d_tmem, make_desc16<8 * C::ROWB, C::LAYOUT>(arow + ks * 2), make_desc16<8 * C::ROWB, C::LAYOUT>(brow + ks * 2), idesc);
+                issue(d_tmem, arow + ks * 2, brow + ks * 2, idesc);
             }
           } else if (C::FUSE) {
             // input (halo) row hr = yi + 1 feeds output rows yo = yi + 1 - ky; row yo lives in column block R-1-yo
@@ -280,7 +308,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
                 const uint32_t brow = wbase + (((kc * 3 + kx) * 3 + k0) * COUT) * RB16;
 #pragma unroll
                 for (int ks = 0; ks < C::KSTEPS; ++ks)
-                  issue(d_tmem, make_desc16<8 * C::ROWB, C::LAYOUT>(arow + ks * 2), make_desc16<8 * C::ROWB, C::LAYOUT>(brow + ks * 2), idesc);
+                  issue(d_tmem, arow + ks * 2, brow + ks * 2, idesc);
               }
             }
           } else {
@@ -302,7 +330,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
                 const uint32_t brow = wbase + ((tap * C::NKC + kc) * COUT) * RB16;
 #pragma unroll
                 for (int ks = 0; ks < C::KSTEPS; ++ks)
-                  issue(d_tmem, make_desc16<8 * C::ROWB, C::LAYOUT>(arow + ks * 2), make_desc16<8 * C::ROWB, C::LAYOUT>(brow + ks * 2), idesc);
+                  issue(d_tmem, arow + ks * 2, brow + ks * 2, idesc);
               }
             }
           }
@@ -310,6 +338,36 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
         }
         if (leader) commit(bar_tfull + 8 * acc);          // accumulators complete
         __syncwarp();
+      }
+    }
+  } else if (X3 && warp >= 6) {
+    // ===== transform warps 6..9: raw fp32 unit -> hi = tf32(x) in place, lo = x - hi into the second plane =====
+    // element-wise at the same offsets: both planes are 1024-byte aligned, so the swizzle TMA applied holds for both
+    const int t = tid - 6 * 32;
+    uint32_t it = 0;
+    for (int tile = blockIdx.x; tile < a.total; tile += gridDim.x) {
+      for (int u = 0; u < C::UNITS; ++u, ++it) {
+        const uint32_t s = it % STAGES, ph = (it / STAGES) & 1;
+        mbar_wait(bar_full + 8 * s, ph);
+#pragma unroll
+        for (int b = 0; b < C::NBOX; ++b) {
+          uint8_t* hi = sA + s * C::STAGE_BYTES + b * C::BOX_AL;
+          uint8_t* lo = hi + C::A_BYTES;
+#pragma unroll 4
+          for (int i = t; i < C::BOX_BYTES / 16; i += 128) {
+            const float4 v = *reinterpret_cast<const float4*>(hi + i * 16);
+            float4 h, l;
+            split_tf32(v.x, h.x, l.x);
+            split_tf32(v.y, h.y, l.y);
+            split_tf32(v.z, h.z, l.z);
+            split_tf32(v.w, h.w, l.w);
+            *reinterpret_cast<float4*>(hi + i * 16) = h;
+            *reinterpret_cast<float4*>(lo + i * 16) = l;
+          }
+        }
+        fence_async_smem();              // generic-proxy writes -> visible to the tensor core
+        __syncwarp();
+        if (lane == 0) mbar_arrive(bar_ready + 8 * s);
       }
     }
   } else {
@@ -644,18 +702,25 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : THREADS, 1) conv_umma_kernel
 // host side
 // ------------------------------------------------------------------------------------------
 // output channels one CTA handles: 128-wide 3x3 layers with 64+ input channels are split so the weights fit in shared memory
-int cout_tile(const TtkConv& cv, int esz) { return (cv.k == 3 && cv.cout_p == 128 && cv.cin_p >= 64) ? (esz == 2 ? 64 : 32) : cv.cout_p; }
-bool fused_ky(const TtkConv& cv, int esz) { return cv.k == 3 && cv.stride == 1 && 3 * cout_tile(cv, esz) <= 256; }
+// 3xTF32 (x3): W_hi and W_lo of a 3x3 slice are 72 cin_p cout_tile bytes; cin_p cout_tile <= 2048 keeps them at <= 144 KB
+int cout_tile(const TtkConv& cv, int esz, bool x3 = false) {
+  if (x3) return cv.k == 3 ? std::min(cv.cout_p, 2048 / cv.cin_p) : cv.cout_p;
+  return (cv.k == 3 && cv.cout_p == 128 && cv.cin_p >= 64) ? (esz == 2 ? 64 : 32) : cv.cout_p;
+}
+bool fused_ky(const TtkConv& cv, int esz, bool x3 = false) { return cv.k == 3 && cv.stride == 1 && 3 * cout_tile(cv, esz, x3) <= 256; }
 // horizontal + vertical tap fusion (one MMA per input row and K step, N = 9 Cout): the thin layer that is bound by its MMA count
 // -- TF32 only: with K = 8 per instruction it has twice the MMAs of the bf16 kernel (4.48 -> 3.50 ms per 32 stacks); in bf16 the extra
 // epilogue work (three accumulator sets, two shuffles per value, edge-lane exchange) outweighs the saved MMAs (1.74 -> 3.00 ms)
-bool fused_h(const TtkConv& cv, int esz) { return esz == 4 && cv.k == 3 && cv.stride == 1 && cv.cin_p == 128 && cv.cout_p == 16; }
+bool fused_h(const TtkConv& cv, int esz, bool x3 = false) { return esz == 4 && !x3 && cv.k == 3 && cv.stride == 1 && cv.cin_p == 128 && cv.cout_p == 16; }
 // channels per K-chunk (one swizzled shared-memory row).  The stride-1 3x3 layers with 64+ input channels are bound by their MMA
 // count (a 128-pixel x 32-byte MMA holds the tensor pipe 45.5 clk at N <= 48 and N / 2 clk from N = 96 on, tools/tf32_probe.cu) and
 // the halo rows of a tile are pure overhead: 3 (R + 2) / R MMAs per K step and output row.  Narrow chunks shrink the staging boxes so
 // that taller tiles fit: bf16 transition1.0 R = 3 -> 8, the 64 -> 64 layers R = 2 -> 4, and the 128 -> 128 layers get a second
 // pipeline stage.  With fp32 elements the 3x3 weights of the wide layers take up to 147 KB, which leaves room for 8-channel chunks.
-int kc_of(const TtkConv& cv, int esz) {
+// x3: the narrowest chunk for every 3x3 layer (one 32-byte row, one MMA K step): the MMA count does not depend on it, and the
+// staging boxes -- two planes each -- stay small enough for two stages next to up to 144 KB of weights.
+int kc_of(const TtkConv& cv, int esz, bool x3 = false) {
+  if (x3) return cv.k == 3 ? 8 : std::min(cv.cin_p, 32);
   if (esz == 2) {
     if (cv.k == 3 && cv.stride == 1 && cv.cin_p >= 64) return 32;
     // stride 2 with 64+ input channels (transition1.1 1.74 -> 1.49 ms): two-row tiles and a third pipeline stage in the same shared memory
@@ -682,12 +747,12 @@ float round_tf32(float v) {      // nearest-even on the 13 dropped mantissa bits
   return v;
 }
 
-template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0>
+template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0, int X3 = 0>
 int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
-  using C = Cfg<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF>;
-  if (C::KC != kc_of(cv, ESZ) || COUT != cout_tile(cv, ESZ) || (HF != 0) != fused_h(cv, ESZ)) {
+  using C = Cfg<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3>;
+  if (C::KC != kc_of(cv, ESZ, X3) || COUT != cout_tile(cv, ESZ, X3) || (HF != 0) != fused_h(cv, ESZ, X3)) {
     ttk_set_error("conv %s: kernel K-chunk %d / output slice %d differ from the packed weights' %d / %d", cv.name.c_str(), C::KC, COUT,
-                  kc_of(cv, ESZ), cout_tile(cv, ESZ));
+                  kc_of(cv, ESZ, X3), cout_tile(cv, ESZ, X3));
     return TTK_ERR_STATE;
   }
   EncodeFn encode = get_encode();
@@ -697,12 +762,13 @@ int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
   }
   static TtkPerDevice attr;
   if (attr.first()) {
-    TTK_CUDA(cudaFuncSetAttribute(conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    TTK_CUDA(cudaFuncSetAttribute(conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   C::SMEM_BYTES));
   }
   if (S == 2 && ((a.hin & 1) || (a.win & 1))) return TTK_ERR_UNSUPPORTED;
-  // the input map's TFLOAT32 type makes TMA round fp32 to TF32 (nearest-even) while it fills shared memory
-  const CUtensorMapDataType in_type = ESZ == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32;
+  // the input map's TFLOAT32 type makes TMA round fp32 to TF32 (nearest-even) while it fills shared memory; 3xTF32 needs the raw values
+  const CUtensorMapDataType in_type =
+      ESZ == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : X3 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32;
   const CUtensorMapDataType res_type = ESZ == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   KMaps maps;
   cuuint32_t box[4] = {(cuuint32_t)C::KC, (cuuint32_t)C::TW, (cuuint32_t)C::TR, 1};
@@ -734,7 +800,8 @@ int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
     }
   }
   KArgs k;
-  k.w = ESZ == 2 ? (const void*)cv.w_umma : (const void*)cv.w_umma32;
+  k.w = ESZ == 2 ? (const void*)cv.w_umma : X3 ? (const void*)cv.w_x3 : (const void*)cv.w_umma32;
+  k.w_lo = X3 ? (const void*)(cv.w_x3 + (size_t)cv.k * cv.k * cv.cin_p * cv.cout_p) : nullptr;      // [W_hi image | W_lo image]
   k.bias = cv.bias;
   k.out = a.out;
   for (int i = 0; i < 3; ++i) {
@@ -758,7 +825,7 @@ int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
   occ = std::max(1, std::min(occ, 2));
   const int gx = std::max(1, std::min(k.total, ttk_num_sms() * occ / nsplit));
   dim3 grid(gx, nsplit);
-  conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF><<<grid, HF ? THREADS_HF : THREADS, C::SMEM_BYTES, st>>>(maps, k);
+  conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3><<<grid, HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, C::SMEM_BYTES, st>>>(maps, k);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }
@@ -791,6 +858,7 @@ int launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a,
   maps.m[2] = maps.m[3] = maps.res = maps.m[0];
   KArgs k;
   k.w = w_dual;
+  k.w_lo = nullptr;
   k.bias = bias_dual;
   k.out = a.out;
   for (int i = 0; i < 3; ++i) {
@@ -841,22 +909,25 @@ void ttk_conv_umma_pack_dual(const float* w3, const float* wd, int esz, std::vec
 //   fused 3x3 stride 1 : [slice][k-chunk][kx][ky][cout_tile][KC]   (B = the three vertical taps side by side)
 //   transition1.0      : [k-chunk][ky][kx][cout][KC]               (B = all nine taps: horizontal + vertical fusion)
 //   otherwise          : [slice][tap][k-chunk][cout_tile][KC]
-// bf16 (w_umma) and TF32-rounded fp32 (w_umma32) images are both kept; they differ in KC and in the slice width of the 128-wide layers.
+// bf16 (w_umma), TF32-rounded fp32 (w_umma32) and 3xTF32 (w_x3: the W_hi = tf32(w) image, then the W_lo = w - W_hi image) are all
+// kept; they differ in KC and in the slice width of the wide layers.
 int ttk_conv_umma_pack(TtkConv& cv, const float* w_host) {
   const int kk = cv.k * cv.k;
-  for (int esz = 2; esz <= 4; esz += 2) {
-    const int KC = kc_of(cv, esz);
+  for (int mode = 0; mode < 3; ++mode) {
+    const int esz = mode == 0 ? 2 : 4;
+    const bool x3 = mode == 2;
+    const int KC = kc_of(cv, esz, x3);
     const int nkc = cv.cin_p / KC;
-    const int ct = cout_tile(cv, esz);
-    const bool fused = fused_ky(cv, esz);
+    const int ct = cout_tile(cv, esz, x3);
+    const bool fused = fused_ky(cv, esz, x3);
     const size_t count = (size_t)kk * cv.cin_p * cv.cout_p;
-    std::vector<uint8_t> w(count * esz, 0);
+    std::vector<uint8_t> w(count * esz * (x3 ? 2 : 1), 0);
     for (int co = 0; co < cv.cout; ++co)
       for (int ci = 0; ci < cv.cin; ++ci)
         for (int t = 0; t < kk; ++t) {
           const int kc = ci / KC, c = ci % KC, sl = co / ct, cl = co % ct;
           size_t row;
-          if (fused_h(cv, esz)) {
+          if (fused_h(cv, esz, x3)) {
             const int ky = t / 3, kx = t % 3;
             row = (((size_t)sl * nkc + kc) * 3 + ky) * 3 + kx;      // [k-chunk][ky][kx][cout]: B of one input row = all nine taps
           } else if (fused) {
@@ -867,19 +938,56 @@ int ttk_conv_umma_pack(TtkConv& cv, const float* w_host) {
           }
           const float v = w_host[((size_t)co * cv.cin + ci) * kk + t];
           const size_t i = (row * ct + cl) * KC + c;
-          if (esz == 2) reinterpret_cast<__nv_bfloat16*>(w.data())[i] = __float2bfloat16_rn(v);
-          else reinterpret_cast<float*>(w.data())[i] = round_tf32(v);
+          if (esz == 2) {
+            reinterpret_cast<__nv_bfloat16*>(w.data())[i] = __float2bfloat16_rn(v);
+          } else {
+            const float hi = round_tf32(v);
+            reinterpret_cast<float*>(w.data())[i] = hi;
+            if (x3) reinterpret_cast<float*>(w.data())[count + i] = v - hi;      // exact
+          }
         }
-    void** dst = esz == 2 ? (void**)&cv.w_umma : (void**)&cv.w_umma32;
+    void** dst = esz == 2 ? (void**)&cv.w_umma : x3 ? (void**)&cv.w_x3 : (void**)&cv.w_umma32;
     if (!*dst) TTK_CUDA(cudaMalloc(dst, w.size()));
     TTK_CUDA(cudaMemcpy(*dst, w.data(), w.size(), cudaMemcpyHostToDevice));
   }
   return TTK_OK;
 }
 
-int ttk_conv_umma_launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st, int esz) {
-  const int ci = cv.cin_p, co = cout_tile(cv, esz);
+int ttk_conv_umma_launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st, int esz, bool x3) {
+  const int ci = cv.cin_p, co = cout_tile(cv, esz, x3);
   const int k = cv.k, s = cv.stride;
+  if (x3) {
+    // ---- 3xTF32: shared memory = 1 KB + 2 planes x (weights + STAGES x box) + bias + barriers (+ 16 KB store staging where it fits) ----
+    // 3x3 boxes of 8 channels: stride 1 (R + 2) x 130 px x 32 B, stride 2 two boxes of (R + 1) x 129 px x 32 B, each 1024-aligned.
+#define TTK_UMMA3(KS_, S_, CI_, CO_, R_, ST_, KC_) \
+  if (k == KS_ && s == S_ && ci == CI_ && co == CO_) return launch<KS_, S_, CI_, CO_, R_, ST_, 0, KC_, 4, 0, 1>(cv, a, st);
+    // 3x3 stride 1 (vertical tap fusion throughout)
+    TTK_UMMA3(3, 1, 16, 64, 4, 2, 8)      // stem conv1: 72 KB weights + 2 x 50 KB stages + 16 KB staging = 190 KB
+    TTK_UMMA3(3, 1, 64, 32, 2, 2, 8)      // stem conv2, quarter-resolution branch (two 32-channel slices): 144 KB + 2 x 34 KB = 213 KB
+    TTK_UMMA3(3, 1, 32, 32, 4, 2, 8)      // half-resolution branch: 72 KB + 2 x 50 KB + 16 KB = 190 KB
+    TTK_UMMA3(3, 1, 16, 16, 8, 2, 8)      // full-resolution branch: 18 KB + 2 x 82 KB = 183 KB
+    TTK_UMMA3(3, 1, 128, 16, 2, 2, 8)     // transition1.0, eighth-resolution branch (eight 16-channel slices): 144 KB + 2 x 34 KB = 213 KB
+    // 3x3 stride 2
+    TTK_UMMA3(3, 2, 16, 16, 2, 3, 8)      // 18 KB + 3 x 52 KB = 175 KB
+    TTK_UMMA3(3, 2, 16, 32, 2, 3, 8)      // 36 KB + 3 x 52 KB = 193 KB
+    TTK_UMMA3(3, 2, 16, 64, 2, 2, 8)      // 72 KB + 2 x 52 KB = 177 KB
+    TTK_UMMA3(3, 2, 16, 128, 1, 2, 8)     // 144 KB + 2 x 36 KB = 218 KB
+    TTK_UMMA3(3, 2, 32, 32, 2, 2, 8)      // 72 KB + 2 x 52 KB = 177 KB
+    TTK_UMMA3(3, 2, 32, 64, 1, 2, 8)      // 32 -> 64 and 32 -> 128 (two slices): 144 KB + 2 x 36 KB = 218 KB
+    TTK_UMMA3(3, 2, 64, 32, 1, 2, 8)      // 64 -> 128 (four slices): 144 KB + 2 x 36 KB = 218 KB
+    TTK_UMMA3(3, 2, 128, 16, 1, 2, 8)     // 128 -> 32 (two slices): 144 KB + 2 x 36 KB = 218 KB
+    // 1x1: 2 x 64 KB per stage of 2 rows x 128 px x 128 B
+    TTK_UMMA3(1, 1, 64, 32, 2, 2, 32)
+    TTK_UMMA3(1, 1, 32, 128, 2, 2, 32)
+    TTK_UMMA3(1, 1, 64, 128, 2, 2, 32)
+    TTK_UMMA3(1, 1, 32, 16, 2, 3, 32)
+    TTK_UMMA3(1, 1, 64, 16, 2, 3, 32)
+    TTK_UMMA3(1, 1, 128, 16, 2, 3, 32)
+    TTK_UMMA3(1, 1, 128, 32, 2, 2, 32)
+    TTK_UMMA3(1, 1, 128, 64, 2, 2, 32)
+#undef TTK_UMMA3
+    return TTK_ERR_UNSUPPORTED;
+  }
   if (esz == 2) {
 #define TTK_UMMA(KS_, S_, CI_, CO_, R_, ST_, RB_) \
   if (k == KS_ && s == S_ && ci == CI_ && co == CO_) return launch<KS_, S_, CI_, CO_, R_, ST_, RB_>(cv, a, st);

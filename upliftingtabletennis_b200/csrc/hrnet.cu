@@ -6,9 +6,11 @@
 // The network is a static plan (ops over NHWC tensors) built once per handle.  Eval-mode batch
 // norm is folded into the conv weights by the host; ReLU, the residual add of a block and the
 // multi-resolution fuse sums (nearest up-sampling = index shift) run in the conv epilogues.
-// Two arithmetic paths share the plan:
-//   TTK_F32  - fp32 SIMT direct convolution (parity with the CPU reference),
-//   TTK_BF16 - bf16 storage, fp32 accumulate, tcgen05 implicit GEMM (conv_umma.cu).
+// The arithmetic paths share the plan:
+//   TTK_F32    - fp32 SIMT direct convolution (parity with the CPU reference),
+//   TTK_TF32   - fp32 storage, tcgen05 implicit GEMM with TF32 operands (conv_umma.cu),
+//   TTK_TF32X3 - fp32 storage, tcgen05 implicit GEMM with three TF32 products of split operands per product (fp32-level results),
+//   TTK_BF16   - bf16 storage, fp32 accumulate, tcgen05 implicit GEMM.
 #include <algorithm>
 #include <map>
 
@@ -561,7 +563,7 @@ int profile_mark(ttk_hrnet* h, int oi, int bs, int H, int W, size_t elem, cudaSt
     r.flops = 2.0 * opix * c.cin * c.cout * c.k * c.k;
     r.bytes = (numel(op.in) + numel(op.out)) * elem + (double)c.cin_p * c.cout_p * c.k * c.k * elem;
     for (int k = 0; k < op.nres; ++k) r.bytes += numel(op.res[k]) * elem;
-    if (h->cur_esz && h->dual_ready && h->use_dual && oi == h->dual_c3_op) {
+    if (h->cur_esz && !h->cur_x3 && h->dual_ready && h->use_dual && oi == h->dual_c3_op) {
       // fused bottleneck tail: the projection shortcut's GEMM rides along and its output tensor never exists
       const TtkOp& ds = h->ops[h->dual_ds_op];
       const TtkConv& dc = h->convs[ds.conv];
@@ -614,17 +616,19 @@ bool is_basic_block(const ttk_hrnet* h, size_t oi) {
   return true;
 }
 
-// esz: 0 = SIMT kernels on T storage, 2 = bf16 tcgen05 path, 4 = TF32 tcgen05 path on fp32 storage
+// esz: 0 = SIMT kernels on T storage, 2 = bf16 tcgen05 path, 4 = TF32 tcgen05 path on fp32 storage (x3: 3xTF32; convolutions only --
+// the fused BasicBlock and bottleneck kernels have no x3 variant, so those convolutions run one by one)
 template <typename T>
-int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, char* ws, int esz, cudaStream_t st) {
+int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, char* ws, int esz, bool x3, cudaStream_t st) {
   const bool umma = esz != 0;
   h->cur_esz = esz;
+  h->cur_x3 = x3;
   bool dual_skipped = false;
   for (size_t oi = 0; oi < h->ops.size(); ++oi) {
     const TtkOp& op = h->ops[oi];
     // TF32: the fused kernels exist (16 channels) and are parity-green, but the thin MMAs of a 16-channel convolution keep them at or
     // above the time of the two HBM-bound convolutions (DESIGN.md section 4.2), so they run only when asked for (use_block_fusion 2 / 3)
-    if (umma && is_basic_block(h, oi) && ((esz == 2 && h->use_block_fusion) || (esz == 4 && h->use_block_fusion >= 2 && h->convs[op.conv].cin_p == 16))) {
+    if (umma && !x3 && is_basic_block(h, oi) && ((esz == 2 && h->use_block_fusion) || (esz == 4 && h->use_block_fusion >= 2 && h->convs[op.conv].cin_p == 16))) {
       const TtkOp& op2 = h->ops[oi + 1];
       const TtkTensor& ti = h->tensors[op.in];
       auto p2 = [&](int t) -> void* { return t == h->input_tensor ? const_cast<void*>(x) : (void*)(ws + h->tensors[t].offset); };
@@ -650,7 +654,7 @@ int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, cha
       if (h->profile) h->recs.pop_back();
     }
     // bottleneck fusion (tensor-core path): the projection shortcut is folded into conv3's GEMM
-    if (umma && h->dual_ready && h->use_dual && (int)oi == h->dual_ds_op) {
+    if (umma && !x3 && h->dual_ready && h->use_dual && (int)oi == h->dual_ds_op) {
       dual_skipped = true;
       continue;
     }
@@ -709,9 +713,13 @@ int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, cha
           rc = ttk_conv_umma_launch(cv, a, st, esz);
         }
       } else if (umma) {
-        rc = ttk_conv_umma_launch(cv, a, st, esz);
+        rc = ttk_conv_umma_launch(cv, a, st, esz, x3);
       }
-      if (rc == TTK_ERR_UNSUPPORTED) rc = launch_conv_simt<T>(cv, a, sizeof(T) == 2, st);
+      if (rc == TTK_ERR_UNSUPPORTED) {
+        // no tensor-core kernel for this shape: the SIMT kernel on the same storage (fp32-level on fp32 tensors)
+        if (umma && h->profile) h->recs.back().simt_fallback = true;
+        rc = launch_conv_simt<T>(cv, a, sizeof(T) == 2, st);
+      }
       if (rc != TTK_OK) return rc;
       h->launches++;
     } else if (op.type == OP_SUM) {
@@ -793,6 +801,7 @@ extern "C" void ttk_hrnet_destroy(ttk_hrnet* h) {
     cudaFree(c.bias);
     cudaFree(c.w_umma);
     cudaFree(c.w_umma32);
+    cudaFree(c.w_x3);
   }
   cudaFree(h->w_dual);
   cudaFree(h->w_dual32);
@@ -872,7 +881,7 @@ extern "C" int ttk_hrnet_forward(ttk_hrnet* h, const void* x_dev, int batch, int
                                  float* heatmaps_dev, void* workspace_dev, size_t workspace_bytes, void* stream) {
   TTK_CHECK_ARG(h, "ttk_hrnet_forward: null handle");
   if (int rc = ttk_bind_device(&h->device, "ttk_hrnet_forward")) return rc;
-  TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_TF32, "ttk_hrnet_forward: bad dtype %d", dtype);
+  TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_TF32 || dtype == TTK_TF32X3, "ttk_hrnet_forward: bad dtype %d", dtype);
   TTK_CHECK_ARG(batch >= 0 && height > 0 && width > 0 && height % 8 == 0 && width % 8 == 0,
                 "ttk_hrnet_forward: height and width must be positive multiples of 8 (got %dx%d)", height, width);
   for (const TtkConv& c : h->convs)
@@ -899,11 +908,11 @@ extern "C" int ttk_hrnet_forward(ttk_hrnet* h, const void* x_dev, int batch, int
     float* heat = heatmaps_dev + (size_t)b0 * h->out_count * height * width;
     int rc;
     if (dtype == TTK_F32)
-      rc = run_plan<float>(h, x, nb, height, width, heat, (char*)workspace_dev, 0, st);
-    else if (dtype == TTK_TF32)
-      rc = run_plan<float>(h, x, nb, height, width, heat, (char*)workspace_dev, h->force_simt ? 0 : 4, st);
+      rc = run_plan<float>(h, x, nb, height, width, heat, (char*)workspace_dev, 0, false, st);
+    else if (dtype == TTK_TF32 || dtype == TTK_TF32X3)
+      rc = run_plan<float>(h, x, nb, height, width, heat, (char*)workspace_dev, h->force_simt ? 0 : 4, dtype == TTK_TF32X3, st);
     else
-      rc = run_plan<__nv_bfloat16>(h, x, nb, height, width, heat, (char*)workspace_dev, h->force_simt ? 0 : 2, st);
+      rc = run_plan<__nv_bfloat16>(h, x, nb, height, width, heat, (char*)workspace_dev, h->force_simt ? 0 : 2, false, st);
     if (rc != TTK_OK) return rc;
   }
   if (h->profile && !h->recs.empty()) TTK_CUDA(cudaEventRecord(h->events[h->recs.size()], st));
@@ -924,7 +933,7 @@ extern "C" int ttk_hrnet_profile_read(ttk_hrnet* h, int i, int* op_type, int* co
   const ttk_hrnet::Rec& r = h->recs[i];
   float t = 0.f;
   TTK_CUDA(cudaEventElapsedTime(&t, h->events[i], h->events[i + 1]));   // caller synchronised the stream
-  if (op_type) *op_type = h->ops[r.op].type;
+  if (op_type) *op_type = r.simt_fallback ? 3 : h->ops[r.op].type;
   if (conv_index) *conv_index = h->ops[r.op].conv;
   if (ms) *ms = t;
   if (flops) *flops = r.flops;
@@ -945,13 +954,14 @@ extern "C" int ttk_hrnet_set_force_simt(ttk_hrnet* h, int enable) {
 }
 
 // Test hook: run ONE convolution of the plan (bias + optional same-shape residual + optional ReLU) on caller buffers.
-// path: 0 = fp32 SIMT (float tensors), 1 = bf16 SIMT, 2 = bf16 tcgen05, 3 = TF32 tcgen05 on float tensors (2 and 3 return
-// TTK_ERR_UNSUPPORTED if the shape has no kernel).
+// path: 0 = fp32 SIMT (float tensors), 1 = bf16 SIMT, 2 = bf16 tcgen05, 3 = TF32 tcgen05 on float tensors, 4 = 3xTF32 tcgen05 on
+// float tensors (2 to 4 return TTK_ERR_UNSUPPORTED if the shape has no kernel).
 extern "C" int ttk_hrnet_debug_conv(ttk_hrnet* h, int conv_index, const void* in_dev, int n, int hin, int win, const void* res_dev,
                                     int relu, int path, void* out_dev, void* stream) {
   TTK_CHECK_ARG(h && conv_index >= 0 && conv_index < (int)h->convs.size() - 1, "ttk_hrnet_debug_conv: bad conv index %d", conv_index);
   const TtkConv& cv = h->convs[conv_index];
   TTK_CHECK_ARG(cv.set, "ttk_hrnet_debug_conv: weights not set");
+  TTK_CHECK_ARG(path >= 0 && path <= 4, "ttk_hrnet_debug_conv: bad path %d", path);
   ConvLaunch a;
   a.in = in_dev;
   a.out = out_dev;
@@ -971,7 +981,7 @@ extern "C" int ttk_hrnet_debug_conv(ttk_hrnet* h, int conv_index, const void* in
   cudaStream_t st = (cudaStream_t)stream;
   if (path == 0) return launch_conv_simt<float>(cv, a, false, st);
   if (path == 1) return launch_conv_simt<__nv_bfloat16>(cv, a, true, st);
-  return ttk_conv_umma_launch(cv, a, st, path == 3 ? 4 : 2);
+  return ttk_conv_umma_launch(cv, a, st, path == 2 ? 2 : 4, path == 4);
 }
 
 // Test hook: one BasicBlock (conv_index = its conv1, conv_index + 1 = its conv2) through the fused tcgen05 kernel on caller buffers:

@@ -17,6 +17,7 @@ struct TtkConv {
   float* bias = nullptr;        // device, [cout_p] float32
   __nv_bfloat16* w_umma = nullptr;  // device, tcgen05 B-operand image, bf16 (see ttk_conv_umma_pack)
   float* w_umma32 = nullptr;        // device, tcgen05 B-operand image for kind::tf32: fp32 containers, values rounded to TF32
+  float* w_x3 = nullptr;            // device, 3xTF32 B-operand images: W_hi = tf32(w), then W_lo = w - W_hi, in the x3 layout
   std::vector<float> w_host, b_host; // folded weights as set by the host (used to build fused variants)
 };
 
@@ -73,20 +74,21 @@ struct ttk_hrnet {
   bool dual_ready = false;
   int use_dual = 1;
   int cur_esz = 0;              // element size of the tensor-core path the running forward uses (0: SIMT), for the profile records
+  bool cur_x3 = false;          // ... and whether it is the 3xTF32 path
   int use_block_fusion = 1;     // BasicBlocks as one kernel (block_umma.cu): the 16- and 32-channel branches in bf16, the 16-channel branch
                                 // in TF32.  Round 1 measured break-even in bf16 because the thin MMAs were issue bound (16 instructions per
                                 // tcgen05.mma); with the warp-uniform issue loop the fused blocks win (DESIGN.md section 4.2)
   // optional per-launch timing (ttk_hrnet_set_profile): events bracket every launch on the caller's stream
   int profile = 0;
   std::vector<cudaEvent_t> events;     // pool, events[i] precedes launch i
-  struct Rec { int op; int n; double flops, bytes; };
+  struct Rec { int op; int n; double flops, bytes; bool simt_fallback = false; };
   std::vector<Rec> recs;
 };
 
 // conv_umma.cu: implicit-GEMM convolution on tcgen05/TMEM fed by TMA.  esz = bytes per activation element: 2 = bf16 (kind::f16),
-// 4 = fp32 activations multiplied as TF32 (kind::tf32).
+// 4 = fp32 activations multiplied as TF32 (kind::tf32); x3 (esz 4 only): every product as three TF32 products of split operands.
 // Returns TTK_ERR_UNSUPPORTED when the shape has no tensor-core kernel (caller falls back to SIMT on the same storage type).
-int ttk_conv_umma_launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st, int esz = 2);
+int ttk_conv_umma_launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st, int esz = 2, bool x3 = false);
 int ttk_conv_umma_pack(TtkConv& cv, const float* w_host);
 // out = relu(W3 a + Wd x + bias): a.in = a (32 ch), a.in2 = x (64 ch); returns TTK_ERR_UNSUPPORTED if the driver rejects the maps
 int ttk_conv_umma_launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a, cudaStream_t st, int esz = 2);

@@ -12,7 +12,7 @@ import torch.nn as nn
 
 from . import _lib
 from ._lib import lib, check, ptr, stream_ptr
-from .precision import PrecisionMixin, TF32, FP32, BF16, lib_enum, storage_dtype
+from .precision import PrecisionMixin, TF32, TF32X3, FP32, BF16, lib_enum, storage_dtype
 
 BN_EPS = 1e-5
 
@@ -74,7 +74,7 @@ class HRNetEngine:
 
     def forward_nhwc16(self, x, out=None, precision=None):
         """x: (B, H, W, 16) float32 or bfloat16 CUDA tensor -> (B, out_count, H, W) float32.
-        precision: 'tf32' / 'fp32' for float32 tensors (default 'fp32': the strict SIMT path), 'bf16' for bfloat16 tensors."""
+        precision: 'tf32' / 'tf32x3' / 'fp32' for float32 tensors (default 'fp32': the strict SIMT path), 'bf16' for bfloat16 tensors."""
         assert self.loaded, 'weights not loaded'
         assert x.is_cuda and x.dim() == 4 and x.shape[3] == 16 and x.is_contiguous()
         B, H, W, _ = x.shape
@@ -111,9 +111,11 @@ def _attach(root, key, tensor, is_param):
 class _HRNetModule(PrecisionMixin, nn.Module):
     """nn.Module shell: holds the reference-named tensors, folds them into the engine lazily.
     ``compute_dtype`` (constructor argument ``dtype``): 'tf32' (default: tcgen05 tensor cores at the precision class of the
-    reference's cuDNN convolutions), 'fp32' (SIMT, strict parity), 'bf16' (tcgen05, bf16 storage)."""
+    reference's cuDNN convolutions), 'tf32x3' (tcgen05 tensor cores, three TF32 products of split operands per product: fp32-level
+    results, the class of the reference on a CPU or with cuDNN's TF32 off), 'fp32' (SIMT, strict parity), 'bf16' (tcgen05, bf16
+    storage)."""
     default_precision = TF32
-    supported_precisions = (TF32, FP32, BF16)
+    supported_precisions = (TF32, TF32X3, FP32, BF16)
 
     def __init__(self, in_ch, out_ch, out_first, out_count, dtype=None):
         super().__init__()

@@ -98,7 +98,7 @@ def _check_model_name(model_name, available):
 
 
 def load_ball_model(model_path, dtype=None):
-    """inference/inference_balldetection.py:40-61.  dtype: arithmetic class ('tf32' / 'fp32' / 'bf16', see precision.py);
+    """inference/inference_balldetection.py:40-61.  dtype: arithmetic class ('tf32' / 'tf32x3' / 'fp32' / 'bf16', see precision.py);
     None = the architecture's default."""
     load_dict = torch.load(model_path, map_location=torch.device('cpu'), weights_only=False)
     info = load_dict['additional_info']
@@ -462,7 +462,7 @@ class BallDetector(_Detector):
     frames_per_stack = 3
 
     def __init__(self, model_name='segformerpp_b2', dtype=None):
-        """dtype: 'tf32' / 'fp32' / 'bf16' (precision.py); None = the architecture's default tensor-core path."""
+        """dtype: 'tf32' / 'tf32x3' / 'fp32' / 'bf16' (precision.py); None = the architecture's default tensor-core path."""
         _check_model_name(model_name, BALL_MODELS)
         self.device = _device()
         self.resolution = (WIDTH, HEIGHT)
