@@ -18,7 +18,8 @@ def ball_detection(model_name='segformerpp_b2', dtype=None, **kwargs):
     """Loads the Ball Detection Model.  B200 kernels exist for 'wasb' and 'vitpose'; the reference's default name is kept, but
     segformer++ is not part of the reference repository and raises NotImplementedError before anything is downloaded.
     dtype: 'tf32' (WASB default: tensor cores at the precision class of the reference's cuDNN convolutions), 'tf32x3' (ViTPose
-    default, WASB on request: float32-class results on the tensor cores), 'fp32' (SIMT), 'bf16'."""
+    default, WASB on request: float32-class results on the tensor cores), 'fp32' (SIMT), 'bf16', 'fp16' (WASB / HRNet only: the bf16 kernels
+    with fp16 storage)."""
     return BallDetector(model_name=model_name, dtype=dtype)
 
 

@@ -30,8 +30,11 @@ enum { TTK_OK = 0, TTK_ERR_ARG = -1, TTK_ERR_CUDA = -2, TTK_ERR_STATE = -3, TTK_
 /* Arithmetic / storage type of a path.  TTK_TF32: fp32 storage, tensor-core products with TF32 operands (inputs rounded to
  * nearest-even TF32 by TMA, fp32 accumulate) -- the class cuDNN uses for the reference's convolutions on a GPU.
  * TTK_TF32X3 (uplifting transformer, ViTPose, HRNet): fp32 storage, every product as three TF32 tensor-core products of split operands
- * (a_hi b_hi + a_lo b_hi + a_hi b_lo) -- fp32-level results, the class of the reference's fp32 Linear layers. */
-enum { TTK_F32 = 0, TTK_BF16 = 1, TTK_TF32 = 2, TTK_TF32X3 = 3 };
+ * (a_hi b_hi + a_lo b_hi + a_hi b_lo) -- fp32-level results, the class of the reference's fp32 Linear layers.
+ * TTK_F16 (HRNet and pre-processing only): IEEE fp16 storage and tensor-core operands, fp32 accumulate -- the tiles and kernels of
+ * TTK_BF16 with 10 mantissa bits instead of 7, the class of torch.autocast('cuda') / model.half().  Its range is +-65504: an activation
+ * past it becomes inf, as under autocast; the library does not rescale. */
+enum { TTK_F32 = 0, TTK_BF16 = 1, TTK_TF32 = 2, TTK_TF32X3 = 3, TTK_F16 = 4 };
 enum { TTK_DECODE_TABLE = 0, TTK_DECODE_BALL = 1 }; /* the two live sub-pixel variants */
 enum { TTK_LAYOUT_NCHW_F32 = 0, TTK_LAYOUT_NHWC16 = 1 };
 
@@ -55,8 +58,8 @@ TTK_API int ttk_device_ok(void);
  *              hub API).  Stack s reads frames s*stack_stride + {0..frames_per_stack-1}.
  * lut_dev    : 3 x 256 float32, lut[c][v] = float32((v/255 - mean[c]) / std[c]) (host float64).
  * out_dev    : layout NCHW_F32: n_stacks x (3*fps) x dst_h x dst_w float32 (the reference tensor)
- *              layout NHWC16  : n_stacks x dst_h x dst_w x 16, dtype f32 or bf16, channels
- *              3*fps..15 zero -- the detector input.
+ *              layout NHWC16  : n_stacks x dst_h x dst_w x 16, dtype f32, bf16 or f16 (the float32
+ *              value rounded to nearest-even), channels 3*fps..15 zero -- the detector input.
  */
 TTK_API int ttk_preprocess_stacks(const uint8_t* frames_dev, int n_frames, int src_h, int src_w,
                           int frames_per_stack, int stack_stride, int n_stacks,
@@ -91,8 +94,9 @@ TTK_API size_t ttk_hrnet_workspace_bytes(const ttk_hrnet* h, int batch, int heig
  * tcgen05 tensor cores with TF32 operands (the reference-on-GPU class, balldetection/models/wasb.py:29-105
  * through cuDNN's default TF32); TTK_TF32X3: float32 tensors as for TTK_TF32, every product as three TF32 tensor-core products of
  * split operands (fp32-level results: the reference on a CPU, or on a GPU with cudnn.allow_tf32 off; no fused BasicBlock or bottleneck
- * kernels); TTK_BF16: tcgen05 path with bf16 storage, fp32 accumulate.  A convolution without a tensor-core kernel for its shape runs
- * on the SIMT kernel of the same storage type. */
+ * kernels); TTK_BF16: tcgen05 path with bf16 storage, fp32 accumulate; TTK_F16: the same kernels with fp16 storage and operands (x and
+ * every activation fp16, heatmaps float32).  A convolution without a tensor-core kernel for its shape runs on the SIMT kernel of the same
+ * storage type. */
 TTK_API int ttk_hrnet_forward(ttk_hrnet* h, const void* x_dev, int batch, int height, int width, int dtype,
                       float* heatmaps_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 /* kernels launched by the last ttk_hrnet_forward on this handle (for bench accounting) */
@@ -106,12 +110,16 @@ TTK_API int ttk_hrnet_set_subbatch(ttk_hrnet* h, int images);
  * no tensor-core kernel), conv index (-1 if none), duration in ms,
  * algorithmic flops (2*MAC on the reference's logical channel counts) and compulsory bytes
  * (inputs + outputs + weights once). */
-TTK_API int ttk_hrnet_set_force_simt(ttk_hrnet* h, int enable);   /* bf16 path through the SIMT kernels (cross-check of the tcgen05 path) */
+TTK_API int ttk_hrnet_set_force_simt(ttk_hrnet* h, int enable);   /* tensor-core paths through the SIMT kernels of their storage type (cross-check) */
 /* Test hook: run one convolution of the plan on caller buffers (NHWC, channels padded to 16): out = act(conv(in) + bias [+ res]).
  * path 0: fp32 SIMT (float32 tensors), 1: bf16 SIMT, 2: bf16 tcgen05, 3: TF32 tcgen05 on float32 tensors, 4: 3xTF32 tcgen05 on
  * float32 tensors (2 to 4 return TTK_ERR_UNSUPPORTED when the shape has no tensor-core kernel; any other path is TTK_ERR_ARG). */
 TTK_API int ttk_hrnet_debug_conv(ttk_hrnet* h, int conv_index, const void* in_dev, int n, int hin, int win, const void* res_dev,
                          int relu, int path, void* out_dev, void* stream);
+/* Test hook: the same on fp16 tensors (fp16-rounded weights): simt 1 = fp16 SIMT kernel, 0 = fp16 tcgen05 kernel
+ * (TTK_ERR_UNSUPPORTED when the shape has none). */
+TTK_API int ttk_hrnet_debug_conv_f16(ttk_hrnet* h, int conv_index, const void* in_dev, int n, int hin, int win, const void* res_dev,
+                             int relu, int simt, void* out_dev, void* stream);
 /* Test hook: one BasicBlock (convs conv_index and conv_index + 1, 16 or 32 padded channels) through the fused tcgen05 kernel:
  * out = relu(conv2(relu(conv1(in))) + in), NHWC bf16.  ttk_hrnet_set_block_fusion: 0 runs the blocks conv by conv (A/B, cross-check),
  * 1 (default) fuses the bf16 blocks of the 16- and 32-channel branches, 2 / 3 also the TF32 16-channel blocks (two 3-row tiles in flight

@@ -6,7 +6,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'libttk.so')
 
-F32, BF16, TF32, TF32X3 = 0, 1, 2, 3
+F32, BF16, TF32, TF32X3, F16 = 0, 1, 2, 3, 4
 DECODE_TABLE, DECODE_BALL = 0, 1
 LAYOUT_NCHW_F32, LAYOUT_NHWC16 = 0, 1
 
@@ -42,6 +42,7 @@ def _load():
         'ttk_hrnet_set_profile': (i32, [vp, i32]),
         'ttk_hrnet_set_force_simt': (i32, [vp, i32]),
         'ttk_hrnet_debug_conv': (i32, [vp, i32, vp, i32, i32, i32, vp, i32, i32, vp, vp]),
+        'ttk_hrnet_debug_conv_f16': (i32, [vp, i32, vp, i32, i32, i32, vp, i32, i32, vp, vp]),
         'ttk_hrnet_debug_block': (i32, [vp, i32, vp, i32, i32, i32, vp, vp]),
         'ttk_hrnet_set_block_fusion': (i32, [vp, i32]),
         'ttk_hrnet_profile_count': (i32, [vp]),

@@ -1,4 +1,4 @@
-// Fused BasicBlock of the HRNet branches on tcgen05 (bf16: 16- and 32-channel branches; TF32 on fp32 activations: the 16-channel
+// Fused BasicBlock of the HRNet branches on tcgen05 (bf16 / fp16: 16- and 32-channel branches; TF32 on fp32 activations: the 16-channel
 // full-resolution branch, whose two convolutions are HBM bound on their own -- 320 bytes per pixel conv by conv, 128 fused):
 //   y = relu(conv2(relu(conv1(x) + b1)) + b2 + x)              balldetection/models/wasb.py:35-64 (BasicBlock.forward, BN folded)
 // The two 3x3 convolutions of a block run in ONE kernel: the intermediate tensor never leaves the SM and the residual is taken
@@ -8,7 +8,7 @@
 // Tile = R output rows x 126 output pixels.  One TMA box brings the (R+4) x 130 pixel input halo (zero fill outside the image).
 //   M1: conv1 on tensor cores for the (R+2) x 128 intermediate pixels the tile needs (vertical tap fusion as in conv_umma.cu:
 //       one MMA per input row and horizontal tap against [W(ky=0) | W(ky=1) | W(ky=2)], accumulators in reverse row order)
-//   E1: accumulators -> + b1, ReLU, zero outside the image (conv2 pads the intermediate TENSOR with zeros) -> bf16 -> shared
+//   E1: accumulators -> + b1, ReLU, zero outside the image (conv2 pads the intermediate TENSOR with zeros) -> bf16 / fp16 -> shared
 //       memory in the same swizzled pixel-row layout TMA produces, so conv2 addresses it with the same descriptors
 //   M2: conv2 from that tile,  E2: + b2 + x (from the staged input tile) -> ReLU -> global.
 // Roles (persistent CTA): warp 0 TMA producer (input ring), warp 1 MMA issuer, warps 2-5 / 6-9 the epilogue groups of slot 0 / 1.
@@ -61,7 +61,7 @@ struct BlockArgs {
 
 // RR output rows from RR + 2 staged rows at `abase`, weights at `wbase`, accumulators at `d_acc` (row yo in column block RR-1-yo).
 // Called by the whole MMA warp with warp-uniform arguments; the elected lane issues (see conv_umma.cu).
-template <int C, int RR, uint32_t LAYOUT, int ESZ>
+template <int C, int RR, uint32_t LAYOUT, int ESZ, int H>
 __device__ __forceinline__ void issue_conv(uint32_t abase, uint32_t wbase, uint32_t d_acc, bool leader) {
   constexpr int ROWB = ESZ * C;
   constexpr uint32_t RB16 = ROWB / 16;
@@ -71,7 +71,7 @@ __device__ __forceinline__ void issue_conv(uint32_t abase, uint32_t wbase, uint3
     const int yi = hr - 1;
     const int k0 = yi + 2 - RR > 0 ? yi + 2 - RR : 0;
     const int k1 = yi + 1 < 2 ? yi + 1 : 2;
-    const uint32_t idesc = ESZ == 2 ? make_idesc(128, (k1 - k0 + 1) * C) : make_idesc_tf32(128, (k1 - k0 + 1) * C);
+    const uint32_t idesc = ESZ == 2 ? make_idesc(128, (k1 - k0 + 1) * C, 0, H) : make_idesc_tf32(128, (k1 - k0 + 1) * C);
     const uint32_t d = d_acc + (RR - 2 - yi + k0) * C;
 #pragma unroll
     for (int kx = 0; kx < 3; ++kx) {
@@ -89,10 +89,12 @@ __device__ __forceinline__ void issue_conv(uint32_t abase, uint32_t wbase, uint3
 
 // Tiles of a CTA are numbered t = 0, 1, 2, ... in the order it takes them; tile t lives in input buffer t % NX and in slot t % SLOTS
 // (slot = its own accumulators and intermediate tile, served by its own group of four epilogue warps), so with two slots the MMAs of
-// one tile run under the epilogues of the other.
-template <int C, int R, int SLOTS, int ESZ = 2, int GRES = 0>
+// one tile run under the epilogues of the other.  H: the 16-bit format (0 bf16, 1 fp16; umma_prims.h: Fmt16).
+template <int C, int R, int SLOTS, int ESZ = 2, int GRES = 0, int H = 0>
 __global__ void __launch_bounds__(THREADS, 1) block_umma_kernel(const __grid_constant__ CUtensorMap xmap, const BlockArgs a) {
   using K = BCfg<C, R, SLOTS, ESZ, GRES>;
+  using F = Fmt16<H>;
+  static_assert(!H || ESZ == 2, "fp16 is a 16-bit element format");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* sW1 = smem;
@@ -174,7 +176,7 @@ __global__ void __launch_bounds__(THREADS, 1) block_umma_kernel(const __grid_con
             const uint32_t s = t % K::NX;
             if (!mbar_test(bar_xfull + 8 * s, (t / K::NX) & 1)) continue;
             fence_after();
-            issue_conv<C, K::R1, K::LAYOUT, ESZ>(smem_u32(sX + s * K::X_AL), smem_u32(sW1), acc1, leader);
+            issue_conv<C, K::R1, K::LAYOUT, ESZ, H>(smem_u32(sX + s * K::X_AL), smem_u32(sW1), acc1, leader);
             if (leader) commit(bar_m1 + 8 * k);
             if (GRES && leader) commit(bar_xempty + 8 * s);      // nothing else reads the input tile
             __syncwarp();
@@ -182,7 +184,7 @@ __global__ void __launch_bounds__(THREADS, 1) block_umma_kernel(const __grid_con
           } else {
             if (!mbar_test(bar_st + 8 * k, (t / SLOTS) & 1)) continue;       // intermediate tile written (and acc1 zeroed again)
             fence_after();
-            issue_conv<C, R, K::LAYOUT, ESZ>(smem_u32(sT + k * K::T_AL), smem_u32(sW2), acc2, leader);
+            issue_conv<C, R, K::LAYOUT, ESZ, H>(smem_u32(sT + k * K::T_AL), smem_u32(sW2), acc2, leader);
             if (leader) commit(bar_m2 + 8 * k);
             __syncwarp();
             stage[k] = 0;
@@ -254,8 +256,7 @@ __global__ void __launch_bounds__(THREADS, 1) block_umma_kernel(const __grid_con
               for (int j = 0; j < C / 2; ++j) {
                 const float f0 = inside ? fmaxf(__uint_as_float(v[g][2 * j]) + sB1[2 * j], 0.f) : 0.f;
                 const float f1 = inside ? fmaxf(__uint_as_float(v[g][2 * j + 1]) + sB1[2 * j + 1], 0.f) : 0.f;
-                __nv_bfloat162 b2 = __floats2bfloat162_rn(f0, f1);
-                pk[j] = *reinterpret_cast<uint32_t*>(&b2);
+                pk[j] = F::pack(f0, f1);
               }
             } else {
               // the intermediate is an operand of kind::tf32, which truncates: round it here (to nearest; the integer form of
@@ -336,10 +337,9 @@ __global__ void __launch_bounds__(THREADS, 1) block_umma_kernel(const __grid_con
             if (ESZ == 2) {
 #pragma unroll
               for (int j = 0; j < C / 2; ++j) {
-                const float f0 = fmaxf(__uint_as_float(v[g][2 * j]) + sB2[2 * j] + __uint_as_float(rv[g][j] << 16), 0.f);
-                const float f1 = fmaxf(__uint_as_float(v[g][2 * j + 1]) + sB2[2 * j + 1] + __uint_as_float(rv[g][j] & 0xffff0000u), 0.f);
-                __nv_bfloat162 b2 = __floats2bfloat162_rn(f0, f1);
-                o[j] = *reinterpret_cast<uint32_t*>(&b2);
+                const float f0 = fmaxf(__uint_as_float(v[g][2 * j]) + sB2[2 * j] + F::lo(rv[g][j]), 0.f);
+                const float f1 = fmaxf(__uint_as_float(v[g][2 * j + 1]) + sB2[2 * j + 1] + F::hi(rv[g][j]), 0.f);
+                o[j] = F::pack(f0, f1);
               }
             } else {
               // the residual is the staged input tile, i.e. x as TMA rounded it to TF32 (2^-12 relative: inside the path's class)
@@ -363,7 +363,7 @@ __global__ void __launch_bounds__(THREADS, 1) block_umma_kernel(const __grid_con
   if (warp == 2) tmem_dealloc(tmem, K::TMEM_COLS);
 }
 
-template <int C, int R, int SLOTS, int ESZ = 2, int GRES = 0>
+template <int C, int R, int SLOTS, int ESZ = 2, int GRES = 0, int H = 0>
 int launch(const TtkConv& c1, const TtkConv& c2, const void* x, void* y, int n, int h, int w, cudaStream_t st) {
   using K = BCfg<C, R, SLOTS, ESZ, GRES>;
   EncodeFn encode = get_encode();
@@ -373,43 +373,44 @@ int launch(const TtkConv& c1, const TtkConv& c2, const void* x, void* y, int n, 
   }
   static TtkPerDevice attr;
   if (attr.first()) {
-    TTK_CUDA(cudaFuncSetAttribute(block_umma_kernel<C, R, SLOTS, ESZ, GRES>, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM_BYTES));
+    TTK_CUDA(cudaFuncSetAttribute(block_umma_kernel<C, R, SLOTS, ESZ, GRES, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, K::SMEM_BYTES));
   }
   CUtensorMap map;
   cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
   cuuint64_t strides[3] = {(cuuint64_t)C * ESZ, (cuuint64_t)w * C * ESZ, (cuuint64_t)h * w * C * ESZ};
   cuuint32_t box[4] = {(cuuint32_t)C, (cuuint32_t)TW, (cuuint32_t)K::RX, 1};
   cuuint32_t es[4] = {1, 1, 1, 1};
-  if (encode(&map, ESZ == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 4, const_cast<void*>(x), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+  if (encode(&map, ESZ == 2 ? Fmt16<H>::MAP : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 4, const_cast<void*>(x), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
              K::ROWB == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) {
     ttk_set_error("cuTensorMapEncodeTiled failed for the fused block %s", c1.name.c_str());
     return TTK_ERR_CUDA;
   }
   BlockArgs a;
-  a.w1 = ESZ == 2 ? (const void*)c1.w_umma : (const void*)c1.w_umma32, a.w2 = ESZ == 2 ? (const void*)c2.w_umma : (const void*)c2.w_umma32;
+  if (ESZ == 2 && H) a.w1 = c1.w_umma_f16, a.w2 = c2.w_umma_f16;
+  else a.w1 = ESZ == 2 ? (const void*)c1.w_umma : (const void*)c1.w_umma32, a.w2 = ESZ == 2 ? (const void*)c2.w_umma : (const void*)c2.w_umma32;
   a.b1 = c1.bias, a.b2 = c2.bias, a.x = x, a.out = y;
   a.n = n, a.h = h, a.w = w;
   a.tiles_x = ttk_cdiv(w, WO), a.tiles_y = ttk_cdiv(h, R);
   a.total = a.tiles_x * a.tiles_y * n;
   const int grid = std::max(1, std::min(a.total, ttk_num_sms()));
-  block_umma_kernel<C, R, SLOTS, ESZ, GRES><<<grid, THREADS, K::SMEM_BYTES, st>>>(map, a);
+  block_umma_kernel<C, R, SLOTS, ESZ, GRES, H><<<grid, THREADS, K::SMEM_BYTES, st>>>(map, a);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }
 
 }  // namespace
 
-// y = relu(conv2(relu(conv1(x))) + x) for two 3x3 stride-1 convolutions with cin = cout = 16 or 32 (padded), NHWC bf16 (esz 2) or, for 16
-// channels, NHWC fp32 multiplied as TF32 (esz 4).
-int ttk_block_umma_launch(const TtkConv& c1, const TtkConv& c2, const void* x, void* y, int n, int h, int w, cudaStream_t st, int esz) {
+// y = relu(conv2(relu(conv1(x))) + x) for two 3x3 stride-1 convolutions with cin = cout = 16 or 32 (padded), NHWC bf16 (esz 2; f16: fp16)
+// or, for 16 channels, NHWC fp32 multiplied as TF32 (esz 4).
+int ttk_block_umma_launch(const TtkConv& c1, const TtkConv& c2, const void* x, void* y, int n, int h, int w, cudaStream_t st, int esz, bool f16) {
   if (c1.k != 3 || c2.k != 3 || c1.stride != 1 || c2.stride != 1 || c1.cin_p != c1.cout_p || c2.cin_p != c1.cin_p || c2.cout_p != c1.cin_p)
     return TTK_ERR_UNSUPPORTED;
   // TF32 (64-byte rows): two 3-row tiles in flight with the fp32 residual from global memory (esz 4), or one 4-row tile with the residual
   // from the staged tile (esz 5: the first version, kept for comparison)
   if (esz == 4) return c1.cin_p == 16 ? launch<16, 3, 2, 4, 1>(c1, c2, x, y, n, h, w, st) : TTK_ERR_UNSUPPORTED;
   if (esz == 5) return c1.cin_p == 16 ? launch<16, 4, 1, 4, 0>(c1, c2, x, y, n, h, w, st) : TTK_ERR_UNSUPPORTED;
-  if (c1.cin_p == 16) return launch<16, 6, 2>(c1, c2, x, y, n, h, w, st);      // two tiles in flight (2 x 224 TMEM columns)
-  if (c1.cin_p == 32) return launch<32, 4, 1>(c1, c2, x, y, n, h, w, st);      // 320 TMEM columns per tile: one slot
+  if (c1.cin_p == 16) return f16 ? launch<16, 6, 2, 2, 0, 1>(c1, c2, x, y, n, h, w, st) : launch<16, 6, 2>(c1, c2, x, y, n, h, w, st);      // two tiles in flight (2 x 224 TMEM columns)
+  if (c1.cin_p == 32) return f16 ? launch<32, 4, 1, 2, 0, 1>(c1, c2, x, y, n, h, w, st) : launch<32, 4, 1>(c1, c2, x, y, n, h, w, st);      // 320 TMEM columns per tile: one slot
   return TTK_ERR_UNSUPPORTED;
 }

@@ -1,7 +1,8 @@
 // Implicit-GEMM convolution (3x3 stride 1/2, 1x1) on the 5th-generation tensor cores:
 // tcgen05.mma with TMEM accumulators, operands staged by TMA, fused bias / residual / ReLU epilogue.
 // Two arithmetic classes share the kernel (template parameter ESZ = bytes per activation element):
-//   ESZ 2: bf16 activations and weights, kind::f16;
+//   ESZ 2: 16-bit activations and weights, kind::f16: bf16, or IEEE fp16 with template parameter H = 1 (umma_prims.h: Fmt16 holds
+//          everything that differs between the two; tiles, dispatch and fusion are the same);
 //   ESZ 4: fp32 activations in HBM, kind::tf32 -- the class cuDNN uses for the reference's convolutions on a GPU (torch enables
 //          TF32 for cuDNN by default).  The tensor map of the input has data type TFLOAT32, so TMA rounds every element to TF32
 //          (nearest-even) on its way into shared memory; the weights are rounded once on the host; kind::tf32 ignores the low 13
@@ -147,10 +148,12 @@ struct KArgs {
   int tiles_x, tiles_y, total;
 };
 
-template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0, int X3 = 0>
+template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0, int X3 = 0, int H = 0>
 __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1) conv_umma_kernel(const __grid_constant__ KMaps maps, const KArgs a) {
   constexpr int NTHR = HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS;
   using C = Cfg<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3>;
+  using F = Fmt16<H>;                                   // ESZ 2: bf16 (H 0) or fp16 (H 1)
+  static_assert(!H || (ESZ == 2 && !X3), "fp16 is a 16-bit element format");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* sW = smem;
@@ -285,7 +288,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1
               const int yi = hr - 1;
               const int k0 = yi + 2 - R > 0 ? yi + 2 - R : 0;
               const int k1 = yi + 1 < 2 ? yi + 1 : 2;
-              const uint32_t idesc = ESZ == 2 ? make_idesc(128, (k1 - k0 + 1) * 3 * COUT) : make_idesc_tf32(128, (k1 - k0 + 1) * 3 * COUT);
+              const uint32_t idesc = ESZ == 2 ? make_idesc(128, (k1 - k0 + 1) * 3 * COUT, 0, H) : make_idesc_tf32(128, (k1 - k0 + 1) * 3 * COUT);
               const uint32_t d_tmem = d_acc + (R - 2 - yi + k0) * 3 * COUT;
               const uint32_t arow = abase + hr * C::TW * RB16;
               const uint32_t brow = wbase + ((kc * 3 + k0) * 3 * COUT) * RB16;
@@ -300,7 +303,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1
               const int yi = hr - 1;
               const int k0 = yi + 2 - R > 0 ? yi + 2 - R : 0;
               const int k1 = yi + 1 < 2 ? yi + 1 : 2;
-              const uint32_t idesc = ESZ == 2 ? make_idesc(128, (k1 - k0 + 1) * COUT) : make_idesc_tf32(128, (k1 - k0 + 1) * COUT);
+              const uint32_t idesc = ESZ == 2 ? make_idesc(128, (k1 - k0 + 1) * COUT, 0, H) : make_idesc_tf32(128, (k1 - k0 + 1) * COUT);
               const uint32_t d_tmem = d_acc + (R - 2 - yi + k0) * COUT;
 #pragma unroll
               for (int kx = 0; kx < 3; ++kx) {
@@ -312,7 +315,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1
               }
             }
           } else {
-            constexpr uint32_t idesc = ESZ == 2 ? make_idesc(128, COUT) : make_idesc_tf32(128, COUT);
+            constexpr uint32_t idesc = ESZ == 2 ? make_idesc(128, COUT, 0, H) : make_idesc_tf32(128, COUT);
 #pragma unroll 1
             for (int r = 0; r < R; ++r) {
               const uint32_t d_tmem = d_acc + (R - 1 - r) * COUT;
@@ -389,13 +392,13 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1
       mbar_arrive(bar_tempty);
       mbar_arrive(bar_tempty + 8);
     }
-    // f += the 16 channels held in w: bf16 pairs are widened by bit placement (keeps the conversion pipe free)
+    // f += the 16 channels held in w (16-bit pairs widened by Fmt16: bf16 by bit placement, fp16 converted)
     auto add_words = [](float* f, const uint32_t* w) {
       if (ESZ == 2) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
-          f[2 * j] += __uint_as_float(w[j] << 16);
-          f[2 * j + 1] += __uint_as_float(w[j] & 0xffff0000u);
+          f[2 * j] += F::lo(w[j]);
+          f[2 * j + 1] += F::hi(w[j]);
         }
       } else {
 #pragma unroll
@@ -474,10 +477,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1
             if (ESZ == 2) {
               uint32_t o[8];
 #pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                __nv_bfloat162 b2 = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
-                o[j] = *reinterpret_cast<uint32_t*>(&b2);
-              }
+              for (int j = 0; j < 8; ++j) o[j] = F::pack(f[2 * j], f[2 * j + 1]);
               stg256(op, o);
             } else {
               uint32_t o[16];
@@ -582,10 +582,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1
             if (ESZ == 2) {
               uint32_t o[8];
 #pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                __nv_bfloat162 b2 = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
-                o[j] = *reinterpret_cast<uint32_t*>(&b2);
-              }
+              for (int j = 0; j < 8; ++j) o[j] = F::pack(f[2 * j], f[2 * j + 1]);
               stg256(op, o);
             } else {
               uint32_t o[16];
@@ -672,10 +669,7 @@ __global__ void __launch_bounds__(HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, 1
           if (ESZ == 2) {
             uint32_t o[8];
 #pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              __nv_bfloat162 b2 = __floats2bfloat162_rn(f[2 * j], f[2 * j + 1]);
-              o[j] = *reinterpret_cast<uint32_t*>(&b2);
-            }
+            for (int j = 0; j < 8; ++j) o[j] = F::pack(f[2 * j], f[2 * j + 1]);
             stg256(op, o);
           } else {
             uint32_t o[16];
@@ -747,7 +741,7 @@ float round_tf32(float v) {      // nearest-even on the 13 dropped mantissa bits
   return v;
 }
 
-template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0, int X3 = 0>
+template <int KS, int S, int CIN, int COUT, int R, int STAGES, int RB, int KCO = 0, int ESZ = 2, int HF = 0, int X3 = 0, int H = 0>
 int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
   using C = Cfg<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3>;
   if (C::KC != kc_of(cv, ESZ, X3) || COUT != cout_tile(cv, ESZ, X3) || (HF != 0) != fused_h(cv, ESZ, X3)) {
@@ -762,14 +756,14 @@ int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
   }
   static TtkPerDevice attr;
   if (attr.first()) {
-    TTK_CUDA(cudaFuncSetAttribute(conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    TTK_CUDA(cudaFuncSetAttribute(conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3, H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   C::SMEM_BYTES));
   }
   if (S == 2 && ((a.hin & 1) || (a.win & 1))) return TTK_ERR_UNSUPPORTED;
   // the input map's TFLOAT32 type makes TMA round fp32 to TF32 (nearest-even) while it fills shared memory; 3xTF32 needs the raw values
   const CUtensorMapDataType in_type =
-      ESZ == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : X3 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32;
-  const CUtensorMapDataType res_type = ESZ == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+      ESZ == 2 ? Fmt16<H>::MAP : X3 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32;
+  const CUtensorMapDataType res_type = ESZ == 2 ? Fmt16<H>::MAP : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
   KMaps maps;
   cuuint32_t box[4] = {(cuuint32_t)C::KC, (cuuint32_t)C::TW, (cuuint32_t)C::TR, 1};
   cuuint32_t es[4] = {1, 1, 1, 1};
@@ -800,7 +794,7 @@ int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
     }
   }
   KArgs k;
-  k.w = ESZ == 2 ? (const void*)cv.w_umma : X3 ? (const void*)cv.w_x3 : (const void*)cv.w_umma32;
+  k.w = ESZ == 2 ? (H ? (const void*)cv.w_umma_f16 : (const void*)cv.w_umma) : X3 ? (const void*)cv.w_x3 : (const void*)cv.w_umma32;
   k.w_lo = X3 ? (const void*)(cv.w_x3 + (size_t)cv.k * cv.k * cv.cin_p * cv.cout_p) : nullptr;      // [W_hi image | W_lo image]
   k.bias = cv.bias;
   k.out = a.out;
@@ -825,14 +819,14 @@ int launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
   occ = std::max(1, std::min(occ, 2));
   const int gx = std::max(1, std::min(k.total, ttk_num_sms() * occ / nsplit));
   dim3 grid(gx, nsplit);
-  conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3><<<grid, HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, C::SMEM_BYTES, st>>>(maps, k);
+  conv_umma_kernel<KS, S, CIN, COUT, R, STAGES, RB, KCO, ESZ, HF, X3, H><<<grid, HF ? THREADS_HF : X3 ? THREADS_X3 : THREADS, C::SMEM_BYTES, st>>>(maps, k);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }
 
-// Bottleneck tail: out = relu(W3 a + Wd x + bias) with a (32 channels) and x (64 channels) K-concatenated.  bf16: two 64-channel
+// Bottleneck tail: out = relu(W3 a + Wd x + bias) with a (32 channels) and x (64 channels) K-concatenated.  bf16 / fp16: two 64-channel
 // K-chunks (the first box reaches past the 32-channel tensor, TMA zero fills); tf32: three 32-channel chunks (a | x[0:32] | x[32:64]).
-template <int ESZ>
+template <int ESZ, int H = 0>
 int launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a, cudaStream_t st) {
   constexpr int R = 2, STAGES = 3, KC = 128 / ESZ, CINK = ESZ == 2 ? 128 : 96;
   using C = Cfg<1, 1, CINK, 128, R, STAGES, 0, 0, ESZ>;
@@ -840,7 +834,8 @@ int launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a,
   if (!encode) return TTK_ERR_UNSUPPORTED;
   static TtkPerDevice attr;
   if (attr.first()) {
-    TTK_CUDA(cudaFuncSetAttribute(conv_umma_kernel<1, 1, CINK, 128, R, STAGES, 0, 0, ESZ>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+    TTK_CUDA(cudaFuncSetAttribute(conv_umma_kernel<1, 1, CINK, 128, R, STAGES, 0, 0, ESZ, 0, 0, H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  C::SMEM_BYTES));
   }
   KMaps maps;
   cuuint32_t box[4] = {(cuuint32_t)KC, (cuuint32_t)BW, (cuuint32_t)R, 1};
@@ -850,7 +845,7 @@ int launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a,
   for (int i = 0; i < 2; ++i) {
     cuuint64_t dims[4] = {(cuuint64_t)cins[i], (cuuint64_t)a.win, (cuuint64_t)a.hin, (cuuint64_t)a.n};
     cuuint64_t strides[3] = {(cuuint64_t)cins[i] * ESZ, (cuuint64_t)a.win * cins[i] * ESZ, (cuuint64_t)a.hin * a.win * cins[i] * ESZ};
-    const CUresult r = encode(&maps.m[i], ESZ == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 4, const_cast<void*>(ins[i]),
+    const CUresult r = encode(&maps.m[i], ESZ == 2 ? Fmt16<H>::MAP : CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 4, const_cast<void*>(ins[i]),
                               dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return TTK_ERR_UNSUPPORTED;      // e.g. a driver that rejects a box wider than the tensor
@@ -877,26 +872,29 @@ int launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a,
   k.tiles_y = ttk_cdiv(a.hout, R);
   k.total = k.tiles_x * k.tiles_y * a.n;
   const int gx = std::max(1, std::min(k.total, ttk_num_sms()));
-  conv_umma_kernel<1, 1, CINK, 128, R, STAGES, 0, 0, ESZ><<<gx, THREADS, C::SMEM_BYTES, st>>>(maps, k);
+  conv_umma_kernel<1, 1, CINK, 128, R, STAGES, 0, 0, ESZ, 0, 0, H><<<gx, THREADS, C::SMEM_BYTES, st>>>(maps, k);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }
 
 }  // namespace
 
-int ttk_conv_umma_launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a, cudaStream_t st, int esz) {
+int ttk_conv_umma_launch_dual(const void* w_dual, const float* bias_dual, const ConvLaunch& a, cudaStream_t st, int esz, bool f16) {
   if (a.cin != 32 || a.cin2 != 64 || a.cout != 128) return TTK_ERR_UNSUPPORTED;
-  return esz == 2 ? launch_dual<2>(w_dual, bias_dual, a, st) : launch_dual<4>(w_dual, bias_dual, a, st);
+  if (esz == 2) return f16 ? launch_dual<2, 1>(w_dual, bias_dual, a, st) : launch_dual<2>(w_dual, bias_dual, a, st);
+  return launch_dual<4>(w_dual, bias_dual, a, st);
 }
 
 // Host image of the fused bottleneck tail's B operand: [k-chunk][cout 128][KC], chunk 0 = conv3 (32 input channels, zero padded to KC),
-// then the projection shortcut's 64 input channels.  bf16: KC = 64 (2 chunks); tf32: KC = 32 (3 chunks), values rounded to TF32.
-void ttk_conv_umma_pack_dual(const float* w3, const float* wd, int esz, std::vector<uint8_t>& out) {
+// then the projection shortcut's 64 input channels.  bf16 / fp16 (f16): KC = 64 (2 chunks); tf32: KC = 32 (3 chunks), values rounded
+// to TF32.
+void ttk_conv_umma_pack_dual(const float* w3, const float* wd, int esz, std::vector<uint8_t>& out, bool f16) {
   const int KC = 128 / esz, nk = esz == 2 ? 2 : 3;
   out.assign((size_t)nk * 128 * KC * esz, 0);
   auto put = [&](int kc, int co, int c, float v) {
     const size_t i = ((size_t)kc * 128 + co) * KC + c;
-    if (esz == 2) reinterpret_cast<__nv_bfloat16*>(out.data())[i] = __float2bfloat16_rn(v);
+    if (esz == 2 && f16) reinterpret_cast<__half*>(out.data())[i] = Fmt16<1>::round(v);
+    else if (esz == 2) reinterpret_cast<__nv_bfloat16*>(out.data())[i] = Fmt16<0>::round(v);
     else reinterpret_cast<float*>(out.data())[i] = round_tf32(v);
   };
   for (int co = 0; co < 128; ++co) {
@@ -909,13 +907,13 @@ void ttk_conv_umma_pack_dual(const float* w3, const float* wd, int esz, std::vec
 //   fused 3x3 stride 1 : [slice][k-chunk][kx][ky][cout_tile][KC]   (B = the three vertical taps side by side)
 //   transition1.0      : [k-chunk][ky][kx][cout][KC]               (B = all nine taps: horizontal + vertical fusion)
 //   otherwise          : [slice][tap][k-chunk][cout_tile][KC]
-// bf16 (w_umma), TF32-rounded fp32 (w_umma32) and 3xTF32 (w_x3: the W_hi = tf32(w) image, then the W_lo = w - W_hi image) are all
-// kept; they differ in KC and in the slice width of the wide layers.
+// bf16 (w_umma), TF32-rounded fp32 (w_umma32), 3xTF32 (w_x3: the W_hi = tf32(w) image, then the W_lo = w - W_hi image) and fp16
+// (w_umma_f16, the bf16 layout) are all kept; the 2- and 4-byte images differ in KC and in the slice width of the wide layers.
 int ttk_conv_umma_pack(TtkConv& cv, const float* w_host) {
   const int kk = cv.k * cv.k;
-  for (int mode = 0; mode < 3; ++mode) {
-    const int esz = mode == 0 ? 2 : 4;
-    const bool x3 = mode == 2;
+  for (int mode = 0; mode < 4; ++mode) {
+    const int esz = mode == 0 || mode == 3 ? 2 : 4;
+    const bool x3 = mode == 2, f16 = mode == 3;
     const int KC = kc_of(cv, esz, x3);
     const int nkc = cv.cin_p / KC;
     const int ct = cout_tile(cv, esz, x3);
@@ -938,22 +936,68 @@ int ttk_conv_umma_pack(TtkConv& cv, const float* w_host) {
           }
           const float v = w_host[((size_t)co * cv.cin + ci) * kk + t];
           const size_t i = (row * ct + cl) * KC + c;
-          if (esz == 2) {
-            reinterpret_cast<__nv_bfloat16*>(w.data())[i] = __float2bfloat16_rn(v);
+          if (f16) {
+            reinterpret_cast<__half*>(w.data())[i] = Fmt16<1>::round(v);
+          } else if (esz == 2) {
+            reinterpret_cast<__nv_bfloat16*>(w.data())[i] = Fmt16<0>::round(v);
           } else {
             const float hi = round_tf32(v);
             reinterpret_cast<float*>(w.data())[i] = hi;
             if (x3) reinterpret_cast<float*>(w.data())[count + i] = v - hi;      // exact
           }
         }
-    void** dst = esz == 2 ? (void**)&cv.w_umma : x3 ? (void**)&cv.w_x3 : (void**)&cv.w_umma32;
+    void** dst = f16 ? (void**)&cv.w_umma_f16 : esz == 2 ? (void**)&cv.w_umma : x3 ? (void**)&cv.w_x3 : (void**)&cv.w_umma32;
     if (!*dst) TTK_CUDA(cudaMalloc(dst, w.size()));
     TTK_CUDA(cudaMemcpy(*dst, w.data(), w.size(), cudaMemcpyHostToDevice));
   }
   return TTK_OK;
 }
 
-int ttk_conv_umma_launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st, int esz, bool x3) {
+namespace {
+// 16-bit elements (H = 0: bf16, 1: fp16): one dispatch table for both formats
+template <int H>
+int launch16(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st) {
+  const int ci = cv.cin_p, co = cout_tile(cv, 2);
+  const int k = cv.k, s = cv.stride;
+#define TTK_UMMA(KS_, S_, CI_, CO_, R_, ST_, RB_) \
+  if (k == KS_ && s == S_ && ci == CI_ && co == CO_) return launch<KS_, S_, CI_, CO_, R_, ST_, RB_, 0, 2, 0, 0, H>(cv, a, st);
+#define TTK_UMMA_KC(KS_, S_, CI_, CO_, R_, ST_, KC_) \
+  if (k == KS_ && s == S_ && ci == CI_ && co == CO_) return launch<KS_, S_, CI_, CO_, R_, ST_, 0, KC_, 2, 0, 0, H>(cv, a, st);
+  // 3x3 stride 1
+  TTK_UMMA(3, 1, 16, 64, 4, 3, 0)     // stem conv1 (9 -> 64, input padded to 16 channels)
+  TTK_UMMA_KC(3, 1, 64, 64, 4, 3, 32)      // stem conv2, quarter-resolution branch
+  if (k == 3 && s == 1 && ci == 32 && co == 32 && a.nres == 0) return launch<3, 1, 32, 32, 8, 2, 0, 0, 2, 0, 0, H>(cv, a, st);   // no residual tiles to stage: taller tile
+  TTK_UMMA(3, 1, 32, 32, 4, 2, 1)     // bottleneck conv2, half-resolution branch
+  TTK_UMMA(3, 1, 16, 16, 8, 3, 1)     // full-resolution branch
+  TTK_UMMA_KC(3, 1, 128, 16, 8, 2, 32)     // transition1.0
+  TTK_UMMA_KC(3, 1, 128, 64, 2, 2, 32)     // eighth-resolution branch (128 -> 128 as two 64-channel output slices)
+  // 3x3 stride 2 (transitions and fuse down-paths)
+  TTK_UMMA_KC(3, 2, 128, 32, 2, 3, 32)
+  TTK_UMMA(3, 2, 16, 16, 4, 3, 0)
+  TTK_UMMA(3, 2, 16, 32, 4, 3, 0)
+  TTK_UMMA(3, 2, 16, 64, 4, 3, 0)
+  TTK_UMMA(3, 2, 16, 128, 2, 3, 0)
+  TTK_UMMA(3, 2, 32, 32, 4, 2, 0)
+  TTK_UMMA(3, 2, 32, 64, 4, 2, 0)
+  TTK_UMMA(3, 2, 32, 128, 2, 2, 0)
+  TTK_UMMA_KC(3, 2, 64, 64, 2, 3, 32)      // 64 -> 128 as two output slices
+  // 1x1
+  TTK_UMMA(1, 1, 64, 32, 4, 2, 0)     // bottleneck conv1, fuse 64 -> 32
+  TTK_UMMA(1, 1, 32, 128, 2, 3, 1)    // bottleneck conv3 (+ projection shortcut as residual)
+  TTK_UMMA(1, 1, 64, 128, 2, 3, 0)    // bottleneck projection shortcut
+  TTK_UMMA(1, 1, 32, 16, 4, 3, 0)     // fuse layers (low -> high resolution)
+  TTK_UMMA(1, 1, 64, 16, 4, 3, 0)
+  TTK_UMMA(1, 1, 128, 16, 4, 2, 0)
+  TTK_UMMA(1, 1, 128, 32, 4, 2, 0)
+  TTK_UMMA(1, 1, 128, 64, 2, 2, 0)
+#undef TTK_UMMA_KC
+#undef TTK_UMMA
+  return TTK_ERR_UNSUPPORTED;
+}
+}  // namespace
+
+int ttk_conv_umma_launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st, int esz, bool x3, bool f16) {
+  if (esz == 2) return f16 ? launch16<1>(cv, a, st) : launch16<0>(cv, a, st);
   const int ci = cv.cin_p, co = cout_tile(cv, esz, x3);
   const int k = cv.k, s = cv.stride;
   if (x3) {
@@ -986,39 +1030,6 @@ int ttk_conv_umma_launch(const TtkConv& cv, const ConvLaunch& a, cudaStream_t st
     TTK_UMMA3(1, 1, 128, 32, 2, 2, 32)
     TTK_UMMA3(1, 1, 128, 64, 2, 2, 32)
 #undef TTK_UMMA3
-    return TTK_ERR_UNSUPPORTED;
-  }
-  if (esz == 2) {
-#define TTK_UMMA(KS_, S_, CI_, CO_, R_, ST_, RB_) \
-  if (k == KS_ && s == S_ && ci == CI_ && co == CO_) return launch<KS_, S_, CI_, CO_, R_, ST_, RB_>(cv, a, st);
-    // 3x3 stride 1
-    TTK_UMMA(3, 1, 16, 64, 4, 3, 0)     // stem conv1 (9 -> 64, input padded to 16 channels)
-    if (k == 3 && s == 1 && ci == 64 && co == 64) return launch<3, 1, 64, 64, 4, 3, 0, 32>(cv, a, st);      // stem conv2, quarter-resolution branch
-    if (k == 3 && s == 1 && ci == 32 && co == 32 && a.nres == 0) return launch<3, 1, 32, 32, 8, 2, 0>(cv, a, st);   // no residual tiles to stage: taller tile
-    TTK_UMMA(3, 1, 32, 32, 4, 2, 1)     // bottleneck conv2, half-resolution branch
-    TTK_UMMA(3, 1, 16, 16, 8, 3, 1)     // full-resolution branch
-    if (k == 3 && s == 1 && ci == 128 && co == 16) return launch<3, 1, 128, 16, 8, 2, 0, 32>(cv, a, st);     // transition1.0
-    if (k == 3 && s == 1 && ci == 128 && co == 64) return launch<3, 1, 128, 64, 2, 2, 0, 32>(cv, a, st);    // eighth-resolution branch (128 -> 128 as two 64-channel output slices)
-    // 3x3 stride 2 (transitions and fuse down-paths)
-    if (k == 3 && s == 2 && ci == 128 && co == 32) return launch<3, 2, 128, 32, 2, 3, 0, 32>(cv, a, st);
-    TTK_UMMA(3, 2, 16, 16, 4, 3, 0)
-    TTK_UMMA(3, 2, 16, 32, 4, 3, 0)
-    TTK_UMMA(3, 2, 16, 64, 4, 3, 0)
-    TTK_UMMA(3, 2, 16, 128, 2, 3, 0)
-    TTK_UMMA(3, 2, 32, 32, 4, 2, 0)
-    TTK_UMMA(3, 2, 32, 64, 4, 2, 0)
-    TTK_UMMA(3, 2, 32, 128, 2, 2, 0)
-    if (k == 3 && s == 2 && ci == 64 && co == 64) return launch<3, 2, 64, 64, 2, 3, 0, 32>(cv, a, st);       // 64 -> 128 as two output slices
-    // 1x1
-    TTK_UMMA(1, 1, 64, 32, 4, 2, 0)     // bottleneck conv1, fuse 64 -> 32
-    TTK_UMMA(1, 1, 32, 128, 2, 3, 1)    // bottleneck conv3 (+ projection shortcut as residual)
-    TTK_UMMA(1, 1, 64, 128, 2, 3, 0)    // bottleneck projection shortcut
-    TTK_UMMA(1, 1, 32, 16, 4, 3, 0)     // fuse layers (low -> high resolution)
-    TTK_UMMA(1, 1, 64, 16, 4, 3, 0)
-    TTK_UMMA(1, 1, 128, 16, 4, 2, 0)
-    TTK_UMMA(1, 1, 128, 32, 4, 2, 0)
-    TTK_UMMA(1, 1, 128, 64, 2, 2, 0)
-#undef TTK_UMMA
     return TTK_ERR_UNSUPPORTED;
   }
   // ---- TF32 (fp32 activations): same tiles, re-sized for 4-byte elements (shared memory: weights + STAGES boxes + residual tiles) ----

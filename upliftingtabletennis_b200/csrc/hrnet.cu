@@ -10,11 +10,14 @@
 //   TTK_F32    - fp32 SIMT direct convolution (parity with the CPU reference),
 //   TTK_TF32   - fp32 storage, tcgen05 implicit GEMM with TF32 operands (conv_umma.cu),
 //   TTK_TF32X3 - fp32 storage, tcgen05 implicit GEMM with three TF32 products of split operands per product (fp32-level results),
-//   TTK_BF16   - bf16 storage, fp32 accumulate, tcgen05 implicit GEMM.
+//   TTK_BF16   - bf16 storage, fp32 accumulate, tcgen05 implicit GEMM,
+//   TTK_F16    - the same with IEEE fp16 storage and operands (umma_prims.h: Fmt16 holds what differs between the two 16-bit formats).
 #include <algorithm>
 #include <map>
+#include <type_traits>
 
 #include "hrnet.h"
+#include "umma_prims.h"
 
 namespace {
 
@@ -273,7 +276,7 @@ size_t plan_memory(ttk_hrnet* h, int bs, int H, int W, size_t elem) {
 }
 
 // ------------------------------------------------------------------------------------------
-// fp32-accumulate SIMT direct convolution on NHWC tensors (T = float or bf16 storage)
+// fp32-accumulate SIMT direct convolution on NHWC tensors (T = float, bf16 or fp16 storage)
 // ------------------------------------------------------------------------------------------
 template <typename T>
 struct Io;
@@ -302,6 +305,17 @@ struct Io<__nv_bfloat16> {
     q.x = *reinterpret_cast<uint32_t*>(&a);
     q.y = *reinterpret_cast<uint32_t*>(&b);
     *reinterpret_cast<uint2*>(p) = q;
+  }
+};
+
+template <>
+struct Io<__half> {
+  static __device__ __forceinline__ void load4(const __half* p, float* v) {
+    const uint2 q = *reinterpret_cast<const uint2*>(p);
+    v[0] = umma::Fmt16<1>::lo(q.x); v[1] = umma::Fmt16<1>::hi(q.x); v[2] = umma::Fmt16<1>::lo(q.y); v[3] = umma::Fmt16<1>::hi(q.y);
+  }
+  static __device__ __forceinline__ void store4(__half* p, const float* v) {
+    *reinterpret_cast<uint2*>(p) = make_uint2(umma::Fmt16<1>::pack(v[0], v[1]), umma::Fmt16<1>::pack(v[2], v[3]));
   }
 };
 
@@ -419,9 +433,10 @@ __global__ void __launch_bounds__(128) conv_simt_kernel(const T* __restrict__ in
   }
 }
 
+// rounded_weights: the weights rounded to the 16-bit storage format T
 template <typename T>
 int launch_conv_simt(const TtkConv& cv, const ConvLaunch& a, bool rounded_weights, cudaStream_t st) {
-  const float* w = rounded_weights ? cv.w_bfr : cv.w_f32;
+  const float* w = !rounded_weights ? cv.w_f32 : std::is_same<T, __half>::value ? cv.w_hfr : cv.w_bfr;
   const int cog = a.cout / COT;
 #define TTK_SIMT(K_, S_)                                                                                              \
   {                                                                                                                   \
@@ -472,11 +487,12 @@ __global__ void __launch_bounds__(256) sum_kernel(const T* __restrict__ in, T* _
     live[u] = e < row_items;
     if (live[u]) sum_ld256(in + (row0 + e) * V, raw[u]);
   }
+  using F16 = umma::Fmt16Of<T>;                     // 16-bit storage: bf16 or fp16
   auto widen = [](const uint32_t* q, float* f, bool add) {
     if (sizeof(T) == 2) {
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
-        const float lo = __uint_as_float(q[j] << 16), hi = __uint_as_float(q[j] & 0xffff0000u);
+        const float lo = F16::lo(q[j]), hi = F16::hi(q[j]);
         f[2 * j % V] = add ? f[2 * j % V] + lo : lo;
         f[(2 * j + 1) % V] = add ? f[(2 * j + 1) % V] + hi : hi;
       }
@@ -504,10 +520,7 @@ __global__ void __launch_bounds__(256) sum_kernel(const T* __restrict__ in, T* _
     uint32_t o[8];
     if (sizeof(T) == 2) {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        __nv_bfloat162 p2 = __floats2bfloat162_rn(v[u][2 * j % V], v[u][(2 * j + 1) % V]);
-        o[j] = *reinterpret_cast<uint32_t*>(&p2);
-      }
+      for (int j = 0; j < 8; ++j) o[j] = F16::pack(v[u][2 * j % V], v[u][(2 * j + 1) % V]);
     } else {
 #pragma unroll
       for (int j = 0; j < 8; ++j) o[j] = __float_as_uint(v[u][j % V]);
@@ -582,7 +595,7 @@ int profile_mark(ttk_hrnet* h, int oi, int bs, int H, int W, size_t elem, cudaSt
   return TTK_OK;
 }
 
-// B operands of the fused bottleneck tail (conv3 and the projection shortcut K-concatenated), bf16 and TF32 images
+// B operands of the fused bottleneck tail (conv3 and the projection shortcut K-concatenated), bf16, fp16 and TF32 images
 int prepare_dual(ttk_hrnet* h) {
   if (h->dual_ds_op < 0) return TTK_OK;
   const TtkConv& ds = h->convs[h->ops[h->dual_ds_op].conv];
@@ -590,10 +603,12 @@ int prepare_dual(ttk_hrnet* h) {
   if (ds.w_host.empty() || c3.w_host.empty()) return TTK_OK;
   std::vector<float> b(128);
   for (int co = 0; co < 128; ++co) b[co] = c3.b_host[co] + ds.b_host[co];
-  for (int esz = 2; esz <= 4; esz += 2) {
+  for (int mode = 0; mode < 3; ++mode) {
+    const int esz = mode == 1 ? 4 : 2;
+    const bool f16 = mode == 2;
     std::vector<uint8_t> w;
-    ttk_conv_umma_pack_dual(c3.w_host.data(), ds.w_host.data(), esz, w);
-    void** dst = esz == 2 ? &h->w_dual : &h->w_dual32;
+    ttk_conv_umma_pack_dual(c3.w_host.data(), ds.w_host.data(), esz, w, f16);
+    void** dst = f16 ? &h->w_dual_f16 : esz == 2 ? &h->w_dual : &h->w_dual32;
     if (!*dst) TTK_CUDA(cudaMalloc(dst, w.size()));
     TTK_CUDA(cudaMemcpy(*dst, w.data(), w.size(), cudaMemcpyHostToDevice));
   }
@@ -616,11 +631,12 @@ bool is_basic_block(const ttk_hrnet* h, size_t oi) {
   return true;
 }
 
-// esz: 0 = SIMT kernels on T storage, 2 = bf16 tcgen05 path, 4 = TF32 tcgen05 path on fp32 storage (x3: 3xTF32; convolutions only --
-// the fused BasicBlock and bottleneck kernels have no x3 variant, so those convolutions run one by one)
+// esz: 0 = SIMT kernels on T storage, 2 = 16-bit tcgen05 path (bf16 or fp16, as T), 4 = TF32 tcgen05 path on fp32 storage (x3:
+// 3xTF32; convolutions only -- the fused BasicBlock and bottleneck kernels have no x3 variant, so those convolutions run one by one)
 template <typename T>
 int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, char* ws, int esz, bool x3, cudaStream_t st) {
   const bool umma = esz != 0;
+  constexpr bool f16 = std::is_same<T, __half>::value;
   h->cur_esz = esz;
   h->cur_x3 = x3;
   bool dual_skipped = false;
@@ -644,7 +660,7 @@ int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, cha
       }
       // TF32: mode 2 = two 3-row tiles in flight (fp32 residual from global memory), mode 3 = one 4-row tile (residual from the staged tile)
       const int rc = ttk_block_umma_launch(h->convs[op.conv], h->convs[op2.conv], p2(op.in), p2(op2.out), bs, H >> ti.shift, W >> ti.shift, st,
-                                           esz == 4 && h->use_block_fusion == 3 ? 5 : esz);
+                                           esz == 4 && h->use_block_fusion == 3 ? 5 : esz, f16);
       if (rc == TTK_OK) {
         h->launches++;
         ++oi;                                      // conv2 is done as well
@@ -693,7 +709,7 @@ int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, cha
         d.nres = 0;
         d.in2 = ptr(ds.in);
         d.cin2 = h->convs[ds.conv].cin_p;
-        rc = ttk_conv_umma_launch_dual(esz == 2 ? h->w_dual : h->w_dual32, h->bias_dual, d, st, esz);
+        rc = ttk_conv_umma_launch_dual(esz == 2 ? (f16 ? h->w_dual_f16 : h->w_dual) : h->w_dual32, h->bias_dual, d, st, esz, f16);
         if (rc == TTK_ERR_UNSUPPORTED) {      // driver refused the maps: run the two convolutions separately from now on
           h->use_dual = 0;
           ConvLaunch s0;
@@ -706,14 +722,14 @@ int run_plan(ttk_hrnet* h, const void* x, int bs, int H, int W, float* heat, cha
           for (int r = 0; r < 3; ++r) { s0.res[r] = nullptr; s0.res_shift[r] = 0; }
           s0.n = bs; s0.hin = H >> dti.shift; s0.win = W >> dti.shift; s0.hout = H >> dto.shift; s0.wout = W >> dto.shift;
           s0.cin = dcv.cin_p; s0.cout = dcv.cout_p; s0.relu = 0;
-          rc = ttk_conv_umma_launch(dcv, s0, st, esz);
+          rc = ttk_conv_umma_launch(dcv, s0, st, esz, false, f16);
           if (rc == TTK_ERR_UNSUPPORTED) rc = launch_conv_simt<T>(dcv, s0, sizeof(T) == 2, st);
           if (rc != TTK_OK) return rc;
           h->launches++;
-          rc = ttk_conv_umma_launch(cv, a, st, esz);
+          rc = ttk_conv_umma_launch(cv, a, st, esz, false, f16);
         }
       } else if (umma) {
-        rc = ttk_conv_umma_launch(cv, a, st, esz, x3);
+        rc = ttk_conv_umma_launch(cv, a, st, esz, x3, f16);
       }
       if (rc == TTK_ERR_UNSUPPORTED) {
         // no tensor-core kernel for this shape: the SIMT kernel on the same storage (fp32-level on fp32 tensors)
@@ -763,7 +779,8 @@ int upload(float** dst, const std::vector<float>& src) {
   return TTK_OK;
 }
 
-float bf16_round(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
+float bf16_round(float v) { return __bfloat162float(umma::Fmt16<0>::round(v)); }
+float f16_round(float v) { return __half2float(umma::Fmt16<1>::round(v)); }
 
 }  // namespace
 
@@ -798,12 +815,15 @@ extern "C" void ttk_hrnet_destroy(ttk_hrnet* h) {
   for (TtkConv& c : h->convs) {
     cudaFree(c.w_f32);
     cudaFree(c.w_bfr);
+    cudaFree(c.w_hfr);
     cudaFree(c.bias);
     cudaFree(c.w_umma);
+    cudaFree(c.w_umma_f16);
     cudaFree(c.w_umma32);
     cudaFree(c.w_x3);
   }
   cudaFree(h->w_dual);
+  cudaFree(h->w_dual_f16);
   cudaFree(h->w_dual32);
   cudaFree(h->bias_dual);
   cudaFree(h->final_w);
@@ -846,7 +866,7 @@ extern "C" int ttk_hrnet_set_conv(ttk_hrnet* h, int i, const float* w_host, cons
     return TTK_OK;
   }
   // [cout][cin][k][k] -> [tap][cin_p][cout_p], zero padded
-  std::vector<float> w((size_t)kk * c.cin_p * c.cout_p, 0.f), wr(w.size(), 0.f), b(c.cout_p, 0.f);
+  std::vector<float> w((size_t)kk * c.cin_p * c.cout_p, 0.f), wr(w.size(), 0.f), wh(w.size(), 0.f), b(c.cout_p, 0.f);
   for (int co = 0; co < c.cout; ++co) {
     b[co] = b_host[co];
     for (int ci = 0; ci < c.cin; ++ci)
@@ -854,6 +874,7 @@ extern "C" int ttk_hrnet_set_conv(ttk_hrnet* h, int i, const float* w_host, cons
         const float v = w_host[((size_t)co * c.cin + ci) * kk + t];
         w[((size_t)t * c.cin_p + ci) * c.cout_p + co] = v;
         wr[((size_t)t * c.cin_p + ci) * c.cout_p + co] = bf16_round(v);
+        wh[((size_t)t * c.cin_p + ci) * c.cout_p + co] = f16_round(v);
       }
   }
   c.w_host.assign(w_host, w_host + (size_t)c.cout * c.cin * kk);
@@ -862,6 +883,8 @@ extern "C" int ttk_hrnet_set_conv(ttk_hrnet* h, int i, const float* w_host, cons
   int rc = upload(&c.w_f32, w);
   if (rc) return rc;
   rc = upload(&c.w_bfr, wr);
+  if (rc) return rc;
+  rc = upload(&c.w_hfr, wh);
   if (rc) return rc;
   rc = upload(&c.bias, b);
   if (rc) return rc;
@@ -874,14 +897,15 @@ extern "C" int ttk_hrnet_set_conv(ttk_hrnet* h, int i, const float* w_host, cons
 extern "C" size_t ttk_hrnet_workspace_bytes(const ttk_hrnet* h, int batch, int height, int width, int dtype) {
   if (!h || batch <= 0 || height <= 0 || width <= 0) return 0;
   const int bs = std::min(batch, h->subbatch);
-  return plan_memory(const_cast<ttk_hrnet*>(h), bs, height, width, dtype == TTK_BF16 ? 2 : 4);      // TTK_TF32 stores fp32
+  return plan_memory(const_cast<ttk_hrnet*>(h), bs, height, width, dtype == TTK_BF16 || dtype == TTK_F16 ? 2 : 4);      // TTK_TF32 stores fp32
 }
 
 extern "C" int ttk_hrnet_forward(ttk_hrnet* h, const void* x_dev, int batch, int height, int width, int dtype,
                                  float* heatmaps_dev, void* workspace_dev, size_t workspace_bytes, void* stream) {
   TTK_CHECK_ARG(h, "ttk_hrnet_forward: null handle");
   if (int rc = ttk_bind_device(&h->device, "ttk_hrnet_forward")) return rc;
-  TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_TF32 || dtype == TTK_TF32X3, "ttk_hrnet_forward: bad dtype %d", dtype);
+  TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_TF32 || dtype == TTK_TF32X3 || dtype == TTK_F16,
+                "ttk_hrnet_forward: bad dtype %d", dtype);
   TTK_CHECK_ARG(batch >= 0 && height > 0 && width > 0 && height % 8 == 0 && width % 8 == 0,
                 "ttk_hrnet_forward: height and width must be positive multiples of 8 (got %dx%d)", height, width);
   for (const TtkConv& c : h->convs)
@@ -897,7 +921,7 @@ extern "C" int ttk_hrnet_forward(ttk_hrnet* h, const void* x_dev, int batch, int
   }
   if (batch == 0) return TTK_OK;
   TTK_CHECK_ARG(x_dev && heatmaps_dev && workspace_dev, "ttk_hrnet_forward: null pointer");
-  const size_t elem = dtype == TTK_BF16 ? 2 : 4;
+  const size_t elem = dtype == TTK_BF16 || dtype == TTK_F16 ? 2 : 4;
   const int bs = std::min(batch, h->subbatch);
   const size_t need = plan_memory(h, bs, height, width, elem);
   TTK_CHECK_ARG(workspace_bytes >= need, "ttk_hrnet_forward: workspace too small (%zu < %zu)", workspace_bytes, need);
@@ -911,6 +935,8 @@ extern "C" int ttk_hrnet_forward(ttk_hrnet* h, const void* x_dev, int batch, int
       rc = run_plan<float>(h, x, nb, height, width, heat, (char*)workspace_dev, 0, false, st);
     else if (dtype == TTK_TF32 || dtype == TTK_TF32X3)
       rc = run_plan<float>(h, x, nb, height, width, heat, (char*)workspace_dev, h->force_simt ? 0 : 4, dtype == TTK_TF32X3, st);
+    else if (dtype == TTK_F16)
+      rc = run_plan<__half>(h, x, nb, height, width, heat, (char*)workspace_dev, h->force_simt ? 0 : 2, false, st);
     else
       rc = run_plan<__nv_bfloat16>(h, x, nb, height, width, heat, (char*)workspace_dev, h->force_simt ? 0 : 2, false, st);
     if (rc != TTK_OK) return rc;
@@ -956,12 +982,8 @@ extern "C" int ttk_hrnet_set_force_simt(ttk_hrnet* h, int enable) {
 // Test hook: run ONE convolution of the plan (bias + optional same-shape residual + optional ReLU) on caller buffers.
 // path: 0 = fp32 SIMT (float tensors), 1 = bf16 SIMT, 2 = bf16 tcgen05, 3 = TF32 tcgen05 on float tensors, 4 = 3xTF32 tcgen05 on
 // float tensors (2 to 4 return TTK_ERR_UNSUPPORTED if the shape has no kernel).
-extern "C" int ttk_hrnet_debug_conv(ttk_hrnet* h, int conv_index, const void* in_dev, int n, int hin, int win, const void* res_dev,
-                                    int relu, int path, void* out_dev, void* stream) {
-  TTK_CHECK_ARG(h && conv_index >= 0 && conv_index < (int)h->convs.size() - 1, "ttk_hrnet_debug_conv: bad conv index %d", conv_index);
-  const TtkConv& cv = h->convs[conv_index];
-  TTK_CHECK_ARG(cv.set, "ttk_hrnet_debug_conv: weights not set");
-  TTK_CHECK_ARG(path >= 0 && path <= 4, "ttk_hrnet_debug_conv: bad path %d", path);
+namespace {
+ConvLaunch debug_launch(const TtkConv& cv, const void* in_dev, int n, int hin, int win, const void* res_dev, int relu, void* out_dev) {
   ConvLaunch a;
   a.in = in_dev;
   a.out = out_dev;
@@ -978,10 +1000,32 @@ extern "C" int ttk_hrnet_debug_conv(ttk_hrnet* h, int conv_index, const void* in
   a.cin = cv.cin_p;
   a.cout = cv.cout_p;
   a.relu = relu;
+  return a;
+}
+}  // namespace
+
+extern "C" int ttk_hrnet_debug_conv(ttk_hrnet* h, int conv_index, const void* in_dev, int n, int hin, int win, const void* res_dev,
+                                    int relu, int path, void* out_dev, void* stream) {
+  TTK_CHECK_ARG(h && conv_index >= 0 && conv_index < (int)h->convs.size() - 1, "ttk_hrnet_debug_conv: bad conv index %d", conv_index);
+  const TtkConv& cv = h->convs[conv_index];
+  TTK_CHECK_ARG(cv.set, "ttk_hrnet_debug_conv: weights not set");
+  TTK_CHECK_ARG(path >= 0 && path <= 4, "ttk_hrnet_debug_conv: bad path %d", path);
+  const ConvLaunch a = debug_launch(cv, in_dev, n, hin, win, res_dev, relu, out_dev);
   cudaStream_t st = (cudaStream_t)stream;
   if (path == 0) return launch_conv_simt<float>(cv, a, false, st);
   if (path == 1) return launch_conv_simt<__nv_bfloat16>(cv, a, true, st);
   return ttk_conv_umma_launch(cv, a, st, path == 2 ? 2 : 4, path == 4);
+}
+
+// Test hook: the same for fp16 tensors: simt 1 = fp16 SIMT, 0 = fp16 tcgen05 (TTK_ERR_UNSUPPORTED if the shape has no kernel).
+extern "C" int ttk_hrnet_debug_conv_f16(ttk_hrnet* h, int conv_index, const void* in_dev, int n, int hin, int win, const void* res_dev,
+                                        int relu, int simt, void* out_dev, void* stream) {
+  TTK_CHECK_ARG(h && conv_index >= 0 && conv_index < (int)h->convs.size() - 1, "ttk_hrnet_debug_conv_f16: bad conv index %d", conv_index);
+  const TtkConv& cv = h->convs[conv_index];
+  TTK_CHECK_ARG(cv.set, "ttk_hrnet_debug_conv_f16: weights not set");
+  const ConvLaunch a = debug_launch(cv, in_dev, n, hin, win, res_dev, relu, out_dev);
+  if (simt) return launch_conv_simt<__half>(cv, a, true, (cudaStream_t)stream);
+  return ttk_conv_umma_launch(cv, a, (cudaStream_t)stream, 2, false, true);
 }
 
 // Test hook: one BasicBlock (conv_index = its conv1, conv_index + 1 = its conv2) through the fused tcgen05 kernel on caller buffers:

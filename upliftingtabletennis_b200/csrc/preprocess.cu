@@ -7,6 +7,7 @@
 #include <algorithm>
 
 #include "ttk_internal.h"
+#include "umma_prims.h"
 
 namespace {
 
@@ -38,7 +39,7 @@ __device__ __forceinline__ AxisTap axis_tap(int d, int n_src, double scale) {
   return t;
 }
 
-template <int F, int MODE>   // F frames per stack; MODE 0: NCHW f32, 1: NHWC16 f32, 2: NHWC16 bf16
+template <int F, int MODE>   // F frames per stack; MODE 0: NCHW f32, 1: NHWC16 f32, 2: NHWC16 bf16, 3: NHWC16 fp16
 __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restrict__ frames, int src_h, int src_w,
                                                          int stack_stride, int dst_h, int dst_w, double scale_x,
                                                          double scale_y, const float* __restrict__ lut,
@@ -85,14 +86,13 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restri
 #pragma unroll
     for (int q = 0; q < 4; ++q) o[q] = make_float4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
   } else {
-    uint4* o = (uint4*)((__nv_bfloat16*)out + ((size_t)(s * dst_h + y) * dst_w + x) * 16);
+    uint4* o = (uint4*)((uint16_t*)out + ((size_t)(s * dst_h + y) * dst_w + x) * 16);
     uint32_t w[8];
 #pragma unroll
     for (int c = 0; c < 8; ++c) {
       const float lo = 2 * c < 3 * F ? v[2 * c] : 0.f;
       const float hi = 2 * c + 1 < 3 * F ? v[2 * c + 1] : 0.f;
-      __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
-      w[c] = *reinterpret_cast<uint32_t*>(&p);
+      w[c] = umma::Fmt16<MODE == 3>::pack(lo, hi);
     }
     o[0] = make_uint4(w[0], w[1], w[2], w[3]);
     o[1] = make_uint4(w[4], w[5], w[6], w[7]);
@@ -225,14 +225,13 @@ __global__ void __launch_bounds__(256) preprocess_tile_kernel(const uint8_t* __r
 #pragma unroll
         for (int q4 = 0; q4 < 4; ++q4) o[q4] = make_float4(w[4 * q4], w[4 * q4 + 1], w[4 * q4 + 2], w[4 * q4 + 3]);
       } else {
-        uint4* o = (uint4*)((__nv_bfloat16*)out + ((size_t)(s * dst_h + y) * dst_w + x) * 16);
+        uint4* o = (uint4*)((uint16_t*)out + ((size_t)(s * dst_h + y) * dst_w + x) * 16);
         uint32_t w[8];
 #pragma unroll
         for (int c = 0; c < 8; ++c) {
           const float lo = 2 * c < 3 * F ? v[2 * c] : 0.f;
           const float hi = 2 * c + 1 < 3 * F ? v[2 * c + 1] : 0.f;
-          __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
-          w[c] = *reinterpret_cast<uint32_t*>(&p);
+          w[c] = umma::Fmt16<MODE == 3>::pack(lo, hi);
         }
         o[0] = make_uint4(w[0], w[1], w[2], w[3]);
         o[1] = make_uint4(w[4], w[5], w[6], w[7]);
@@ -266,8 +265,10 @@ int launch(int mode, dim3 grid, cudaStream_t st, const uint8_t* frames, int src_
       preprocess_tile_kernel<F, 0><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
     else if (mode == 1)
       preprocess_tile_kernel<F, 1><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
-    else
+    else if (mode == 2)
       preprocess_tile_kernel<F, 2><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
+    else
+      preprocess_tile_kernel<F, 3><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
     TTK_LAUNCH_CHECK();
     return TTK_OK;
   }
@@ -275,8 +276,10 @@ int launch(int mode, dim3 grid, cudaStream_t st, const uint8_t* frames, int src_
     preprocess_kernel<F, 0><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
   else if (mode == 1)
     preprocess_kernel<F, 1><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
-  else
+  else if (mode == 2)
     preprocess_kernel<F, 2><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
+  else
+    preprocess_kernel<F, 3><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }
@@ -299,8 +302,8 @@ extern "C" int ttk_preprocess_stacks(const uint8_t* frames_dev, int n_frames, in
     TTK_CHECK_ARG(dtype == TTK_F32, "ttk_preprocess_stacks: NCHW output is float32 only");
     mode = 0;
   } else if (layout == TTK_LAYOUT_NHWC16) {
-    TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16, "ttk_preprocess_stacks: bad dtype");
-    mode = dtype == TTK_F32 ? 1 : 2;
+    TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_F16, "ttk_preprocess_stacks: bad dtype");
+    mode = dtype == TTK_F32 ? 1 : dtype == TTK_BF16 ? 2 : 3;
   } else {
     ttk_set_error("ttk_preprocess_stacks: bad layout %d", layout);
     return TTK_ERR_ARG;

@@ -6,7 +6,10 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 namespace umma {
 
@@ -85,9 +88,11 @@ __device__ __forceinline__ uint64_t make_desc16(uint32_t addr16) {
   constexpr uint32_t hi = ((SBO_BYTES >> 4) & 0x3FFF) | (1u << 14) | ((LAYOUT & 7) << 29);
   return ((uint64_t)hi << 32) | (uint64_t)(addr16 + 0x10000u);
 }
-// kind::f16 instruction descriptor: D f32, A/B bf16, K-major unless the transpose bit is set (bit 15: A, bit 16: B MN-major)
-__host__ __device__ constexpr uint32_t make_idesc(int M, int N, int b_mn_major = 0) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+// kind::f16 instruction descriptor: D f32, A/B bf16 (f16 = 1: IEEE fp16), K-major unless the transpose bit is set (bit 15: A, bit 16:
+// B MN-major)
+__host__ __device__ constexpr uint32_t make_idesc(int M, int N, int b_mn_major = 0, int f16 = 0) {
+  return (1u << 4) | ((f16 ? 0u : 1u) << 7) | ((f16 ? 0u : 1u) << 10) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(N >> 3) << 17) |
+         ((uint32_t)(M >> 4) << 24);
 }
 __device__ __forceinline__ void mma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -96,7 +101,7 @@ __device__ __forceinline__ void mma(uint32_t tmem_d, uint64_t da, uint64_t db, u
       "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// Operand formats of the instruction descriptor (bits 7-9: A, 10-12: B): 1 = bf16 (kind::f16), 2 = tf32 (kind::tf32, fp32 containers
+// Operand formats of the instruction descriptor (bits 7-9: A, 10-12: B): 0 = fp16, 1 = bf16 (kind::f16), 2 = tf32 (kind::tf32, fp32 containers
 // whose low 13 mantissa bits the tensor core ignores)
 __host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
@@ -200,6 +205,41 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t tmem, uint32_t cols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(cols));
 }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
+// The two 16-bit element formats of the kind::f16 paths: H = 0 bf16, H = 1 IEEE fp16 (same 2-byte storage and tiles; fp16 has 10
+// mantissa bits against bf16's 7, and a range of +-65504).  Everything that differs between them is here: storage type, TMA element
+// type, instruction-descriptor operand format and the conversions.
+template <int H>
+struct Fmt16 {
+  using T = typename std::conditional<H != 0, __half, __nv_bfloat16>::type;
+  static constexpr CUtensorMapDataType MAP = H ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  // two values -> one 32-bit word (lo in the low half), round to nearest-even
+  static __device__ __forceinline__ uint32_t pack(float lo, float hi) {
+    if constexpr (H != 0) {
+      __half2 p = __floats2half2_rn(lo, hi);
+      return *reinterpret_cast<uint32_t*>(&p);
+    } else {
+      __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
+      return *reinterpret_cast<uint32_t*>(&p);
+    }
+  }
+  // the low / high value of a word: bf16 is widened by bit placement (keeps the conversion pipe free), fp16 needs a real conversion
+  static __device__ __forceinline__ float lo(uint32_t w) {
+    if constexpr (H != 0) return __half2float(__ushort_as_half((unsigned short)(w & 0xffffu)));
+    else return __uint_as_float(w << 16);
+  }
+  static __device__ __forceinline__ float hi(uint32_t w) {
+    if constexpr (H != 0) return __half2float(__ushort_as_half((unsigned short)(w >> 16)));
+    else return __uint_as_float(w & 0xffff0000u);
+  }
+  // host: round a float32 to the format, nearest-even
+  static T round(float v) {
+    if constexpr (H != 0) return __float2half_rn(v);
+    else return __float2bfloat16_rn(v);
+  }
+};
+template <typename T>
+using Fmt16Of = Fmt16<std::is_same<T, __half>::value ? 1 : 0>;
 
 typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                              const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);

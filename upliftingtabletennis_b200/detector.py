@@ -12,7 +12,7 @@ import torch.nn as nn
 
 from . import _lib
 from ._lib import lib, check, ptr, stream_ptr
-from .precision import PrecisionMixin, TF32, TF32X3, FP32, BF16, lib_enum, storage_dtype
+from .precision import PrecisionMixin, TF32, TF32X3, FP32, BF16, FP16, lib_enum, storage_dtype
 
 BN_EPS = 1e-5
 
@@ -73,14 +73,15 @@ class HRNetEngine:
         self.loaded = True
 
     def forward_nhwc16(self, x, out=None, precision=None):
-        """x: (B, H, W, 16) float32 or bfloat16 CUDA tensor -> (B, out_count, H, W) float32.
-        precision: 'tf32' / 'tf32x3' / 'fp32' for float32 tensors (default 'fp32': the strict SIMT path), 'bf16' for bfloat16 tensors."""
+        """x: (B, H, W, 16) float32, bfloat16 or float16 CUDA tensor -> (B, out_count, H, W) float32.
+        precision: 'tf32' / 'tf32x3' / 'fp32' for float32 tensors (default 'fp32': the strict SIMT path), 'bf16' for bfloat16 tensors,
+        'fp16' for float16 tensors."""
         assert self.loaded, 'weights not loaded'
         assert x.is_cuda and x.dim() == 4 and x.shape[3] == 16 and x.is_contiguous()
         B, H, W, _ = x.shape
-        assert x.dtype in (torch.float32, torch.bfloat16)
+        assert x.dtype in (torch.float32, torch.bfloat16, torch.float16)
         if precision is None:
-            precision = FP32 if x.dtype == torch.float32 else BF16
+            precision = {torch.float32: FP32, torch.bfloat16: BF16, torch.float16: FP16}[x.dtype]
         assert storage_dtype(precision) == x.dtype, 'precision %r needs %s tensors' % (precision, storage_dtype(precision))
         dt = lib_enum(precision)
         need = lib.ttk_hrnet_workspace_bytes(self.h, B, H, W, dt)
@@ -113,9 +114,9 @@ class _HRNetModule(PrecisionMixin, nn.Module):
     ``compute_dtype`` (constructor argument ``dtype``): 'tf32' (default: tcgen05 tensor cores at the precision class of the
     reference's cuDNN convolutions), 'tf32x3' (tcgen05 tensor cores, three TF32 products of split operands per product: fp32-level
     results, the class of the reference on a CPU or with cuDNN's TF32 off), 'fp32' (SIMT, strict parity), 'bf16' (tcgen05, bf16
-    storage)."""
+    storage), 'fp16' (tcgen05, fp16 storage: the bf16 kernels with 10 mantissa bits, range +-65504)."""
     default_precision = TF32
-    supported_precisions = (TF32, TF32X3, FP32, BF16)
+    supported_precisions = (TF32, TF32X3, FP32, BF16, FP16)
 
     def __init__(self, in_ch, out_ch, out_first, out_count, dtype=None):
         super().__init__()

@@ -15,7 +15,7 @@ import torch
 
 from . import _lib, ops
 from .detector import MyHRNet, WASBNet
-from .precision import TF32, TF32X3, canonical
+from .precision import FP16, TF32, TF32X3, canonical
 from .vitpose import TableVitPose, VitPose
 from .uplift import get_model as get_uplifting_model
 
@@ -98,8 +98,8 @@ def _check_model_name(model_name, available):
 
 
 def load_ball_model(model_path, dtype=None):
-    """inference/inference_balldetection.py:40-61.  dtype: arithmetic class ('tf32' / 'tf32x3' / 'fp32' / 'bf16', see precision.py);
-    None = the architecture's default."""
+    """inference/inference_balldetection.py:40-61.  dtype: arithmetic class ('tf32' / 'tf32x3' / 'fp32' / 'bf16', and 'fp16' for
+    WASB; see precision.py); None = the architecture's default."""
     load_dict = torch.load(model_path, map_location=torch.device('cpu'), weights_only=False)
     info = load_dict['additional_info']
     model_name, resolution, in_frames = info['model_name'], info['image_resolution'], info['in_frames']
@@ -582,7 +582,13 @@ class TableTennisPipeline:
 
     def __init__(self, ball_model='vitpose', ball_model_aux='wasb', table_model='vitpose', table_model_aux='hrnet', dtype=None):
         """dtype: None / 'tf32' / 'tf32x3' = every component on its reference-class tensor-core path (TF32 convolutions, 3xTF32
-        Linear layers and attention); 'bf16' or 'fp32' = every component on that path."""
+        Linear layers and attention); 'bf16' or 'fp32' = every component on that path.  'fp16' is refused: only the WASB / HRNet
+        detectors have an fp16 path (switch one with ``pipe.<detector>.model.compute_dtype = 'fp16'``)."""
+        if dtype is not None and canonical(dtype) == FP16:
+            raise NotImplementedError("TableTennisPipeline has no fp16 path: fp16 exists for the WASB / HRNet detectors only (ViTPose and "
+                                      "the uplifting transformer have none); build the pipeline with another dtype and set "
+                                      "pipe.ball_detector_aux.model.compute_dtype = 'fp16' / pipe.table_detector_aux.model.compute_dtype = "
+                                      "'fp16' on a WASB / HRNet detector")
         self.device = _device()
         if dtype is not None and canonical(dtype) in (TF32, TF32X3):
             dtype = None

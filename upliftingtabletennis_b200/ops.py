@@ -35,10 +35,13 @@ def preprocess_stacks(frames, frames_per_stack, stack_stride, n_stacks, dst_w, d
         shape, lay = (n_stacks, 3 * frames_per_stack, dst_h, dst_w), _lib.LAYOUT_NCHW_F32
     else:
         shape, lay = (n_stacks, dst_h, dst_w, 16), _lib.LAYOUT_NHWC16
+    dts = {torch.float32: _lib.F32, torch.bfloat16: _lib.BF16, torch.float16: _lib.F16}
+    if dtype not in dts:
+        raise ValueError('preprocess_stacks: dtype must be torch.float32, torch.bfloat16 or torch.float16, got %r' % (dtype,))
     if out is None:
         out = torch.empty(shape, dtype=dtype, device=frames.device)
     assert tuple(out.shape) == shape and out.dtype == dtype and out.is_contiguous()
-    dt = _lib.F32 if dtype == torch.float32 else _lib.BF16
+    dt = dts[dtype]
     check(lib.ttk_preprocess_stacks(ptr(frames), n, sh, sw, frames_per_stack, stack_stride, n_stacks, dst_h, dst_w,
                                     ptr(normalize_lut(frames.device)), ptr(out), lay, dt, stream_ptr()))
     return out
