@@ -65,6 +65,13 @@ TTK_API int ttk_preprocess_stacks(const uint8_t* frames_dev, int n_frames, int s
                           int frames_per_stack, int stack_stride, int n_stacks,
                           int dst_h, int dst_w, const float* lut_dev,
                           void* out_dev, int layout, int dtype, void* stream);
+/* The same output, with stack s reading frames first_frame_dev[s] + {0..frames_per_stack-1} (int32, device): stacks of several clips
+ * in one pass, no window crossing a clip.  Bytes are identical to ttk_preprocess_stacks for the same frames.  The caller guarantees
+ * 0 <= first_frame_dev[s] <= n_frames - frames_per_stack (the table is device memory and is not read on the host). */
+TTK_API int ttk_preprocess_stacks_indexed(const uint8_t* frames_dev, int n_frames, int src_h, int src_w,
+                          int frames_per_stack, const int32_t* first_frame_dev, int n_stacks,
+                          int dst_h, int dst_w, const float* lut_dev,
+                          void* out_dev, int layout, int dtype, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * HRNet-W18-small heatmap network (WASB ball detector / HRNet table detector).
@@ -206,6 +213,14 @@ TTK_API int ttk_decode_profile_read(float* argmax_ms, float* fit_ms);
 TTK_API int ttk_filter_ball(const double* pos1_dev, const double* pos2_dev, int n_frames, double fps, double threshold_px,
                     double* out_xy_dev, int64_t* out_idx_dev, double* out_times_dev, int32_t* out_offsets_dev,
                     void* stream);
+/* ttk_filter_ball over n_clips clips in one launch.  pos*_dev: the clips' n_frames x 3 detections concatenated;
+ * frame_offsets_dev[n_clips+1] int32 (device): clip c is frames [offs[c], offs[c+1]), offs[0] = 0, non-decreasing, offs[n_clips] =
+ * n_frames (empty clips allowed).  Each clip is filtered exactly like ttk_filter_ball: out_idx and out_times (= idx / fps) count from
+ * the clip's first frame.  The kept rows are packed in clip order; out_offsets_dev[n_clips+1] receives the per-clip prefix sums on the
+ * device, in the format ttk_trajectory_pack reads.  Capacity n_frames rows per output. */
+TTK_API int ttk_filter_ball_clips(const double* pos1_dev, const double* pos2_dev, int n_clips, const int32_t* frame_offsets_dev,
+                    int n_frames, double fps, double threshold_px, double* out_xy_dev, int64_t* out_idx_dev,
+                    double* out_times_dev, int32_t* out_offsets_dev, void* stream);
 
 /* ttk_filter_table replaces filter_trajectory_table (inference/utils.py:137-169) and
  * _filter_keypoints_with_dbscan (:172-232; scikit-learn DBSCAN semantics, see csrc/filters.cu):
@@ -219,6 +234,12 @@ TTK_API size_t ttk_filter_table_workspace_bytes(int n_clips, int n_frames, int n
 TTK_API int ttk_filter_table(const double* pos1_dev, const double* pos2_dev, int n_clips, int n_frames, int n_keypoints,
                      double agree_px, double eps, int min_samples, double* out_dev, void* workspace_dev,
                      size_t workspace_bytes, void* stream);
+/* ttk_filter_table over n_clips clips of different lengths: pos*_dev hold the clips' frames concatenated (n_frames x n_keypoints x 3),
+ * frame_offsets_dev as for ttk_filter_ball_clips.  out_dev: n_clips x n_keypoints x 3, each clip bit-identical to ttk_filter_table on
+ * that clip alone.  workspace: ttk_filter_table_workspace_bytes(1, n_frames, n_keypoints). */
+TTK_API int ttk_filter_table_clips(const double* pos1_dev, const double* pos2_dev, int n_clips, const int32_t* frame_offsets_dev,
+                     int n_frames, int n_keypoints, double agree_px, double eps, int min_samples, double* out_dev,
+                     void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Trajectory packing: pixel -> [0,1] normalisation, pad/crop to seq_len, mask.

@@ -30,6 +30,7 @@ def _load():
         'ttk_host_blocking_sync': (i32, [i32, C.POINTER(C.c_uint)]),
         'ttk_device_ok': (i32, []),
         'ttk_preprocess_stacks': (i32, [vp, i32, i32, i32, i32, i32, i32, i32, i32, vp, vp, i32, i32, vp]),
+        'ttk_preprocess_stacks_indexed': (i32, [vp, i32, i32, i32, i32, vp, i32, i32, i32, vp, vp, i32, i32, vp]),
         'ttk_hrnet_create': (i32, [i32, i32, i32, i32, C.POINTER(vp)]),
         'ttk_hrnet_destroy': (None, [vp]),
         'ttk_hrnet_num_convs': (i32, [vp]),
@@ -64,8 +65,10 @@ def _load():
         'ttk_decode_set_profile': (i32, [i32]),
         'ttk_decode_profile_read': (i32, [C.POINTER(C.c_float), C.POINTER(C.c_float)]),
         'ttk_filter_ball': (i32, [vp, vp, i32, C.c_double, C.c_double, vp, vp, vp, vp, vp]),
+        'ttk_filter_ball_clips': (i32, [vp, vp, i32, vp, i32, C.c_double, C.c_double, vp, vp, vp, vp, vp]),
         'ttk_filter_table_workspace_bytes': (sz, [i32, i32, i32]),
         'ttk_filter_table': (i32, [vp, vp, i32, i32, i32, C.c_double, C.c_double, i32, vp, vp, sz, vp]),
+        'ttk_filter_table_clips': (i32, [vp, vp, i32, vp, i32, i32, C.c_double, C.c_double, i32, vp, vp, sz, vp]),
         'ttk_calibrate_workspace_bytes': (sz, [i32, i32]),
         'ttk_calibrate_camera': (i32, [vp, vp, vp, i32, i32, i32, i32, i32, C.c_double, vp, vp, vp, vp, sz, vp]),
         'ttk_trajectory_pack': (i32, [vp, vp, vp, vp, i32, i32, C.c_double, C.c_double, vp, vp, vp, vp, vp]),

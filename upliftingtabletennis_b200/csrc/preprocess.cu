@@ -39,11 +39,13 @@ __device__ __forceinline__ AxisTap axis_tap(int d, int n_src, double scale) {
   return t;
 }
 
-template <int F, int MODE>   // F frames per stack; MODE 0: NCHW f32, 1: NHWC16 f32, 2: NHWC16 bf16, 3: NHWC16 fp16
+// F frames per stack; MODE 0: NCHW f32, 1: NHWC16 f32, 2: NHWC16 bf16, 3: NHWC16 fp16.  IDX: stack s starts at frame first_frame[s]
+// instead of s * stack_stride (first_frame is the last parameter, so the strided instantiations keep their parameter offsets).
+template <int F, int MODE, bool IDX>
 __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restrict__ frames, int src_h, int src_w,
                                                          int stack_stride, int dst_h, int dst_w, double scale_x,
                                                          double scale_y, const float* __restrict__ lut,
-                                                         void* __restrict__ out) {
+                                                         void* __restrict__ out, const int32_t* __restrict__ first_frame) {
   __shared__ float s_lut[768];
   for (int i = threadIdx.x; i < 768; i += blockDim.x) s_lut[i] = lut[i];
   __syncthreads();
@@ -57,7 +59,7 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restri
   float v[3 * F];
 #pragma unroll
   for (int f = 0; f < F; ++f) {
-    const uint8_t* img = frames + (size_t)(s * stack_stride + f) * src_h * src_w * 3;
+    const uint8_t* img = frames + (size_t)((IDX ? __ldg(first_frame + s) : s * stack_stride) + f) * src_h * src_w * 3;
     const uint8_t* r0 = img + ((size_t)ty.s0 * src_w) * 3;
     const uint8_t* r1 = img + ((size_t)ty.s1 * src_w) * 3;
 #pragma unroll
@@ -113,11 +115,11 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t* __restri
 constexpr int PRE_ROW_BYTES = 1536;      // >= (256 outputs * max scale 1.6 + 3) * 3 bytes + alignment slack
 constexpr int PRE_STAGE = 3;             // 128-bit staging loads per thread and tile (3 frames x 2 rows x <= 96 vectors / 256 threads)
 constexpr int LUT_COPIES = 8;            // normalisation table replicated so that random look-ups spread over the banks
-template <int F, int MODE>
+template <int F, int MODE, bool IDX>
 __global__ void __launch_bounds__(256) preprocess_tile_kernel(const uint8_t* __restrict__ frames, int src_h, int src_w,
                                                               int stack_stride, int n_stacks, int dst_h, int dst_w, int nxb,
                                                               double scale_x, double scale_y, const float* __restrict__ lut,
-                                                              void* __restrict__ out) {
+                                                              void* __restrict__ out, const int32_t* __restrict__ first_frame) {
   __shared__ float s_lut[768 * LUT_COPIES];                    // [entry][copy]
   __shared__ __align__(16) uint8_t s_rows[2][F * 2 * PRE_ROW_BYTES];
   for (int i = threadIdx.x; i < 768 * LUT_COPIES; i += blockDim.x) s_lut[i] = lut[i / LUT_COPIES];
@@ -153,7 +155,7 @@ __global__ void __launch_bounds__(256) preprocess_tile_kernel(const uint8_t* __r
   }
   uint4 q[PRE_STAGE];
   auto fetch = [&](int s, const AxisTap& ty) {                 // global -> registers
-    const uint8_t* base = frames + (size_t)s * stack_stride * frame_bytes;
+    const uint8_t* base = frames + (IDX ? (size_t)__ldg(first_frame + s) * frame_bytes : (size_t)s * stack_stride * frame_bytes);
     const uint8_t* up = base + (size_t)ty.s0 * row_bytes;
     const uint8_t* low = base + (size_t)ty.s1 * row_bytes;
 #pragma unroll
@@ -243,9 +245,9 @@ __global__ void __launch_bounds__(256) preprocess_tile_kernel(const uint8_t* __r
   }
 }
 
-template <int F>
+template <int F, bool IDX>
 int launch(int mode, dim3 grid, cudaStream_t st, const uint8_t* frames, int src_h, int src_w, int stack_stride, int dst_h,
-           int dst_w, const float* lut, void* out) {
+           int dst_w, const float* lut, void* out, const int32_t* first) {
   const double sx = (double)src_w / (double)dst_w, sy = (double)src_h / (double)dst_h;
   const bool staged = !(src_h == dst_h && src_w == dst_w) && ((size_t)src_w * 3) % 16 == 0 && ((uintptr_t)frames & 15) == 0 &&
                       (256.0 * sx + 4.0) * 3.0 + 32.0 <= PRE_ROW_BYTES;
@@ -262,29 +264,49 @@ int launch(int mode, dim3 grid, cudaStream_t st, const uint8_t* frames, int src_
     const int walkers = (int)std::max(1LL, std::min<long long>(n_tiles, (n_sm * 5) / nxb));
     const dim3 g(nxb * walkers);
     if (mode == 0)
-      preprocess_tile_kernel<F, 0><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
+      preprocess_tile_kernel<F, 0, IDX><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out,
+                                                          first);
     else if (mode == 1)
-      preprocess_tile_kernel<F, 1><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
+      preprocess_tile_kernel<F, 1, IDX><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out,
+                                                          first);
     else if (mode == 2)
-      preprocess_tile_kernel<F, 2><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
+      preprocess_tile_kernel<F, 2, IDX><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out,
+                                                          first);
     else
-      preprocess_tile_kernel<F, 3><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out);
+      preprocess_tile_kernel<F, 3, IDX><<<g, 256, 0, st>>>(frames, src_h, src_w, stack_stride, n_stacks, dst_h, dst_w, nxb, sx, sy, lut, out,
+                                                          first);
     TTK_LAUNCH_CHECK();
     return TTK_OK;
   }
   if (mode == 0)
-    preprocess_kernel<F, 0><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
+    preprocess_kernel<F, 0, IDX><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out, first);
   else if (mode == 1)
-    preprocess_kernel<F, 1><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
+    preprocess_kernel<F, 1, IDX><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out, first);
   else if (mode == 2)
-    preprocess_kernel<F, 2><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
+    preprocess_kernel<F, 2, IDX><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out, first);
   else
-    preprocess_kernel<F, 3><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out);
+    preprocess_kernel<F, 3, IDX><<<grid, 256, 0, st>>>(frames, src_h, src_w, stack_stride, dst_h, dst_w, sx, sy, lut, out, first);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }
 
 }  // namespace
+
+// layout / dtype -> kernel MODE, or -1 (the error is set)
+static int preprocess_mode(const char* fn, int layout, int dtype) {
+  if (layout == TTK_LAYOUT_NCHW_F32) {
+    if (dtype == TTK_F32) return 0;
+    ttk_set_error("%s: NCHW output is float32 only", fn);
+    return -1;
+  }
+  if (layout == TTK_LAYOUT_NHWC16) {
+    if (dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_F16) return dtype == TTK_F32 ? 1 : dtype == TTK_BF16 ? 2 : 3;
+    ttk_set_error("%s: bad dtype", fn);
+    return -1;
+  }
+  ttk_set_error("%s: bad layout %d", fn, layout);
+  return -1;
+}
 
 extern "C" int ttk_preprocess_stacks(const uint8_t* frames_dev, int n_frames, int src_h, int src_w, int frames_per_stack,
                                      int stack_stride, int n_stacks, int dst_h, int dst_w, const float* lut_dev,
@@ -297,20 +319,30 @@ extern "C" int ttk_preprocess_stacks(const uint8_t* frames_dev, int n_frames, in
                 "ttk_preprocess_stacks: stacks read past the last frame (%d stacks, stride %d, %d frames)", n_stacks,
                 stack_stride, n_frames);
   TTK_CHECK_ARG(n_stacks <= 65535 && dst_h <= 65535, "ttk_preprocess_stacks: grid too large");
-  int mode;
-  if (layout == TTK_LAYOUT_NCHW_F32) {
-    TTK_CHECK_ARG(dtype == TTK_F32, "ttk_preprocess_stacks: NCHW output is float32 only");
-    mode = 0;
-  } else if (layout == TTK_LAYOUT_NHWC16) {
-    TTK_CHECK_ARG(dtype == TTK_F32 || dtype == TTK_BF16 || dtype == TTK_F16, "ttk_preprocess_stacks: bad dtype");
-    mode = dtype == TTK_F32 ? 1 : dtype == TTK_BF16 ? 2 : 3;
-  } else {
-    ttk_set_error("ttk_preprocess_stacks: bad layout %d", layout);
-    return TTK_ERR_ARG;
-  }
+  const int mode = preprocess_mode("ttk_preprocess_stacks", layout, dtype);
+  if (mode < 0) return TTK_ERR_ARG;
   if (n_stacks == 0) return TTK_OK;
   dim3 grid(ttk_cdiv(dst_w, 256), dst_h, n_stacks);
   cudaStream_t st = (cudaStream_t)stream;
-  if (frames_per_stack == 3) return launch<3>(mode, grid, st, frames_dev, src_h, src_w, stack_stride, dst_h, dst_w, lut_dev, out_dev);
-  return launch<1>(mode, grid, st, frames_dev, src_h, src_w, stack_stride, dst_h, dst_w, lut_dev, out_dev);
+  if (frames_per_stack == 3)
+    return launch<3, false>(mode, grid, st, frames_dev, src_h, src_w, stack_stride, dst_h, dst_w, lut_dev, out_dev, nullptr);
+  return launch<1, false>(mode, grid, st, frames_dev, src_h, src_w, stack_stride, dst_h, dst_w, lut_dev, out_dev, nullptr);
+}
+
+extern "C" int ttk_preprocess_stacks_indexed(const uint8_t* frames_dev, int n_frames, int src_h, int src_w, int frames_per_stack,
+                                             const int32_t* first_frame_dev, int n_stacks, int dst_h, int dst_w,
+                                             const float* lut_dev, void* out_dev, int layout, int dtype, void* stream) {
+  TTK_CHECK_ARG(frames_dev && lut_dev && out_dev && first_frame_dev, "ttk_preprocess_stacks_indexed: null pointer");
+  TTK_CHECK_ARG(frames_per_stack == 1 || frames_per_stack == 3, "ttk_preprocess_stacks_indexed: frames_per_stack must be 1 or 3");
+  TTK_CHECK_ARG(n_stacks >= 0 && n_frames >= frames_per_stack && src_h > 0 && src_w > 0 && dst_h > 0 && dst_w > 0,
+                "ttk_preprocess_stacks_indexed: bad sizes");
+  TTK_CHECK_ARG(n_stacks <= 65535 && dst_h <= 65535, "ttk_preprocess_stacks_indexed: grid too large");
+  const int mode = preprocess_mode("ttk_preprocess_stacks_indexed", layout, dtype);
+  if (mode < 0) return TTK_ERR_ARG;
+  if (n_stacks == 0) return TTK_OK;
+  dim3 grid(ttk_cdiv(dst_w, 256), dst_h, n_stacks);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (frames_per_stack == 3)
+    return launch<3, true>(mode, grid, st, frames_dev, src_h, src_w, 1, dst_h, dst_w, lut_dev, out_dev, first_frame_dev);
+  return launch<1, true>(mode, grid, st, frames_dev, src_h, src_w, 1, dst_h, dst_w, lut_dev, out_dev, first_frame_dev);
 }

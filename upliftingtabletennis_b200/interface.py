@@ -13,11 +13,11 @@ import zipfile
 import numpy as np
 import torch
 
-from . import _lib, ops
+from . import _lib, ops, sharding
 from .detector import MyHRNet, WASBNet
-from .precision import FP16, TF32, TF32X3, canonical
+from .precision import BF16, FP16, TF32, TF32X3, canonical
 from .vitpose import TableVitPose, VitPose
-from .uplift import get_model as get_uplifting_model
+from .uplift import MASK_FORMAT_ERROR, MultiStageModel, get_model as get_uplifting_model
 
 HEIGHT, WIDTH = 1080, 1920          # inference/utils.py:22
 BALL_VISIBLE = 1
@@ -236,18 +236,17 @@ class _ReadyMarks:
 
 
 _POOL = None
-_UPLOADER = None
+_UPLOADERS = {}
 
 
-def _uploader():
-    """One background thread that walks the staging ring of an upload, so that predict() can launch the first network pass while
-    later frames are still being staged (the staging loop on the calling thread held back every kernel launch for the whole upload:
-    15 ms of a 66 ms call for 96 copied 1080p frames)."""
-    global _UPLOADER
-    if _UPLOADER is None:
+def _uploader(device_index):
+    """One background thread per device that walks the staging ring of an upload, so that predict() can launch the first network pass
+    while later frames are still being staged (the staging loop on the calling thread held back every kernel launch for the whole upload:
+    15 ms of a 66 ms call for 96 copied 1080p frames).  Per device, so that predict_clips' uploads to several GPUs run side by side."""
+    if device_index not in _UPLOADERS:
         from concurrent.futures import ThreadPoolExecutor
-        _UPLOADER = ThreadPoolExecutor(max_workers=1, thread_name_prefix='ttk-upload')
-    return _UPLOADER
+        _UPLOADERS.setdefault(device_index, ThreadPoolExecutor(max_workers=1, thread_name_prefix='ttk-upload%d' % device_index))
+    return _UPLOADERS[device_index]
 
 
 def _staging_pool():
@@ -261,19 +260,99 @@ def _staging_pool():
     return _POOL
 
 
+# ---- several clips in one call (TableTennisPipeline.predict_clips) -----------------------------------
+def clip_stack_plan(lengths, frames_per_stack):
+    """Stacks of clips of the given lengths, concatenated in clip order: a sliding window of frames_per_stack frames over each clip
+    (stride 1, like predict), never crossing a clip.  Returns the first frame of every stack and the (n + 1,) prefix sums of the stack
+    counts per clip."""
+    first, offsets, f0 = [], [0], 0
+    for n in lengths:
+        k = max(n - frames_per_stack + 1, 0)
+        first.extend(range(f0, f0 + k))
+        offsets.append(offsets[-1] + k)
+        f0 += n
+    return first, offsets
+
+
+def clip_blocks(lengths, max_frames):
+    """Contiguous [(first clip, end)] blocks of at most max_frames frames each (a longer clip is a block of its own): bounds the device
+    memory of predict_clips like _Detector.segment bounds predict()'s."""
+    blocks, a, frames = [], 0, 0
+    for i, n in enumerate(lengths):
+        if i > a and frames + n > max_frames:
+            blocks.append((a, i))
+            a, frames = i, 0
+        frames += n
+    if a < len(lengths):
+        blocks.append((a, len(lengths)))
+    return blocks
+
+
+def parse_devices(devices, device_count):
+    """predict_clips' `devices`: a list of CUDA device indices, torch.device('cuda', i) or 'cuda:i' strings (a device may repeat: one
+    replica of the models per entry).  Returns the indices; anything else raises ValueError."""
+    if isinstance(devices, (str, int, torch.device)) or not hasattr(devices, '__iter__'):
+        raise ValueError('devices must be a list of CUDA devices (indices, torch.device or "cuda:N"), got %r' % (devices,))
+    out = []
+    for d in devices:
+        if isinstance(d, bool) or not isinstance(d, (int, str, torch.device)):
+            raise ValueError('devices: %r is not a CUDA device index, torch.device or "cuda:N" string' % (d,))
+        if not isinstance(d, int):
+            try:
+                dv = torch.device(d)
+            except (RuntimeError, ValueError) as e:
+                raise ValueError('devices: %r is not a CUDA device (%s)' % (d, e)) from None
+            if dv.type != 'cuda' or dv.index is None:
+                raise ValueError('devices: %r is not an indexed CUDA device ("cuda:N")' % (d,))
+            d = dv.index
+        if not 0 <= d < device_count:
+            raise ValueError('devices: CUDA device %d does not exist (%d visible)' % (d, device_count))
+        out.append(d)
+    if not out:
+        raise ValueError('devices must name at least one CUDA device')
+    return out
+
+
+def _replicate(model, device):
+    """A copy of a detector / uplifting model shell on `device`: same architecture, state dict and compute_dtype.  Its weights reach the
+    library on its first forward, which must run with `device` current."""
+    if isinstance(model, WASBNet):
+        m = WASBNet(in_frames=model.in_ch // 3, resolution=model.resolution)
+    elif isinstance(model, MyHRNet):
+        m = MyHRNet(resolution=model.resolution)
+    elif isinstance(model, VitPose):
+        m = VitPose(in_frames=model.in_ch // 3, resolution=model.resolution)
+    elif isinstance(model, TableVitPose):
+        m = TableVitPose(resolution=model.resolution)
+    elif isinstance(model, MultiStageModel):
+        m = MultiStageModel(model.dim, model.depth, model.num_heads, model.mode, model.time_rotation, model.use_skipconnection)
+    else:
+        raise TypeError('no replica for %s' % type(model).__name__)
+    m.compute_dtype = model.compute_dtype
+    m.load_state_dict(model.state_dict())
+    return m.to(device).eval()
+
+
+def _fingerprint(model):
+    """Changes when the model's compute_dtype, one of its tensors (replaced) or their contents (in-place writes, load_state_dict) do."""
+    return model.compute_dtype, tuple((k, v.data_ptr(), v._version) for k, v in model.state_dict().items())
+
+
 # ---- public classes ---------------------------------------------------------------------------------
 class _Detector:
     frames_per_stack = 1
     chunk = 16                     # stacks per network pass: bounds the workspace and lets uploads overlap compute
     ramp = (4, 12)                 # stacks of the first passes while a clip's frames are still being uploaded
 
-    def _run(self, frames_u8, stack_stride, n_stacks, return_heatmaps, ready=None, heatmaps_to_host=False):
+    def _run(self, frames_u8, stack_stride, n_stacks, return_heatmaps, ready=None, heatmaps_to_host=False, first=None):
         """frames_u8: (n, H, W, 3) uint8 CUDA.  Returns positions (n_stacks, C, 3) float64 CUDA and heatmaps or None.
         heatmaps_to_host: the heatmaps come back as ONE pinned host tensor (n_stacks, C, h, w) instead of a CUDA tensor: each pass's
         maps are copied out on a third stream while the next pass computes (predict() returns 3.6 MB per map to the host, like the
         reference does; through pageable memory that copy alone cost more than the network).
         `ready`: [(last frame index, event)] from _upload -- a chunk starts as soon as its frames have arrived, so the
-        host->device copy of later frames overlaps the network on earlier ones."""
+        host->device copy of later frames overlaps the network on earlier ones.
+        `first`: (host list, (n_stacks,) int32 CUDA tensor) of each stack's first frame, replacing s * stack_stride -- stacks of several
+        clips (clip_stack_plan); the passes are then all full but the last."""
         w, h = self.model.resolution
         prec, dt = self.model.compute_dtype, self.model.storage_dtype
         pos, hms = [], []
@@ -281,20 +360,29 @@ class _Detector:
         waited = 0
         # while frames are still arriving the first passes are short (4, then 12 stacks), so that the network starts after 6 frames
         # instead of 18; afterwards full chunks
-        for s0, ns in self._pass_plan(n_stacks, self.chunk, ready is not None, self.ramp):
-            f0 = s0 * stack_stride
-            f_hi = f0 + (ns - 1) * stack_stride + self.frames_per_stack - 1
+        for s0, ns in self._pass_plan(n_stacks, self.chunk, ready is not None and first is None, self.ramp):
+            if first is not None:
+                f_hi = max(first[0][s0:s0 + ns]) + self.frames_per_stack - 1
+            else:
+                f0 = s0 * stack_stride
+                f_hi = f0 + (ns - 1) * stack_stride + self.frames_per_stack - 1
             while ready is not None and waited < len(ready) and (waited == 0 or ready[waited - 1][0] < f_hi):
                 main.wait_event(ready[waited][1])
                 waited += 1
             if getattr(self.model, 'input_layout', 'nhwc16') == 'nchw':       # ViTPose: the reference's NCHW float32 tensor
                 with _nvtx('ttk:preprocess'):
-                    x = ops.preprocess_stacks(frames_u8[f0:f_hi + 1], self.frames_per_stack, stack_stride, ns, w, h, layout='nchw')
+                    if first is not None:
+                        x = ops.preprocess_stacks_indexed(frames_u8, self.frames_per_stack, first[1][s0:s0 + ns], w, h, layout='nchw')
+                    else:
+                        x = ops.preprocess_stacks(frames_u8[f0:f_hi + 1], self.frames_per_stack, stack_stride, ns, w, h, layout='nchw')
                 with _nvtx('ttk:heatmap_network'):
                     hm = self.model.heatmaps(x)
             else:
                 with _nvtx('ttk:preprocess'):
-                    x = ops.preprocess_stacks(frames_u8[f0:f_hi + 1], self.frames_per_stack, stack_stride, ns, w, h, layout='nhwc16', dtype=dt)
+                    if first is not None:
+                        x = ops.preprocess_stacks_indexed(frames_u8, self.frames_per_stack, first[1][s0:s0 + ns], w, h, layout='nhwc16', dtype=dt)
+                    else:
+                        x = ops.preprocess_stacks(frames_u8[f0:f_hi + 1], self.frames_per_stack, stack_stride, ns, w, h, layout='nhwc16', dtype=dt)
                 with _nvtx('ttk:heatmap_network'):
                     hm = self.model.heatmaps_from_nhwc16(x, prec)
             # interface.py:116,169 decode with the TABLE variant of extract_position_torch_gaussian.  It runs on a second stream:
@@ -453,7 +541,7 @@ class _Detector:
             except BaseException as e:      # noqa: BLE001 - handed to the thread that reads the marks
                 marks.fail(e)
 
-        _uploader().submit(run)
+        _uploader(dev_index).submit(run)
         return out, order, marks
 
 
@@ -621,6 +709,154 @@ class TableTennisPipeline:
                                                                         SEQ_LEN, WIDTH, HEIGHT)
         with _nvtx('ttk:uplift'):
             return self.uplifting_model.predict_without_normalization(ball_coords, table_coords, mask, times)
+
+    def predict_clips(self, clips, fps, devices=None):
+        """Many rallies in one call: returns [(spin, pos3d), ...], exactly [self.predict(c, fps) for c in clips] (same types, spin on
+        the same device, same values bit for bit).  clips: list of clips, each a list of HWC uint8 BGR frames like predict takes, all
+        of one frame size.
+        On one device each distinct frame is uploaded once; each detector runs full passes whose stacks come from several clips (no
+        window crosses a clip); the ball and table filters, the trajectory packing, the uplifting transformer and the spin rotation run
+        once for all clips.  Work goes a block of clips (at most _Detector.segment frames) at a time, which bounds device memory.
+        devices: None = the current device.  Otherwise a list of CUDA device indices, torch.device or 'cuda:N' strings: the clips
+        are split into contiguous blocks (sharding.shard_range), one per entry, and each entry runs the one-device path on its block
+        from a launcher thread of its own, with its own copy of the five models (built from this pipeline's models, rebuilt when their
+        state dict or compute_dtype change; the first entry on the pipeline's device uses the pipeline's models).  A device may
+        appear twice.  Only the per-clip results come back to the calling thread, whose current device stays as it was.
+        Raises ValueError, naming the clip, when predict would raise ValueError for one (0, or 50 or more agreeing ball detections:
+        the first such clip), before any uplift runs; and for a clip of fewer than 3 frames, which has no ball stack."""
+        clips = [list(c) for c in clips]
+        for i, c in enumerate(clips):
+            if len(c) < 3:
+                raise ValueError('clip %d: %d frames; a clip needs at least 3 (one (prev, cur, next) ball stack)' % (i, len(c)))
+        if devices is None:
+            if not clips:
+                return []
+            parts = self._parts()
+            packed, counts = self._detect_clips(parts, clips, fps)
+            counts = counts.cpu().tolist()
+            self._check_counts(counts, 0)
+            spin, pos = self._uplift_clips(parts, packed, counts)
+            return [(spin[i], pos[i, :c]) for i, c in enumerate(counts)]
+        idx = parse_devices(devices, torch.cuda.device_count())
+        if not clips:
+            return []
+        blocks = [sharding.shard_range(len(clips), r, len(idx)) for r in range(len(idx))]
+        home = self._home_device()          # where predict computes, and where the spins are returned
+        own = idx.index(home.index) if home.index in idx else -1
+        pool = getattr(self, '_launchers', None)
+        if pool is None or pool._max_workers < len(idx):
+            from concurrent.futures import ThreadPoolExecutor
+            pool = self._launchers = ThreadPoolExecutor(max_workers=len(idx), thread_name_prefix='ttk-launch')
+
+        def detect(r):
+            torch.cuda.set_device(idx[r])
+            parts = self._parts() if r == own else self._replica_parts(r, idx[r])
+            a, b = blocks[r]
+            if a == b:
+                return parts, None, []
+            packed, counts = self._detect_clips(parts, clips[a:b], fps)
+            return parts, packed, counts.cpu().tolist()
+
+        def uplift(r, parts, packed, counts):
+            torch.cuda.set_device(idx[r])
+            if not counts:
+                return []
+            spin, pos = self._uplift_clips(parts, packed, counts)
+            spin = spin.to(home)
+            return [(spin[i], pos[i, :c]) for i, c in enumerate(counts)]
+
+        stage1 = self._join([pool.submit(detect, r) for r in range(len(idx))])
+        for r, (_, _, counts) in enumerate(stage1):
+            self._check_counts(counts, blocks[r][0])
+        stage2 = self._join([pool.submit(uplift, r, *stage1[r]) for r in range(len(idx))])
+        return [res for part in stage2 for res in part]
+
+    @staticmethod
+    def _join(futures):
+        """Results in order, after every launcher has finished (a failing one does not leave the others running)."""
+        from concurrent.futures import wait
+        wait(futures)
+        return [f.result() for f in futures]
+
+    def _parts(self):
+        return self.ball_detector, self.ball_detector_aux, self.table_detector, self.table_detector_aux, self.uplifting_model
+
+    def _home_device(self):
+        return next(iter(self.uplifting_model.model.state_dict().values())).device
+
+    def _replica_parts(self, slot, device_index):
+        """The five models of launcher `slot` on device_index, rebuilt when the pipeline's models changed.  Runs on the launcher's
+        thread with device_index current."""
+        own = self._parts()
+        key = (device_index,) + tuple(_fingerprint(p.model) for p in own)
+        cache = self.__dict__.setdefault('_replicas', {})
+        hit = cache.get(slot)
+        if hit is not None and hit[0] == key:
+            return hit[1]
+        dev = torch.device('cuda', device_index)
+        parts = []
+        for p in own:
+            q = type(p).__new__(type(p))
+            q.__dict__.update({k: v for k, v in p.__dict__.items() if k not in ('model', '_copy_stream', '_decode_stream', '_d2h_stream',
+                                                                                  '_stage', '_stage_ev')})
+            q.device, q.model = dev, _replicate(p.model, dev)
+            parts.append(q)
+        cache[slot] = (key, tuple(parts))
+        return cache[slot][1]
+
+    def _detect_clips(self, parts, clips, fps):
+        """Detectors, both filters and the trajectory packing of `clips` on the current device, a block of clips at a time.
+        Returns the packed uplift inputs (ball, table, times, mask) of all clips and the (n,) int32 CUDA agreeing-detection counts."""
+        ball, ball_aux, table, table_aux, _ = parts
+        dev = torch.device('cuda', torch.cuda.current_device())
+        packed, counts = [], []
+        for a, b in clip_blocks([len(c) for c in clips], ball.segment):
+            lengths = [len(c) for c in clips[a:b]]
+            n = sum(lengths)
+            frames, order, ready = ball._upload([f for c in clips[a:b] for f in c], dev)
+            if order != list(range(n)):
+                torch.cuda.current_stream().wait_event(ready[-1][1])
+                frames, ready = frames[torch.tensor(order, device=dev)], None
+            bfirst, boffs = clip_stack_plan(lengths, ball.frames_per_stack)
+            tfirst, toffs = clip_stack_plan(lengths, table.frames_per_stack)
+            plan = torch.tensor(bfirst + boffs + tfirst + toffs, dtype=torch.int32).pin_memory().to(dev, non_blocking=True)
+            bfirst_d, boffs_d, tfirst_d, toffs_d = plan.split([len(bfirst), len(boffs), len(tfirst), len(toffs)])
+            with torch.no_grad():
+                bpos = ball._run(frames, 1, len(bfirst), False, ready, first=(bfirst, bfirst_d))[0][:, 0]
+                bpos_aux = ball_aux._run(frames, 1, len(bfirst), False, None, first=(bfirst, bfirst_d))[0][:, 0]
+                ball_xy, _, times_ball, offsets = ops.filter_ball_clips(bpos, bpos_aux, boffs_d, float(fps))
+                tpos = table._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
+                tpos_aux = table_aux._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
+            with _nvtx('ttk:filters_pack'):
+                tab = ops.filter_table_clips(tpos, tpos_aux, toffs_d)
+                packed.append(ops.trajectory_pack(ball_xy, times_ball, offsets, tab, SEQ_LEN, WIDTH, HEIGHT))
+                counts.append(offsets[1:] - offsets[:-1])
+        return [torch.cat(x) for x in zip(*packed)], torch.cat(counts)
+
+    @staticmethod
+    def _check_counts(counts, first_clip):
+        """predict() raises ValueError (the uplifting model's mask check) for 0 or >= SEQ_LEN agreeing detections."""
+        for i, c in enumerate(counts):
+            if c == 0 or c >= SEQ_LEN:
+                raise ValueError('clip %d (%d agreeing ball detections): %s' % (first_clip + i, c, MASK_FORMAT_ERROR))
+
+    @staticmethod
+    def _uplift_clips(parts, packed, counts):
+        """The uplifting transformer on the packed clips (one forward for all of them): spins (n, 3) on the device and positions
+        (n, SEQ_LEN, 3) as one host array."""
+        up = parts[4]
+        ball, table, times, mask = packed
+        with _nvtx('ttk:uplift'), torch.no_grad():
+            if up.model.compute_dtype == BF16:
+                # the bf16 stacks are not batch invariant: a row's tensor-core sums depend on where its keys sit in the 128-row tile,
+                # and the 1-ulp differences can flip a bf16 rounding (tests/test_gpu_full_size.py); one trajectory per forward then
+                # gives what predict computes
+                outs = [up.model(ball[i:i + 1], table[i:i + 1], mask[i:i + 1], times[i:i + 1]) for i in range(len(counts))]
+                rot, pos = torch.cat([o[0] for o in outs]), torch.cat([o[1] for o in outs])
+            else:
+                rot, pos = up.model(ball, table, mask, times)
+            spin = ops.rotation_local(rot, pos) if up.transform_mode == 'global' else rot
+        return spin, pos.cpu().numpy()
 
     def calibrate_camera(self, keypoints):
         return calibrate_camera(keypoints)

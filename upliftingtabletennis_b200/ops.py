@@ -47,6 +47,29 @@ def preprocess_stacks(frames, frames_per_stack, stack_stride, n_stacks, dst_w, d
     return out
 
 
+def preprocess_stacks_indexed(frames, frames_per_stack, first_frame, dst_w, dst_h, layout='nhwc16', dtype=torch.float32):
+    """preprocess_stacks with stack s reading frames first_frame[s] + {0..frames_per_stack-1}: first_frame is an (n_stacks,) int32
+    CUDA tensor whose entries the caller has checked against len(frames) (it is not read on the host).  Same bytes per stack."""
+    _lib.require_device()
+    assert frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 4 and frames.shape[3] == 3
+    assert first_frame.is_cuda and first_frame.dtype == torch.int32 and first_frame.dim() == 1
+    frames, first_frame = frames.contiguous(), first_frame.contiguous()
+    n, sh, sw, _ = frames.shape
+    n_stacks = first_frame.shape[0]
+    if layout == 'nchw':
+        assert dtype == torch.float32
+        shape, lay = (n_stacks, 3 * frames_per_stack, dst_h, dst_w), _lib.LAYOUT_NCHW_F32
+    else:
+        shape, lay = (n_stacks, dst_h, dst_w, 16), _lib.LAYOUT_NHWC16
+    dts = {torch.float32: _lib.F32, torch.bfloat16: _lib.BF16, torch.float16: _lib.F16}
+    if dtype not in dts:
+        raise ValueError('preprocess_stacks_indexed: dtype must be torch.float32, torch.bfloat16 or torch.float16, got %r' % (dtype,))
+    out = torch.empty(shape, dtype=dtype, device=frames.device)
+    check(lib.ttk_preprocess_stacks_indexed(ptr(frames), n, sh, sw, frames_per_stack, ptr(first_frame), n_stacks, dst_h, dst_w,
+                                            ptr(normalize_lut(frames.device)), ptr(out), lay, dts[dtype], stream_ptr()))
+    return out
+
+
 def decode_heatmaps(heatmaps, image_width, image_height, variant='table', return_debug=False):
     """heatmaps: (..., H, W) float32 CUDA tensor -> (..., 3) float64 CUDA tensor [x_img, y_img, 1].
     variant 'table': tabledetection/helper_tabledetection.py:50-156; 'ball': balldetection/helper_balldetection.py:29-110."""
@@ -127,6 +150,41 @@ def filter_ball(pos1, pos2, fps, threshold=20.0):
     check(lib.ttk_filter_ball(ptr(pos1), ptr(pos2), T, float(fps), float(threshold), ptr(xy), ptr(idx), ptr(times), ptr(offs),
                               stream_ptr()))
     return xy, idx, times, offs
+
+
+def filter_ball_clips(pos1, pos2, frame_offsets, fps, threshold=20.0):
+    """filter_ball over n clips in one launch.  pos1/pos2: (sum T, 3) float64 CUDA, the clips concatenated; frame_offsets: (n+1,)
+    int32 CUDA prefix sums of the clip lengths.  Returns xy (sum T, 2), idx (sum T,) int64 and times (sum T,) counted from each
+    clip's first frame, and offsets (n+1,) int32: clip c's kept rows are offsets[c]:offsets[c+1] -- `trajectory_pack`'s format."""
+    _lib.require_device()
+    assert pos1.is_cuda and pos1.dtype == torch.float64 and pos1.shape == pos2.shape and pos1.dim() == 2 and pos1.shape[1] == 3
+    assert frame_offsets.is_cuda and frame_offsets.dtype == torch.int32 and frame_offsets.dim() == 1
+    pos1, pos2, frame_offsets = pos1.contiguous(), pos2.contiguous(), frame_offsets.contiguous()
+    T, dev, n = pos1.shape[0], pos1.device, frame_offsets.shape[0] - 1
+    xy = torch.empty((T, 2), dtype=torch.float64, device=dev)
+    idx = torch.empty((T,), dtype=torch.int64, device=dev)
+    times = torch.empty((T,), dtype=torch.float64, device=dev)
+    offs = torch.empty((n + 1,), dtype=torch.int32, device=dev)
+    check(lib.ttk_filter_ball_clips(ptr(pos1), ptr(pos2), n, ptr(frame_offsets), T, float(fps), float(threshold), ptr(xy), ptr(idx),
+                                    ptr(times), ptr(offs), stream_ptr()))
+    return xy, idx, times, offs
+
+
+def filter_table_clips(pos1, pos2, frame_offsets, agree=10.0, eps=10.0, min_samples=3):
+    """filter_table over n clips of different lengths: pos1/pos2 (sum T, K, 3) float64 CUDA, the clips concatenated; frame_offsets
+    (n+1,) int32 CUDA prefix sums.  Returns (n, K, 3) float64, each clip bit-identical to filter_table on that clip alone."""
+    _lib.require_device()
+    assert pos1.is_cuda and pos1.dtype == torch.float64 and pos1.shape == pos2.shape and pos1.dim() == 3 and pos1.shape[-1] == 3
+    assert frame_offsets.is_cuda and frame_offsets.dtype == torch.int32 and frame_offsets.dim() == 1
+    a, b, frame_offsets = pos1.contiguous(), pos2.contiguous(), frame_offsets.contiguous()
+    T, K, _ = a.shape
+    n = frame_offsets.shape[0] - 1
+    out = torch.empty((n, K, 3), dtype=torch.float64, device=a.device)
+    ws_bytes = lib.ttk_filter_table_workspace_bytes(1, T, K)
+    ws = torch.empty((max(ws_bytes, 8),), dtype=torch.uint8, device=a.device)
+    check(lib.ttk_filter_table_clips(ptr(a), ptr(b), n, ptr(frame_offsets), T, K, float(agree), float(eps), int(min_samples), ptr(out),
+                                     ptr(ws), ws_bytes, stream_ptr()))
+    return out
 
 
 def filter_table(pos1, pos2, agree=10.0, eps=10.0, min_samples=3):

@@ -13,6 +13,7 @@ from ._lib import lib, check, ptr, stream_ptr
 from .detector import _attach
 from .precision import BF16, FP32, TF32X3, PrecisionMixin, lib_enum
 
+MASK_FORMAT_ERROR = 'wrong format for masks. Should be 0, 1 or -1e9, 0.'
 SIZES = {'small': (32, 8, 4), 'base': (64, 12, 4), 'large': (128, 16, 4), 'huge': (192, 16, 8)}   # uplifting/model.py:574-603
 PARAM_SHAPES = {'cls_token': lambda d: (1, 1, d)}
 
@@ -103,6 +104,7 @@ class MultiStageModel(PrecisionMixin, nn.Module):
             raise NotImplementedError("only tabletoken_mode='dynamic' with time_rotation='new' (the released 'ours' model) has kernels")
         self.engine = UpliftEngine(dim, num_heads, depth, use_skipconnection)
         self.dim, self.mode, self.time_rotation, self.use_skipconnection = dim, mode, time_rotation, use_skipconnection
+        self.depth, self.num_heads = depth, num_heads
         for name, numel in self.engine.params:
             shape = _shape_of(name, numel, dim)
             assert int(torch.tensor(shape).prod()) == numel, (name, shape, numel)
@@ -126,7 +128,7 @@ class MultiStageModel(PrecisionMixin, nn.Module):
         elif mx == 0 and mn < -1e8:
             additive = True
         else:
-            raise ValueError('wrong format for masks. Should be 0, 1 or -1e9, 0.')
+            raise ValueError(MASK_FORMAT_ERROR)
         self._sync()
         return self.engine.forward(ball_pos, table_pos, mask, times, self.compute_dtype, mask_additive=additive)
 
