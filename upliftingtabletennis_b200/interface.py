@@ -451,36 +451,48 @@ class _Detector:
                 hms.append(hm.numpy())          # (a view of the pinned block; the array keeps it alive)
         return (pos[0] if len(pos) == 1 else np.concatenate(pos)), ((hms[0] if len(hms) == 1 else np.concatenate(hms)) if return_heatmaps else None)
 
-    def _upload(self, images, dev):
+    def _upload(self, images, dev, out=None):
         """Upload each distinct frame once, asynchronously on a copy stream.  numpy frames (pageable memory, what cv2 delivers) go
         through a small ring of pinned staging slots: host threads copy frame i into slot i % stage_slots (numpy releases the GIL for
         it) as soon as the transfer that last used the slot has finished (one event per slot -- no stream-wide synchronisation), and
         the slot is sent as soon as it is staged, so the host memcpy pipelines with the PCIe transfer.  torch CPU tensors (e.g.
         already pinned) are copied directly.  Returns the (n, H, W, 3) uint8 CUDA tensor, per input image its row in it, and
-        [(frame index, event)] marking how far the copy has got."""
+        [(frame index, event)] marking how far the copy has got.
+        out: a (len(images), H, W, 3) uint8 CUDA tensor to write into instead (a slice of a LiveSession's frame pool): every image gets
+        its own row, in order, host tensors too go through the staging ring, and the caller keeps `out` alive until the copy stream
+        has passed the last mark."""
         torch.cuda.nvtx.range_push('ttk:upload')
         try:
-            return self._upload_frames(images, dev)
+            return self._upload_frames(images, dev, out)
         finally:
             torch.cuda.nvtx.range_pop()
 
-    def _upload_frames(self, images, dev):
+    def _upload_frames(self, images, dev, out=None):
         slots, order, uniq = {}, [], []
-        for im in images:
-            # frames are recognised by their memory, not by the Python object: clip[i] creates a new view object on every indexing,
-            # and a sliding window over a clip names every frame three times
-            k = self._frame_key(im)
-            if k not in slots:
-                slots[k] = len(uniq)
-                uniq.append(im)
-            order.append(slots[k])
+        if out is not None:
+            uniq, order = list(images), list(range(len(images)))
+        else:
+            for im in images:
+                # frames are recognised by their memory, not by the Python object: clip[i] creates a new view object on every indexing,
+                # and a sliding window over a clip names every frame three times
+                k = self._frame_key(im)
+                if k not in slots:
+                    slots[k] = len(uniq)
+                    uniq.append(im)
+                order.append(slots[k])
         fshape = tuple(uniq[0].shape)
         for u in uniq:
             if tuple(u.shape) != fshape or len(fshape) != 3 or fshape[2] != 3 or (u.dtype != torch.uint8 if isinstance(u, torch.Tensor) else u.dtype != np.uint8):
                 raise ValueError('frames must be uint8 arrays of one common shape (H, W, 3); got %s %s (first frame %s)' % (tuple(u.shape), u.dtype, fshape))
         n = len(uniq)
-        out = torch.empty((n,) + fshape, dtype=torch.uint8, device=dev)
-        all_torch = all(isinstance(u, torch.Tensor) for u in uniq)
+        own = out is None
+        if own:
+            out = torch.empty((n,) + fshape, dtype=torch.uint8, device=dev)
+        elif tuple(out.shape) != (n,) + fshape:
+            raise ValueError('upload target of shape %s for %d frames of shape %s' % (tuple(out.shape), n, fshape))
+        # into a given `out` (LiveSession.push), host tensors are staged like numpy frames: the caller may reuse them once the marks
+        # are recorded, whereas a direct non_blocking copy from pinned memory would still be reading them
+        all_torch = all(isinstance(u, torch.Tensor) and (own or u.is_cuda) for u in uniq)
         copy_stream = getattr(self, '_copy_stream', None)
         if copy_stream is None:
             copy_stream = self._copy_stream = torch.cuda.Stream(device=dev)
@@ -507,7 +519,8 @@ class _Detector:
         view, slot_ev = stage.numpy(), self._stage_ev
         slot_ptr = [stage[k].data_ptr() for k in range(ns)]
         marks = _ReadyMarks([i for i in range(n) if i % 2 == 1 or i == n - 1])      # an event every other frame: the first pass (4 stacks) starts after 6 frames
-        out.record_stream(copy_stream)
+        if own:
+            out.record_stream(copy_stream)
         dev_index = torch.cuda.current_device()
 
         def stage_one(i, ev):
@@ -700,15 +713,29 @@ class TableTennisPipeline:
         with torch.no_grad():
             ball_positions = self.ball_detector._run(frames, 1, n - 2, False, ready)[0][:, 0]       # sliding (prev, cur, next) window
             ball_positions_aux = self.ball_detector_aux._run(frames, 1, n - 2, False, None)[0][:, 0]
-            ball_xy, _, times_ball, offsets = ops.filter_ball(ball_positions, ball_positions_aux, float(fps))
             table_keypoints = self.table_detector._run(frames, 1, n, False, None)[0]
             table_keypoints_aux = self.table_detector_aux._run(frames, 1, n, False, None)[0]
+        return self._tail(ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps)
+
+    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps):
+        """predict's steps after the four detectors, shared with LiveSession.end_rally: the ball filter, the table filters, the
+        trajectory packing, the uplifting transformer and the spin rotation.  Takes the (n - 2, 3) ball and (n, K, 3) table positions
+        of one clip on the device; returns predict's (spin, pos3d)."""
+        ball_xy, _, times_ball, offsets = ops.filter_ball(ball_positions, ball_positions_aux, float(fps))
         with _nvtx('ttk:filters_pack'):
             filtered_table_keypoints = ops.filter_table(table_keypoints, table_keypoints_aux)
             ball_coords, table_coords, times, mask = ops.trajectory_pack(ball_xy, times_ball, offsets, filtered_table_keypoints[None],
                                                                         SEQ_LEN, WIDTH, HEIGHT)
         with _nvtx('ttk:uplift'):
             return self.uplifting_model.predict_without_normalization(ball_coords, table_coords, mask, times)
+
+    def live(self, fps, streams=1, k=None, slots=None):
+        """A LiveSession (upliftingtabletennis_b200/live.py) over `streams` cameras at `fps`: frames are pushed as they arrive, the
+        detectors run on them while the rally goes on, and end_rally(stream) returns exactly what predict(the rally's frames, fps)
+        returns.  k: ready stacks that launch a detector pass (default live.DEFAULT_K); slots: device frame slots per stream (default
+        live.DEFAULT_SLOTS)."""
+        from .live import LiveSession
+        return LiveSession(self, fps, streams, k, slots)
 
     def predict_clips(self, clips, fps, devices=None):
         """Many rallies in one call: returns [(spin, pos3d), ...], exactly [self.predict(c, fps) for c in clips] (same types, spin on
