@@ -717,25 +717,29 @@ class TableTennisPipeline:
             table_keypoints_aux = self.table_detector_aux._run(frames, 1, n, False, None)[0]
         return self._tail(ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps)
 
-    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps):
+    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps, uplifting_model=None):
         """predict's steps after the four detectors, shared with LiveSession.end_rally: the ball filter, the table filters, the
         trajectory packing, the uplifting transformer and the spin rotation.  Takes the (n - 2, 3) ball and (n, K, 3) table positions
-        of one clip on the device; returns predict's (spin, pos3d)."""
+        of one clip on the device; returns predict's (spin, pos3d).  uplifting_model: a replica of self.uplifting_model to run instead
+        (on the positions' device)."""
+        up = self.uplifting_model if uplifting_model is None else uplifting_model
         ball_xy, _, times_ball, offsets = ops.filter_ball(ball_positions, ball_positions_aux, float(fps))
         with _nvtx('ttk:filters_pack'):
             filtered_table_keypoints = ops.filter_table(table_keypoints, table_keypoints_aux)
             ball_coords, table_coords, times, mask = ops.trajectory_pack(ball_xy, times_ball, offsets, filtered_table_keypoints[None],
                                                                         SEQ_LEN, WIDTH, HEIGHT)
         with _nvtx('ttk:uplift'):
-            return self.uplifting_model.predict_without_normalization(ball_coords, table_coords, mask, times)
+            return up.predict_without_normalization(ball_coords, table_coords, mask, times)
 
-    def live(self, fps, streams=1, k=None, slots=None):
+    def live(self, fps, streams=1, k=None, slots=None, devices=None):
         """A LiveSession (upliftingtabletennis_b200/live.py) over `streams` cameras at `fps`: frames are pushed as they arrive, the
         detectors run on them while the rally goes on, and end_rally(stream) returns exactly what predict(the rally's frames, fps)
         returns.  k: ready stacks that launch a detector pass (default live.DEFAULT_K); slots: device frame slots per stream (default
-        live.DEFAULT_SLOTS)."""
+        live.DEFAULT_SLOTS).  devices: None = the current device, passes launched on the caller's thread; or a list of CUDA devices
+        as predict_clips takes: entry r serves streams sharding.shard_range(streams, r, len(devices)) on devices[r], with its own
+        copy of the models and a launcher thread of its own; k and slots apply per entry."""
         from .live import LiveSession
-        return LiveSession(self, fps, streams, k, slots)
+        return LiveSession(self, fps, streams, k, slots, devices)
 
     def predict_clips(self, clips, fps, devices=None):
         """Many rallies in one call: returns [(spin, pos3d), ...], exactly [self.predict(c, fps) for c in clips] (same types, spin on
