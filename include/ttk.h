@@ -326,6 +326,16 @@ TTK_API int ttk_rotation_local(const float* rot_dev, const float* pos_dev, int b
  * path of the reference), else float32 (its torch path). */
 TTK_API int ttk_project(const void* points_dev, const void* mext_dev, const void* mint_dev, int n,
                 int dtype_f64, void* out_dev, void* stream);
+/* ttk_project (float64) over n_clips clips of different lengths, each with its own camera, and each clip's reprojection error.
+ * points_dev: the clips' n_points x 3 points concatenated; offsets_dev[n_clips+1] int32 (device): clip c is rows [offs[c], offs[c+1]),
+ * offs[0] = 0, non-decreasing, offs[n_clips] = n_points -- the format ttk_filter_ball_clips writes.  mint_dev n_clips x 3 x 4 (its
+ * leading 3x3 is used), mext_dev n_clips x 4 x 4, float64; valid_dev n_clips int32; det_xy_dev n_points x 2 float64, the 2D detection
+ * of each row.  out_xy_dev n_points x 2: every point bit-identical to ttk_project(dtype_f64 = 1) on its clip alone.  out_err_dev
+ * n_clips x 2: mean and max over the clip's rows of the Euclidean distance between reprojection and detection, the mean summed in row
+ * order (NaN for an empty clip).  A clip with valid == 0 gets NaN points and errors. */
+TTK_API int ttk_reproject_clips(const double* points_dev, int n_points, const int32_t* offsets_dev, int n_clips,
+                const double* mint_dev, const double* mext_dev, const int32_t* valid_dev, const double* det_xy_dev,
+                double* out_xy_dev, double* out_err_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -3,7 +3,7 @@
 # Usage (on the GPU box): bash tools/run_sanitizer.sh [outdir]   -- logs go to <outdir>/sanitizer_<tool>.log
 out=${1:-gpurun_out}
 mkdir -p "$out"
-TESTS="tests/test_gpu_conv_umma.py::test_every_conv_umma_vs_simt_and_cpu[shape1] tests/test_gpu_output_parity.py::test_every_conv_tf32_vs_exact_tf32_arithmetic[shape1] tests/test_gpu_conv_umma.py::test_fused_basic_block_vs_separate_convs_and_cpu[shape2] tests/test_gpu_vitpose.py::test_gemm_umma[2100-1152-384-0-False-True] tests/test_gpu_vitpose.py::test_gemm_umma[300-384-384-0-True-False] tests/test_gpu_vitpose.py::test_gemm_umma[130-128-64-2-False-True] tests/test_gpu_vitpose.py::test_attention_umma[2-128] tests/test_gpu_vitpose.py::test_attention_umma[3-60] tests/test_gpu_parity.py::test_uplift_bf16_tensor_core_bound tests/test_gpu_parity.py::test_uplift_golden[connectstage-tf32x3] tests/test_gpu_vitpose.py::test_gemm_x3[300-384-384-0-True-False] tests/test_gpu_vitpose.py::test_gemm_x3[24-1152-384-0-False-True] tests/test_gpu_vitpose.py::test_attention_x3[2-128] tests/test_gpu_vitpose.py::test_attention_x3[3-60] tests/test_gpu_vitpose.py::test_vitpose_x3_vs_oracle[res0-2] tests/test_gpu_conv_umma.py::test_network_block_fusion_tf32"
+TESTS="tests/test_gpu_conv_umma.py::test_every_conv_umma_vs_simt_and_cpu[shape1] tests/test_gpu_output_parity.py::test_every_conv_tf32_vs_exact_tf32_arithmetic[shape1] tests/test_gpu_conv_umma.py::test_fused_basic_block_vs_separate_convs_and_cpu[shape2] tests/test_gpu_vitpose.py::test_gemm_umma[2100-1152-384-0-False-True] tests/test_gpu_vitpose.py::test_gemm_umma[300-384-384-0-True-False] tests/test_gpu_vitpose.py::test_gemm_umma[130-128-64-2-False-True] tests/test_gpu_vitpose.py::test_attention_umma[2-128] tests/test_gpu_vitpose.py::test_attention_umma[3-60] tests/test_gpu_parity.py::test_uplift_bf16_tensor_core_bound tests/test_gpu_parity.py::test_uplift_golden[connectstage-tf32x3] tests/test_gpu_vitpose.py::test_gemm_x3[300-384-384-0-True-False] tests/test_gpu_vitpose.py::test_gemm_x3[24-1152-384-0-False-True] tests/test_gpu_vitpose.py::test_attention_x3[2-128] tests/test_gpu_vitpose.py::test_attention_x3[3-60] tests/test_gpu_vitpose.py::test_vitpose_x3_vs_oracle[res0-2] tests/test_gpu_conv_umma.py::test_network_block_fusion_tf32 tests/test_gpu_rally_cameras.py::test_reproject_clips_equals_project_per_clip tests/test_gpu_rally_cameras.py::test_reproject_clips_invalid_clips_are_nan"
 # gemm3_umma_kernel (uplift tf32x3) uses 232 064 of the 232 448 bytes of shared memory a CTA can have; synccheck keeps its barrier
 # bookkeeping in shared memory too and then reports "Missing init" for every mbarrier wait of that kernel (and kills it), while the
 # same kernel built with a 2-stage ring (32 KB less) is clean.  So synccheck runs without the tf32x3 uplift tests on the stock library,

@@ -84,6 +84,7 @@ def _load():
         'ttk_uplift_debug_attention3': (i32, [i32, i32, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]),
         'ttk_rotation_local': (i32, [vp, vp, i32, i32, vp, vp]),
         'ttk_project': (i32, [vp, vp, vp, i32, i32, vp, vp]),
+        'ttk_reproject_clips': (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)       # AttributeError if include/ttk.h and the library disagree

@@ -2,6 +2,7 @@
 //   ttk_trajectory_pack : inference/utils.py:268-309 (_uplifting_transform), batched over clips
 //   ttk_rotation_local  : uplifting/helper.py:394-420 (transform_rotationaxes)
 //   ttk_project         : uplifting/helper.py:137-204 (world2cam, cam2img), interface.py:301-312
+//   ttk_reproject_clips : ttk_project over many clips of different lengths, each with its own camera, plus the reprojection error
 #include "ttk_internal.h"
 
 namespace {
@@ -51,6 +52,21 @@ __global__ void rotation_local_kernel(const float* __restrict__ rot, const float
   out[b * 3 + 2] = r2;
 }
 
+// cam2img(world2cam(p)) of one point with the matrices in shared memory: s_e the 4x4 Mext, s_i the leading 3x3 of Mint, both row
+// major.  project_kernel and reproject_clips_kernel both call it, so a point comes out with the same bits from either.
+template <typename T>
+__device__ __forceinline__ void project_point(const T* s_e, const T* s_i, T x, T y, T z, T& u, T& v) {
+  T c[4];
+#pragma unroll
+  for (int r = 0; r < 4; ++r) c[r] = s_e[r * 4] * x + s_e[r * 4 + 1] * y + s_e[r * 4 + 2] * z + s_e[r * 4 + 3];
+  const T cx = c[0] / c[3], cy = c[1] / c[3], cz = c[2] / c[3];
+  T q[3];
+#pragma unroll
+  for (int r = 0; r < 3; ++r) q[r] = s_i[r * 3] * cx + s_i[r * 3 + 1] * cy + s_i[r * 3 + 2] * cz;
+  u = q[0] / q[2];
+  v = q[1] / q[2];
+}
+
 template <typename T>
 __global__ void project_kernel(const T* __restrict__ pts, const T* __restrict__ mext, const T* __restrict__ mint, int n,
                                T* __restrict__ out) {
@@ -60,16 +76,57 @@ __global__ void project_kernel(const T* __restrict__ pts, const T* __restrict__ 
   __syncthreads();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  const T x = pts[(size_t)i * 3], y = pts[(size_t)i * 3 + 1], z = pts[(size_t)i * 3 + 2];
-  T c[4];
-#pragma unroll
-  for (int r = 0; r < 4; ++r) c[r] = s_e[r * 4] * x + s_e[r * 4 + 1] * y + s_e[r * 4 + 2] * z + s_e[r * 4 + 3];
-  const T cx = c[0] / c[3], cy = c[1] / c[3], cz = c[2] / c[3];
-  T q[3];
-#pragma unroll
-  for (int r = 0; r < 3; ++r) q[r] = s_i[r * 3] * cx + s_i[r * 3 + 1] * cy + s_i[r * 3 + 2] * cz;
-  out[(size_t)i * 2] = q[0] / q[2];
-  out[(size_t)i * 2 + 1] = q[1] / q[2];
+  T u, v;
+  project_point(s_e, s_i, pts[(size_t)i * 3], pts[(size_t)i * 3 + 1], pts[(size_t)i * 3 + 2], u, v);
+  out[(size_t)i * 2] = u;
+  out[(size_t)i * 2 + 1] = v;
+}
+
+constexpr int RC_THREADS = 128;
+
+// one CTA per clip: its points offs[c] .. offs[c+1]-1 through project_point with the clip's Mext and the leading 3x3 of its (3, 4) Mint,
+// and the Euclidean distance of each to the detection of the same row.  Thread 0 sums the distances in row order (sequential float64
+// adds) and keeps the largest, so that a host loop over the rows gives the same bits; a NaN distance makes both NaN.  A clip with
+// valid[c] == 0 writes NaN for its points and errors.
+__global__ void __launch_bounds__(RC_THREADS) reproject_clips_kernel(const double* __restrict__ pts, const int32_t* __restrict__ offs,
+                                                                     const double* __restrict__ mint, const double* __restrict__ mext,
+                                                                     const int32_t* __restrict__ valid, const double* __restrict__ det,
+                                                                     double* __restrict__ out, double* __restrict__ err) {
+  __shared__ double s_e[16], s_i[9], s_d[RC_THREADS];
+  const int clip = blockIdx.x;
+  const int begin = offs[clip], n = offs[clip + 1] - begin;
+  const bool ok = valid[clip] != 0;
+  const double nan = __longlong_as_double(0x7ff8000000000000LL);
+  if (threadIdx.x < 16) s_e[threadIdx.x] = mext[(size_t)clip * 16 + threadIdx.x];
+  if (threadIdx.x < 9) s_i[threadIdx.x] = mint[(size_t)clip * 12 + (threadIdx.x / 3) * 4 + threadIdx.x % 3];
+  __syncthreads();
+  double sum = 0.0, worst = nan;
+  for (int t0 = 0; t0 < n; t0 += RC_THREADS) {
+    const int t = t0 + threadIdx.x;
+    if (t < n) {
+      const size_t r = (size_t)begin + t;
+      double u = nan, v = nan;
+      if (ok) project_point(s_e, s_i, pts[r * 3], pts[r * 3 + 1], pts[r * 3 + 2], u, v);
+      out[r * 2] = u;
+      out[r * 2 + 1] = v;
+      const double dx = __dsub_rn(u, det[r * 2]), dy = __dsub_rn(v, det[r * 2 + 1]);
+      s_d[threadIdx.x] = sqrt(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      const int m = min(RC_THREADS, n - t0);
+      for (int i = 0; i < m; ++i) {
+        const double d = s_d[i];
+        sum = __dadd_rn(sum, d);
+        if (t0 + i == 0 || d > worst || isnan(d)) worst = d;
+      }
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    err[(size_t)clip * 2] = ok ? sum / (double)n : nan;         // n == 0: 0 / 0, NaN
+    err[(size_t)clip * 2 + 1] = ok ? worst : nan;
+  }
 }
 
 }  // namespace
@@ -108,6 +165,19 @@ extern "C" int ttk_project(const void* points_dev, const void* mext_dev, const v
   else
     project_kernel<float><<<ttk_cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>((const float*)points_dev, (const float*)mext_dev,
                                                                             (const float*)mint_dev, n, (float*)out_dev);
+  TTK_LAUNCH_CHECK();
+  return TTK_OK;
+}
+
+extern "C" int ttk_reproject_clips(const double* points_dev, int n_points, const int32_t* offsets_dev, int n_clips, const double* mint_dev,
+                                   const double* mext_dev, const int32_t* valid_dev, const double* det_xy_dev, double* out_xy_dev,
+                                   double* out_err_dev, void* stream) {
+  TTK_CHECK_ARG(n_clips >= 0 && n_points >= 0, "ttk_reproject_clips: bad sizes");
+  if (n_clips == 0) return TTK_OK;
+  TTK_CHECK_ARG(offsets_dev && mint_dev && mext_dev && valid_dev && out_err_dev, "ttk_reproject_clips: null pointer");
+  TTK_CHECK_ARG(n_points == 0 || (points_dev && det_xy_dev && out_xy_dev), "ttk_reproject_clips: null pointer");
+  reproject_clips_kernel<<<n_clips, RC_THREADS, 0, (cudaStream_t)stream>>>(points_dev, offsets_dev, mint_dev, mext_dev, valid_dev,
+                                                                           det_xy_dev, out_xy_dev, out_err_dev);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }

@@ -7,6 +7,7 @@ round-trip per frame), and the segformer++ detectors, whose architecture is not 
 repository (fetched from another hub repo at construction time, ``balldetection/models/segformer_pp.py:12-19``),
 are substituted by the in-repo WASB / HRNet architectures unless their weights are unavailable.
 """
+import collections
 import os
 import zipfile
 
@@ -630,6 +631,16 @@ class TableDetector(_Detector):
         return filter_trajectory_table(table_keypoints, table_keypoints_aux)
 
 
+def calibration_error(info):
+    """The message of the ValueError that calibrate_camera raises for a clip whose ops.calibrate_camera info row (inliers, best
+    hypothesis, BFGS status, DLT ok) is `info`, or None when the calibration succeeded."""
+    if not info[3]:
+        return "Intrinsic matrix K has K[2,2] close to zero, indicating a degenerate camera."      # my_dlt.py:128
+    if info[0] == 0:
+        return "RANSAC failed to find a valid model."
+    return None
+
+
 def calibrate_camera(table_coords):
     """inference/utils.py:312-329: DLT start + 100-hypothesis RANSAC of BFGS fits + refit on the inliers
     (dataprocessing/regress_cameramatrices.py), all hypotheses concurrently on the GPU (ttk_calibrate_camera).
@@ -638,12 +649,56 @@ def calibrate_camera(table_coords):
     samples = ops.ransac_sample_table(kp)
     dev = _device()
     mint, mext, info = ops.calibrate_camera(torch.from_numpy(kp).to(dev), torch.from_numpy(samples).to(dev), WIDTH, HEIGHT)
-    info = info.cpu().numpy()[0]
-    if not info[3]:
-        raise ValueError("Intrinsic matrix K has K[2,2] close to zero, indicating a degenerate camera.")     # my_dlt.py:128
-    if info[0] == 0:
-        raise ValueError("RANSAC failed to find a valid model.")
+    error = calibration_error(info.cpu().numpy()[0])
+    if error is not None:
+        raise ValueError(error)
     return mint[0].cpu().numpy(), mext[0].cpu().numpy()
+
+
+RallyCamera = collections.namedtuple('RallyCamera', ['keypoints', 'Mint', 'Mext', 'ball_2d', 'detections_2d', 'error_px', 'error'])
+RallyCamera.__doc__ = """The camera of one rally and its ball path in the image (predict_clips / LiveSession.end_rally with cameras=True).
+keypoints      (13, 3) float64: the filtered table keypoints, filter_trajectory_table(table_kp, table_kp_aux) of the rally
+Mint, Mext     (3, 4), (4, 4) float64: calibrate_camera(keypoints), or None when it raises
+ball_2d        (T', 2) float64: reproject(pos3d, Mint, Mext), or None
+detections_2d  (T', 2) float64: the filtered ball detections the uplift used, row t belonging to pos3d[t]
+error_px       (mean, max) Euclidean distance in pixels between ball_2d and detections_2d, or None
+error          None, or the message of the exception calibrate_camera(keypoints) raises: AssertionError for fewer than 6 visible
+               keypoints, ValueError for a degenerate camera or a RANSAC failure"""
+
+
+def _rally_cameras(keypoints, det_xy, counts, positions):
+    """RallyCamera records of n rallies, computed on keypoints' device: keypoints (n, 13, 3) float64 CUDA, the filtered table keypoints;
+    det_xy (sum T', 2) float64 CUDA, the rallies' filtered ball detections one after the other; counts, the T' of each; positions, the
+    rallies' (T', 3) pos3d.  One calibration over the rallies with at least 6 visible keypoints (the others fail as the reference's
+    sample draw does) and one ttk_reproject_clips launch for all; each result equals calibrate_camera / reproject on its rally alone."""
+    dev = keypoints.device
+    n = len(counts)
+    kp = keypoints.cpu().numpy()            # the records' keypoints, and the visibility the sample tables depend on
+    enough = np.flatnonzero((kp[:, :, 2] == KEYPOINT_VISIBLE).sum(axis=1) >= ops.RANSAC_POINTS)
+    mint = torch.zeros((n, 3, 4), dtype=torch.float64, device=dev)
+    mext = torch.zeros((n, 4, 4), dtype=torch.float64, device=dev)
+    valid = torch.zeros((n,), dtype=torch.int32, device=dev)
+    info = None
+    if len(enough):
+        sel = torch.from_numpy(enough).to(dev)
+        samples = torch.from_numpy(ops.ransac_sample_table_cached(kp[enough])).to(dev)
+        mi, me, info = ops.calibrate_camera(keypoints[sel], samples, WIDTH, HEIGHT)
+        mint[sel], mext[sel] = mi, me
+        valid[sel] = ((info[:, 3] != 0) & (info[:, 0] != 0)).to(torch.int32)
+    offsets = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+    points = torch.from_numpy(np.concatenate(positions).astype(np.float64)).to(dev)
+    xy, err = ops.reproject_clips(points, torch.from_numpy(offsets).to(dev), mint, mext, valid, det_xy)
+    info = {} if info is None else dict(zip(enough.tolist(), info.cpu().numpy()))
+    mint, mext, xy, err, det = (t.cpu().numpy() for t in (mint, mext, xy, err, det_xy))
+    out = []
+    for i in range(n):
+        a, b = offsets[i], offsets[i + 1]
+        error = calibration_error(info[i]) if i in info else ops.TOO_FEW_POINTS
+        if error is None:
+            out.append(RallyCamera(kp[i], mint[i], mext[i], xy[a:b], det[a:b], (float(err[i, 0]), float(err[i, 1])), None))
+        else:
+            out.append(RallyCamera(kp[i], None, None, None, det[a:b], None, error))
+    return out
 
 
 class UpliftingModel:
@@ -717,11 +772,11 @@ class TableTennisPipeline:
             table_keypoints_aux = self.table_detector_aux._run(frames, 1, n, False, None)[0]
         return self._tail(ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps)
 
-    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps, uplifting_model=None):
+    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps, uplifting_model=None, cameras=False):
         """predict's steps after the four detectors, shared with LiveSession.end_rally: the ball filter, the table filters, the
         trajectory packing, the uplifting transformer and the spin rotation.  Takes the (n - 2, 3) ball and (n, K, 3) table positions
         of one clip on the device; returns predict's (spin, pos3d).  uplifting_model: a replica of self.uplifting_model to run instead
-        (on the positions' device)."""
+        (on the positions' device).  cameras: return (spin, pos3d, RallyCamera) instead."""
         up = self.uplifting_model if uplifting_model is None else uplifting_model
         ball_xy, _, times_ball, offsets = ops.filter_ball(ball_positions, ball_positions_aux, float(fps))
         with _nvtx('ttk:filters_pack'):
@@ -729,7 +784,11 @@ class TableTennisPipeline:
             ball_coords, table_coords, times, mask = ops.trajectory_pack(ball_xy, times_ball, offsets, filtered_table_keypoints[None],
                                                                         SEQ_LEN, WIDTH, HEIGHT)
         with _nvtx('ttk:uplift'):
-            return up.predict_without_normalization(ball_coords, table_coords, mask, times)
+            spin, pos3d = up.predict_without_normalization(ball_coords, table_coords, mask, times)
+        if not cameras:
+            return spin, pos3d
+        with _nvtx('ttk:cameras'):
+            return spin, pos3d, _rally_cameras(filtered_table_keypoints[None], ball_xy[:len(pos3d)], [len(pos3d)], [pos3d])[0]
 
     def live(self, fps, streams=1, k=None, slots=None, devices=None):
         """A LiveSession (upliftingtabletennis_b200/live.py) over `streams` cameras at `fps`: frames are pushed as they arrive, the
@@ -741,7 +800,7 @@ class TableTennisPipeline:
         from .live import LiveSession
         return LiveSession(self, fps, streams, k, slots, devices)
 
-    def predict_clips(self, clips, fps, devices=None):
+    def predict_clips(self, clips, fps, devices=None, cameras=False):
         """Many rallies in one call: returns [(spin, pos3d), ...], exactly [self.predict(c, fps) for c in clips] (same types, spin on
         the same device, same values bit for bit).  clips: list of clips, each a list of HWC uint8 BGR frames like predict takes, all
         of one frame size.
@@ -754,7 +813,12 @@ class TableTennisPipeline:
         state dict or compute_dtype change; the first entry on the pipeline's device uses the pipeline's models).  A device may
         appear twice.  Only the per-clip results come back to the calling thread, whose current device stays as it was.
         Raises ValueError, naming the clip, when predict would raise ValueError for one (0, or 50 or more agreeing ball detections:
-        the first such clip), before any uplift runs; and for a clip of fewer than 3 frames, which has no ball stack."""
+        the first such clip), before any uplift runs; and for a clip of fewer than 3 frames, which has no ball stack.
+        cameras: each result becomes (spin, pos3d, camera), camera a RallyCamera: the clip's filtered table keypoints, the
+        calibrate_camera matrices, reproject(pos3d, Mint, Mext), the filtered ball detections the uplift used and the pixel error between
+        the two; a clip whose calibration fails reports the message in camera.error instead of raising.  The keypoints and detections
+        are the ones the pipeline computed anyway; per device one calibration over its clips and one reprojection launch are added, on
+        the device and stream of the uplift.  cameras=False launches and synchronises nothing of this."""
         clips = [list(c) for c in clips]
         for i, c in enumerate(clips):
             if len(c) < 3:
@@ -763,11 +827,12 @@ class TableTennisPipeline:
             if not clips:
                 return []
             parts = self._parts()
-            packed, counts = self._detect_clips(parts, clips, fps)
+            packed, counts, kept = self._detect_clips(parts, clips, fps)
             counts = counts.cpu().tolist()
             self._check_counts(counts, 0)
             spin, pos = self._uplift_clips(parts, packed, counts)
-            return [(spin[i], pos[i, :c]) for i, c in enumerate(counts)]
+            out = [(spin[i], pos[i, :c]) for i, c in enumerate(counts)]
+            return self._with_cameras(out, kept, counts) if cameras else out
         idx = parse_devices(devices, torch.cuda.device_count())
         if not clips:
             return []
@@ -784,20 +849,23 @@ class TableTennisPipeline:
             parts = self._parts() if r == own else self._replica_parts(r, idx[r])
             a, b = blocks[r]
             if a == b:
-                return parts, None, []
-            packed, counts = self._detect_clips(parts, clips[a:b], fps)
-            return parts, packed, counts.cpu().tolist()
+                return parts, None, [], None
+            packed, counts, kept = self._detect_clips(parts, clips[a:b], fps)
+            return parts, packed, counts.cpu().tolist(), kept
 
-        def uplift(r, parts, packed, counts):
+        def uplift(r, parts, packed, counts, kept):
             torch.cuda.set_device(idx[r])
             if not counts:
                 return []
             spin, pos = self._uplift_clips(parts, packed, counts)
+            out = [(spin[i], pos[i, :c]) for i, c in enumerate(counts)]
+            if cameras:
+                out = self._with_cameras(out, kept, counts)
             spin = spin.to(home)
-            return [(spin[i], pos[i, :c]) for i, c in enumerate(counts)]
+            return [(spin[i],) + res[1:] for i, res in enumerate(out)]
 
         stage1 = self._join([pool.submit(detect, r) for r in range(len(idx))])
-        for r, (_, _, counts) in enumerate(stage1):
+        for r, (_, _, counts, _) in enumerate(stage1):
             self._check_counts(counts, blocks[r][0])
         stage2 = self._join([pool.submit(uplift, r, *stage1[r]) for r in range(len(idx))])
         return [res for part in stage2 for res in part]
@@ -837,10 +905,12 @@ class TableTennisPipeline:
 
     def _detect_clips(self, parts, clips, fps):
         """Detectors, both filters and the trajectory packing of `clips` on the current device, a block of clips at a time.
-        Returns the packed uplift inputs (ball, table, times, mask) of all clips and the (n,) int32 CUDA agreeing-detection counts."""
+        Returns the packed uplift inputs (ball, table, times, mask) of all clips, the (n,) int32 CUDA agreeing-detection counts and,
+        per block, its filtered table keypoints (clips, 13, 3) and ball detections (rows of its clips in order, then unused capacity):
+        what _with_cameras reads."""
         ball, ball_aux, table, table_aux, _ = parts
         dev = torch.device('cuda', torch.cuda.current_device())
-        packed, counts = [], []
+        packed, counts, kept = [], [], []
         for a, b in clip_blocks([len(c) for c in clips], ball.segment):
             lengths = [len(c) for c in clips[a:b]]
             n = sum(lengths)
@@ -862,7 +932,21 @@ class TableTennisPipeline:
                 tab = ops.filter_table_clips(tpos, tpos_aux, toffs_d)
                 packed.append(ops.trajectory_pack(ball_xy, times_ball, offsets, tab, SEQ_LEN, WIDTH, HEIGHT))
                 counts.append(offsets[1:] - offsets[:-1])
-        return [torch.cat(x) for x in zip(*packed)], torch.cat(counts)
+            kept.append((tab, ball_xy))
+        return [torch.cat(x) for x in zip(*packed)], torch.cat(counts), kept
+
+    @staticmethod
+    def _with_cameras(results, kept, counts):
+        """predict_clips' (spin, pos3d) results of one device extended by their RallyCamera, from _detect_clips' per-block keypoints and
+        ball detections (`kept`) and the host counts."""
+        rows, a = [], 0
+        for tab, ball_xy in kept:
+            m = tab.shape[0]
+            rows.append(ball_xy[:sum(counts[a:a + m])])
+            a += m
+        with _nvtx('ttk:cameras'):
+            cams = _rally_cameras(torch.cat([tab for tab, _ in kept]), torch.cat(rows), counts, [pos for _, pos in results])
+        return [res + (cam,) for res, cam in zip(results, cams)]
 
     @staticmethod
     def _check_counts(counts, first_clip):

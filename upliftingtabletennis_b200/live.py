@@ -117,7 +117,10 @@ class LiveSession:
     runs over them.
 
     end_rally(stream) runs the stream's ready stacks, then predict's tail (TableTennisPipeline._tail), and returns (spin, pos3d):
-    exactly what pipe.predict(the frames pushed since the last end_rally, fps) returns, the spin on the pipeline's device.  (With
+    exactly what pipe.predict(the frames pushed since the last end_rally, fps) returns, the spin on the pipeline's device.
+    end_rally(stream, cameras=True) returns (spin, pos3d, camera) instead, camera the rally's interface.RallyCamera, exactly what
+    pipe.predict_clips([the rally's frames], fps, cameras=True)[0] holds; it is computed by the same task as the tail (on the entry's
+    launcher with devices=[...]) and comes back as numpy.  (With
     devices=[...] the spin is computed, and copied to the pipeline's device, on the launcher thread's default streams, as in
     predict_clips; a caller that reads it on another stream of that device orders that stream after the default stream.)  The stream
     then starts a new rally; it does so also when end_rally raises: ValueError for a rally of fewer than 3 frames, predict's ValueError
@@ -197,7 +200,7 @@ class LiveSession:
                 if len(e.pending[BALL]) >= self.k or len(e.pending[TABLE]) >= self.k:
                     self._launch(e)
 
-    def end_rally(self, stream):
+    def end_rally(self, stream, cameras=False):
         s = self._stream(stream)
         e, n = self._entry[s], self._n[s]
         try:
@@ -205,7 +208,7 @@ class LiveSession:
             if n < 3:
                 raise ValueError('stream %d: a rally of %d frames; a rally needs at least 3 (one (prev, cur, next) ball stack)' % (s, n))
             self._launch(e, {s})
-            return self._run(e, self._finish, s, n, wait=True)
+            return self._run(e, self._finish, *((s, n, True) if cameras else (s, n)), wait=True)
         finally:
             self._reset(s)
 
@@ -482,10 +485,10 @@ class LiveSession:
         if e.copy is not None:
             torch.cuda.synchronize()
 
-    def _finish(self, s, n):
+    def _finish(self, s, n, cameras=False):
         e = self._entry[s]
         b, b_aux, t, t_aux = e.pos[s]
         if e.launcher is None:
-            return self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps)
-        spin, pos3d = self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, e.parts[4])
-        return spin.to(self.pipe._home_device()), pos3d
+            return self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, cameras=cameras)
+        out = self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, e.parts[4], cameras=cameras)
+        return (out[0].to(self.pipe._home_device()),) + out[1:]

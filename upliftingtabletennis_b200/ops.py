@@ -135,6 +135,28 @@ def project(points, mext, mint):
     return out
 
 
+def reproject_clips(points, offsets, mint, mext, valid, det_xy):
+    """`project` (float64) over n clips of different lengths in one launch.  points (sum T', 3) float64 CUDA, the clips concatenated;
+    offsets (n+1,) int32 CUDA prefix sums (filter_ball_clips' format); mint (n, 3, 4), mext (n, 4, 4) float64 CUDA; valid (n,) int32
+    CUDA; det_xy (sum T', 2) float64 CUDA, each row's 2D detection.  Returns xy (sum T', 2), each clip bit-identical to `project` on it
+    alone, and err (n, 2): mean (summed in row order) and max Euclidean distance between xy and det_xy.  A clip with valid == 0 gets
+    NaN points and errors."""
+    _lib.require_device()
+    assert points.is_cuda and points.dtype == torch.float64 and points.dim() == 2 and points.shape[1] == 3
+    assert det_xy.is_cuda and det_xy.dtype == torch.float64 and tuple(det_xy.shape) == (points.shape[0], 2)
+    assert offsets.is_cuda and offsets.dtype == torch.int32 and offsets.dim() == 1
+    n = offsets.shape[0] - 1
+    assert mint.is_cuda and mext.is_cuda and valid.is_cuda
+    assert mint.dtype == mext.dtype == torch.float64 and tuple(mint.shape) == (n, 3, 4) and tuple(mext.shape) == (n, 4, 4)
+    assert valid.dtype == torch.int32 and tuple(valid.shape) == (n,)
+    pts, offs, mi, me, ok, det = (t.contiguous() for t in (points, offsets, mint, mext, valid, det_xy))
+    xy = torch.empty((pts.shape[0], 2), dtype=torch.float64, device=pts.device)
+    err = torch.empty((n, 2), dtype=torch.float64, device=pts.device)
+    check(lib.ttk_reproject_clips(ptr(pts), pts.shape[0], ptr(offs), n, ptr(mi), ptr(me), ptr(ok), ptr(det), ptr(xy), ptr(err),
+                                  stream_ptr()))
+    return xy, err
+
+
 def filter_ball(pos1, pos2, fps, threshold=20.0):
     """filter_trajectory_ball (inference/utils.py:70-102) on the device.  pos1/pos2: (T, 3) float64 CUDA (x, y, v).
     Returns compacted xy (T, 2) f64, idx (T,) int64, times (T,) f64 (the first n rows are valid) and offsets (2,) int32
@@ -213,6 +235,7 @@ TABLE_POINTS = np.array([                                           # uplifting/
     [0.0, -(TABLE_WIDTH / 2 + 0.1525), TABLE_HEIGHT + 0.1525], [-TABLE_LENGTH / 2, 0, TABLE_HEIGHT],
     [TABLE_LENGTH / 2, 0, TABLE_HEIGHT]], dtype=np.float64)
 RANSAC_ITERATIONS, RANSAC_POINTS, RANSAC_FIXED_KEYS, RANSAC_THRESHOLD = 100, 6, (10, 11), 3.5     # regress_cameramatrices.py:129-136
+TOO_FEW_POINTS = 'not enough points for DLT'                       # the reference's AssertionError (:211)
 
 
 def ransac_sample_table(keypoints_host):
@@ -222,11 +245,29 @@ def ransac_sample_table(keypoints_host):
     tables = []
     for kp in keypoints_host:
         keys = [i + 1 for i in range(len(kp)) if kp[i][2] == 1]
-        assert len(keys) >= 6, 'not enough points for DLT'
+        assert len(keys) >= RANSAC_POINTS, TOO_FEW_POINTS
         rnd = np.random.default_rng(seed=42)
         pool = [k for k in keys if k not in RANSAC_FIXED_KEYS]
         tables.append([[int(s) for s in rnd.choice(pool, size=RANSAC_POINTS - len(RANSAC_FIXED_KEYS), replace=False)]
                        for _ in range(RANSAC_ITERATIONS)])
+    return np.asarray(tables, dtype=np.int32)
+
+
+_SAMPLE_TABLES = {}     # 13-bit visibility pattern -> (100, 4) int32 table
+
+
+def ransac_sample_table_cached(keypoints_host):
+    """ransac_sample_table with each clip's table looked up by its visibility pattern: the table depends on which keypoints are visible
+    and on nothing else (Generator(42).choice over the visible non-fixed keys), so each pattern is drawn once per process.  Returns
+    identical tables; raises the same AssertionError for fewer than 6 visible keypoints."""
+    tables = []
+    for kp in keypoints_host:
+        bits = sum(1 << i for i in range(len(kp)) if kp[i][2] == 1)
+        t = _SAMPLE_TABLES.get(bits)
+        if t is None:
+            t = _SAMPLE_TABLES[bits] = ransac_sample_table(np.asarray(kp)[None])[0]
+            t.flags.writeable = False
+        tables.append(t)
     return np.asarray(tables, dtype=np.int32)
 
 
