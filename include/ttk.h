@@ -221,6 +221,16 @@ TTK_API int ttk_filter_ball(const double* pos1_dev, const double* pos2_dev, int 
 TTK_API int ttk_filter_ball_clips(const double* pos1_dev, const double* pos2_dev, int n_clips, const int32_t* frame_offsets_dev,
                     int n_frames, double fps, double threshold_px, double* out_xy_dev, int64_t* out_idx_dev,
                     double* out_times_dev, int32_t* out_offsets_dev, void* stream);
+/* ttk_filter_ball / ttk_filter_ball_clips with capture times instead of fps, for frames that are not 1 / fps apart.
+ * stamps_dev[n_frames] float64 (device): one time per row of pos*_dev, in the same layout.  A kept row t gets
+ * out_times = stamps[t] - stamps[first row of its clip] (row 0 for ttk_filter_ball_timed); out_xy, out_idx and the offsets are
+ * exactly those of the untimed call.  With stamps[t] = t / fps per clip the times are bit-identical to the untimed call's. */
+TTK_API int ttk_filter_ball_timed(const double* pos1_dev, const double* pos2_dev, int n_frames, const double* stamps_dev,
+                    double threshold_px, double* out_xy_dev, int64_t* out_idx_dev, double* out_times_dev,
+                    int32_t* out_offsets_dev, void* stream);
+TTK_API int ttk_filter_ball_clips_timed(const double* pos1_dev, const double* pos2_dev, int n_clips, const int32_t* frame_offsets_dev,
+                    int n_frames, const double* stamps_dev, double threshold_px, double* out_xy_dev, int64_t* out_idx_dev,
+                    double* out_times_dev, int32_t* out_offsets_dev, void* stream);
 
 /* ttk_filter_table replaces filter_trajectory_table (inference/utils.py:137-169) and
  * _filter_keypoints_with_dbscan (:172-232; scikit-learn DBSCAN semantics, see csrc/filters.cu):

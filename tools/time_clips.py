@@ -6,8 +6,11 @@ uplifting transformer; main and auxiliary detectors share their weights so that 
   short : 64 clips of 12 to 49 frames
 On one GPU: [pipe.predict(c, fps) for c in clips] against pipe.predict_clips(clips, fps); then predict_clips over 1, 2, 4 and 8 devices
 (those that exist) and over two replicas on GPU 0 (devices=[0, 0]).  Results of the two arms are compared bit for bit.  Writes one JSON file.
+--timestamps: instead, the rally workload on one GPU through predict_clips with fps against predict_clips with per-frame capture
+timestamps (fps=None, stamps (k - 1) / fps, so that both arms must return the same bits).
 
     python tools/time_clips.py --out profiles/r05_clips_timing.json [--reps 5]
+    python tools/time_clips.py --timestamps --out profiles/r09_timestamps_timing.json [--reps 9]
 """
 import argparse
 import json
@@ -64,10 +67,29 @@ def same(a, b):
     return len(a) == len(b) and all(torch.equal(s.cpu(), s2.cpu()) and np.array_equal(p, p2) for (s, p), (s2, p2) in zip(a, b))
 
 
+def time_timestamps(pipe, clips, reps):
+    """predict_clips(clips, fps) against predict_clips(clips, None, timestamps=...) on one GPU, arms alternating."""
+    fps = 50.0
+    stamps = [(np.arange(len(c), dtype=np.float64) - 1) / fps for c in clips]
+    plain = lambda: pipe.predict_clips(clips, fps)
+    stamped = lambda: pipe.predict_clips(clips, None, timestamps=stamps)
+    _, want = timed(plain)                                        # warm-up of both arms
+    _, got = timed(stamped)
+    t_fps, t_stamps = [], []
+    for _ in range(reps):
+        t_fps.append(timed(plain)[0])
+        t_stamps.append(timed(stamped)[0])
+    return {'clips': len(clips), 'frames': sum(len(c) for c in clips), 'identical': same(got, want),
+            'fps_ms': float(np.median(t_fps)), 'timestamps_ms': float(np.median(t_stamps)),
+            'fps_ms_spread': [float(min(t_fps)), float(max(t_fps))], 'timestamps_ms_spread': [float(min(t_stamps)), float(max(t_stamps))],
+            'fps_ms_all': t_fps, 'timestamps_ms_all': t_stamps}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--out', required=True)
     ap.add_argument('--reps', type=int, default=5)
+    ap.add_argument('--timestamps', action='store_true', help='time predict_clips with per-frame stamps against fps (rally workload)')
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit('time_clips.py measures on a GPU; none is visible')
@@ -84,6 +106,13 @@ def main():
     result = {'gpus': [l.strip() for l in q.strip().splitlines()], 'device_count': torch.cuda.device_count(), 'reps': args.reps,
               'pipeline': 'WASB main + aux at %dx%d (tf32), HRNet main + aux (tf32), uplift (tf32x3); 1080p numpy frames' % RES,
               'workloads': {}}
+    if args.timestamps:
+        result['timestamps'] = time_timestamps(pipe, make_clips(workloads['rally'], pool), args.reps)
+        print('timestamps', json.dumps({k: v for k, v in result['timestamps'].items() if not k.endswith('_all')}), flush=True)
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, 'w') as f:
+            json.dump(result, f, indent=1)
+        return
     for name, lengths in workloads.items():
         clips = make_clips(lengths, pool)
         frames = sum(lengths)

@@ -66,6 +66,8 @@ def _load():
         'ttk_decode_profile_read': (i32, [C.POINTER(C.c_float), C.POINTER(C.c_float)]),
         'ttk_filter_ball': (i32, [vp, vp, i32, C.c_double, C.c_double, vp, vp, vp, vp, vp]),
         'ttk_filter_ball_clips': (i32, [vp, vp, i32, vp, i32, C.c_double, C.c_double, vp, vp, vp, vp, vp]),
+        'ttk_filter_ball_timed': (i32, [vp, vp, i32, vp, C.c_double, vp, vp, vp, vp, vp]),
+        'ttk_filter_ball_clips_timed': (i32, [vp, vp, i32, vp, i32, vp, C.c_double, vp, vp, vp, vp, vp]),
         'ttk_filter_table_workspace_bytes': (sz, [i32, i32, i32]),
         'ttk_filter_table': (i32, [vp, vp, i32, i32, i32, C.c_double, C.c_double, i32, vp, vp, sz, vp]),
         'ttk_filter_table_clips': (i32, [vp, vp, i32, vp, i32, i32, C.c_double, C.c_double, i32, vp, vp, sz, vp]),

@@ -8,6 +8,8 @@
 // the lowest-numbered cluster that has a core point in its neighbourhood (clusters are grown one after the other);
 // Counter.most_common(1) returns, among equally large clusters, the one that appears first in point order.
 // ttk_filter_ball_clips and ttk_filter_table_clips run the same per-clip arithmetic over n clips of different lengths in one launch.
+// ttk_filter_ball_timed / ttk_filter_ball_clips_timed take each row's capture time instead of fps: a kept row's time is its stamp minus
+// the stamp of its clip's first row, for frames that are not 1 / fps apart (variable frame rate, dropped frames).
 // All arithmetic is float64 without contraction, sums run in point order like numpy's axis-0 reduction.
 #include <limits.h>
 
@@ -18,10 +20,14 @@ namespace {
 constexpr int FB_THREADS = 1024;
 
 // ---- ball: one CTA, ordered stream compaction -------------------------------------------------------------------
+// TIMED: a kept row's time is stamps[t] - stamps[0] instead of t / fps (stamps is the last parameter, so the untimed instantiation keeps
+// its parameter offsets).
+template <bool TIMED>
 __global__ void __launch_bounds__(FB_THREADS) filter_ball_kernel(const double* __restrict__ p1, const double* __restrict__ p2,
                                                                  int T, double fps, double threshold, double visible,
                                                                  double* __restrict__ out_xy, int64_t* __restrict__ out_idx,
-                                                                 double* __restrict__ out_times, int32_t* __restrict__ out_offsets) {
+                                                                 double* __restrict__ out_times, int32_t* __restrict__ out_offsets,
+                                                                 const double* __restrict__ stamps) {
   __shared__ int s_warp[FB_THREADS / 32];
   __shared__ int s_base;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -48,7 +54,10 @@ __global__ void __launch_bounds__(FB_THREADS) filter_ball_kernel(const double* _
       out_xy[(size_t)o * 2] = x;
       out_xy[(size_t)o * 2 + 1] = y;
       out_idx[o] = t;
-      out_times[o] = (double)t / fps;             // float(t / fps)
+      if (TIMED)
+        out_times[o] = __dsub_rn(stamps[t], stamps[0]);
+      else
+        out_times[o] = (double)t / fps;           // float(t / fps)
     }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -67,13 +76,16 @@ __global__ void __launch_bounds__(FB_THREADS) filter_ball_kernel(const double* _
 // ---- ball over n clips: one CTA, ordered compaction of the concatenation --------------------------------------------------
 // Compacting the concatenated clips in frame order packs each clip's rows contiguously in clip order, so the per-clip
 // result of filter_ball_kernel is this kernel's rows out_offsets[c] .. out_offsets[c+1]-1 once idx and times count from
-// the clip's first frame.  out_offsets[c] is the number of kept frames before frame offs[c].
+// the clip's first frame.  out_offsets[c] is the number of kept frames before frame offs[c].  TIMED: as in filter_ball_kernel, from the
+// stamp of the clip's first frame.
+template <bool TIMED>
 __global__ void __launch_bounds__(FB_THREADS) filter_ball_clips_kernel(const double* __restrict__ p1, const double* __restrict__ p2,
                                                                        const int32_t* __restrict__ offs, int n_clips, int T,
                                                                        double fps, double threshold, double visible,
                                                                        double* __restrict__ out_xy, int64_t* __restrict__ out_idx,
                                                                        double* __restrict__ out_times,
-                                                                       int32_t* __restrict__ out_offsets) {
+                                                                       int32_t* __restrict__ out_offsets,
+                                                                       const double* __restrict__ stamps) {
   __shared__ int s_warp[FB_THREADS / 32];
   __shared__ int s_base;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -111,7 +123,10 @@ __global__ void __launch_bounds__(FB_THREADS) filter_ball_clips_kernel(const dou
       out_xy[(size_t)o * 2] = x;
       out_xy[(size_t)o * 2 + 1] = y;
       out_idx[o] = local;
-      out_times[o] = (double)local / fps;     // float(t / fps) of the clip's own frame index
+      if (TIMED)
+        out_times[o] = __dsub_rn(stamps[t], stamps[offs[c_last]]);
+      else
+        out_times[o] = (double)local / fps;   // float(t / fps) of the clip's own frame index
     }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -315,8 +330,21 @@ extern "C" int ttk_filter_ball(const double* pos1_dev, const double* pos2_dev, i
   TTK_CHECK_ARG(n_frames >= 0, "ttk_filter_ball: bad n_frames");
   TTK_CHECK_ARG(out_offsets_dev, "ttk_filter_ball: null pointer");
   TTK_CHECK_ARG(n_frames == 0 || (pos1_dev && pos2_dev && out_xy_dev && out_idx_dev && out_times_dev), "ttk_filter_ball: null pointer");
-  filter_ball_kernel<<<1, FB_THREADS, 0, (cudaStream_t)stream>>>(pos1_dev, pos2_dev, n_frames, fps, threshold_px, 1.0, out_xy_dev,
-                                                                out_idx_dev, out_times_dev, out_offsets_dev);
+  filter_ball_kernel<false><<<1, FB_THREADS, 0, (cudaStream_t)stream>>>(pos1_dev, pos2_dev, n_frames, fps, threshold_px, 1.0, out_xy_dev,
+                                                                       out_idx_dev, out_times_dev, out_offsets_dev, nullptr);
+  TTK_LAUNCH_CHECK();
+  return TTK_OK;
+}
+
+extern "C" int ttk_filter_ball_timed(const double* pos1_dev, const double* pos2_dev, int n_frames, const double* stamps_dev,
+                                     double threshold_px, double* out_xy_dev, int64_t* out_idx_dev, double* out_times_dev,
+                                     int32_t* out_offsets_dev, void* stream) {
+  TTK_CHECK_ARG(n_frames >= 0, "ttk_filter_ball_timed: bad n_frames");
+  TTK_CHECK_ARG(out_offsets_dev, "ttk_filter_ball_timed: null pointer");
+  TTK_CHECK_ARG(n_frames == 0 || (pos1_dev && pos2_dev && stamps_dev && out_xy_dev && out_idx_dev && out_times_dev),
+                "ttk_filter_ball_timed: null pointer");
+  filter_ball_kernel<true><<<1, FB_THREADS, 0, (cudaStream_t)stream>>>(pos1_dev, pos2_dev, n_frames, 0.0, threshold_px, 1.0, out_xy_dev,
+                                                                      out_idx_dev, out_times_dev, out_offsets_dev, stamps_dev);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }
@@ -349,9 +377,23 @@ extern "C" int ttk_filter_ball_clips(const double* pos1_dev, const double* pos2_
   TTK_CHECK_ARG(n_clips >= 0 && n_frames >= 0, "ttk_filter_ball_clips: bad sizes");
   TTK_CHECK_ARG(frame_offsets_dev && out_offsets_dev, "ttk_filter_ball_clips: null pointer");
   TTK_CHECK_ARG(n_frames == 0 || (pos1_dev && pos2_dev && out_xy_dev && out_idx_dev && out_times_dev), "ttk_filter_ball_clips: null pointer");
-  filter_ball_clips_kernel<<<1, FB_THREADS, 0, (cudaStream_t)stream>>>(pos1_dev, pos2_dev, frame_offsets_dev, n_clips, n_frames, fps,
-                                                                      threshold_px, 1.0, out_xy_dev, out_idx_dev, out_times_dev,
-                                                                      out_offsets_dev);
+  filter_ball_clips_kernel<false><<<1, FB_THREADS, 0, (cudaStream_t)stream>>>(pos1_dev, pos2_dev, frame_offsets_dev, n_clips, n_frames,
+                                                                             fps, threshold_px, 1.0, out_xy_dev, out_idx_dev,
+                                                                             out_times_dev, out_offsets_dev, nullptr);
+  TTK_LAUNCH_CHECK();
+  return TTK_OK;
+}
+
+extern "C" int ttk_filter_ball_clips_timed(const double* pos1_dev, const double* pos2_dev, int n_clips, const int32_t* frame_offsets_dev,
+                                           int n_frames, const double* stamps_dev, double threshold_px, double* out_xy_dev,
+                                           int64_t* out_idx_dev, double* out_times_dev, int32_t* out_offsets_dev, void* stream) {
+  TTK_CHECK_ARG(n_clips >= 0 && n_frames >= 0, "ttk_filter_ball_clips_timed: bad sizes");
+  TTK_CHECK_ARG(frame_offsets_dev && out_offsets_dev, "ttk_filter_ball_clips_timed: null pointer");
+  TTK_CHECK_ARG(n_frames == 0 || (pos1_dev && pos2_dev && stamps_dev && out_xy_dev && out_idx_dev && out_times_dev),
+                "ttk_filter_ball_clips_timed: null pointer");
+  filter_ball_clips_kernel<true><<<1, FB_THREADS, 0, (cudaStream_t)stream>>>(pos1_dev, pos2_dev, frame_offsets_dev, n_clips, n_frames,
+                                                                            0.0, threshold_px, 1.0, out_xy_dev, out_idx_dev,
+                                                                            out_times_dev, out_offsets_dev, stamps_dev);
   TTK_LAUNCH_CHECK();
   return TTK_OK;
 }

@@ -275,6 +275,58 @@ def clip_stack_plan(lengths, frames_per_stack):
     return first, offsets
 
 
+def check_time_source(fps, timestamps):
+    """A call or live session takes its frame times from exactly one source: fps (frames 1 / fps apart), or timestamps with fps=None."""
+    if (fps is None) == (timestamps is None):
+        raise ValueError('give either fps, or timestamps with fps=None (got fps=%r and %s)'
+                         % (fps, 'no timestamps' if timestamps is None else 'timestamps'))
+
+
+def check_timestamps(timestamps, n, what):
+    """The capture times of n frames, in seconds: a (n,) float64 array, finite and strictly increasing (the clock's origin does not
+    matter).  Raises ValueError naming `what` (the clip or stream)."""
+    try:
+        ts = np.asarray(timestamps, dtype=np.float64)
+    except (TypeError, ValueError) as e:
+        raise ValueError('%s: timestamps must be numbers in seconds (%s)' % (what, e)) from None
+    if ts.shape != (n,):
+        raise ValueError('%s: timestamps of shape %s for %d frames; give one per frame' % (what, ts.shape, n))
+    bad = np.flatnonzero(~np.isfinite(ts))
+    if len(bad):
+        raise ValueError('%s: timestamp %d is %r; timestamps must be finite' % (what, bad[0], float(ts[bad[0]])))
+    back = np.flatnonzero(ts[1:] <= ts[:-1])
+    if len(back):
+        i = int(back[0]) + 1
+        raise ValueError('%s: timestamp %d (%r) does not follow timestamp %d (%r); timestamps must increase strictly'
+                         % (what, i, float(ts[i]), i - 1, float(ts[i - 1])))
+    return ts
+
+
+def ball_row_stamps(stamps):
+    """The stamps of the ball rows of clips whose frames have the stamps `stamps` (one (n,) float64 array per clip), in the layout of
+    clip_stack_plan's ball stacks: row j of a clip is the stack centred on its frame j + 1, so the clip contributes stamps[1:n - 1]."""
+    return np.concatenate([np.zeros(0)] + [np.asarray(ts[1:len(ts) - 1], dtype=np.float64) for ts in stamps])
+
+
+def _upload_stamps(stamps, dev):
+    """float64 host stamps as a tensor on dev, through pinned memory: the copy is queued behind the detectors on the current stream
+    instead of waiting for them, as a copy from pageable memory would."""
+    return torch.from_numpy(np.ascontiguousarray(stamps, dtype=np.float64)).pin_memory().to(dev, non_blocking=True)
+
+
+def _upload_plan(plan, stamps, dev):
+    """_detect_clips' host tables of a block in one host-to-device copy: the int32 stack `plan` and, when given, the float64 ball-row
+    `stamps` (placed first, so that both device views are aligned).  Returns the int32 plan and the float64 stamps (or None) on dev."""
+    if stamps is None:
+        return torch.tensor(plan, dtype=torch.int32).pin_memory().to(dev, non_blocking=True), None
+    nb = 8 * len(stamps)
+    host = torch.empty((nb + 4 * len(plan),), dtype=torch.uint8).pin_memory()
+    host[:nb].view(torch.float64).numpy()[:] = stamps
+    host[nb:].view(torch.int32).numpy()[:] = plan
+    dev_buf = host.to(dev, non_blocking=True)
+    return dev_buf[nb:].view(torch.int32), dev_buf[:nb].view(torch.float64)
+
+
 def clip_blocks(lengths, max_frames):
     """Contiguous [(first clip, end)] blocks of at most max_frames frames each (a longer clip is a block of its own): bounds the device
     memory of predict_clips like _Detector.segment bounds predict()'s."""
@@ -755,10 +807,17 @@ class TableTennisPipeline:
         self.uplifting_model = UpliftingModel(dtype=dtype)
         self.KEYPOINT_VISIBLE = self.table_detector.KEYPOINT_VISIBLE
 
-    def predict(self, images, fps):
+    def predict(self, images, fps, timestamps=None):
         """interface.py:263-289.  Detections, both filters, the normalise/pad step and the transformer stay on the
-        device: the only host visit is the final result (and T' for slicing it, as in the reference)."""
+        device: the only host visit is the final result (and T' for slicing it, as in the reference).
+        timestamps: with fps=None, the capture time of each frame in seconds (finite, strictly increasing, any origin), for frames that
+        are not 1 / fps apart (variable frame rate, dropped frames).  The stack centred on frame k then has the time
+        timestamps[k] - timestamps[1] instead of (k - 1) / fps; with timestamps[k] = (k - 1) / fps the result is predict(images, fps)
+        bit for bit.  Raises ValueError before any device work for a wrong number of stamps, a non-finite or a non-increasing one, and
+        when both fps and timestamps, or neither, are given."""
+        check_time_source(fps, timestamps)
         n = len(images)
+        stamps = None if timestamps is None else check_timestamps(timestamps, n, 'timestamps')
         # every frame crosses PCIe once: the four detector passes (ball / table, main / auxiliary) share the uploaded clip, and the
         # first pass starts while later frames are still arriving
         frames, order, ready = self.ball_detector._upload(list(images), self.device)
@@ -770,15 +829,22 @@ class TableTennisPipeline:
             ball_positions_aux = self.ball_detector_aux._run(frames, 1, n - 2, False, None)[0][:, 0]
             table_keypoints = self.table_detector._run(frames, 1, n, False, None)[0]
             table_keypoints_aux = self.table_detector_aux._run(frames, 1, n, False, None)[0]
-        return self._tail(ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps)
+        return self._tail(ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps,
+                          stamps=None if stamps is None else stamps[1:n - 1])
 
-    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps, uplifting_model=None, cameras=False):
+    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps, uplifting_model=None, cameras=False,
+              stamps=None):
         """predict's steps after the four detectors, shared with LiveSession.end_rally: the ball filter, the table filters, the
         trajectory packing, the uplifting transformer and the spin rotation.  Takes the (n - 2, 3) ball and (n, K, 3) table positions
         of one clip on the device; returns predict's (spin, pos3d).  uplifting_model: a replica of self.uplifting_model to run instead
-        (on the positions' device).  cameras: return (spin, pos3d, RallyCamera) instead."""
+        (on the positions' device).  cameras: return (spin, pos3d, RallyCamera) instead.  stamps: the (n - 2,) float64 host stamps of
+        the clip's centre frames (timestamps[1:n - 1]), used instead of fps."""
         up = self.uplifting_model if uplifting_model is None else uplifting_model
-        ball_xy, _, times_ball, offsets = ops.filter_ball(ball_positions, ball_positions_aux, float(fps))
+        if stamps is None:
+            ball_xy, _, times_ball, offsets = ops.filter_ball(ball_positions, ball_positions_aux, float(fps))
+        else:
+            ball_xy, _, times_ball, offsets = ops.filter_ball_timed(ball_positions, ball_positions_aux,
+                                                                    _upload_stamps(stamps, ball_positions.device))
         with _nvtx('ttk:filters_pack'):
             filtered_table_keypoints = ops.filter_table(table_keypoints, table_keypoints_aux)
             ball_coords, table_coords, times, mask = ops.trajectory_pack(ball_xy, times_ball, offsets, filtered_table_keypoints[None],
@@ -793,14 +859,15 @@ class TableTennisPipeline:
     def live(self, fps, streams=1, k=None, slots=None, devices=None):
         """A LiveSession (upliftingtabletennis_b200/live.py) over `streams` cameras at `fps`: frames are pushed as they arrive, the
         detectors run on them while the rally goes on, and end_rally(stream) returns exactly what predict(the rally's frames, fps)
-        returns.  k: ready stacks that launch a detector pass (default live.DEFAULT_K); slots: device frame slots per stream (default
-        live.DEFAULT_SLOTS).  devices: None = the current device, passes launched on the caller's thread; or a list of CUDA devices
-        as predict_clips takes: entry r serves streams sharding.shard_range(streams, r, len(devices)) on devices[r], with its own
+        returns.  fps=None: a timestamped session, whose push takes each frame's capture time (push(stream, frames, timestamps=...))
+        and whose end_rally returns predict(the rally's frames, None, timestamps=their stamps).  k: ready stacks that launch a detector
+        pass (default live.DEFAULT_K); slots: device frame slots per stream (default live.DEFAULT_SLOTS).  devices: None = the current
+        device, passes launched on the caller's thread; or a list of CUDA devices as predict_clips takes: entry r serves streams sharding.shard_range(streams, r, len(devices)) on devices[r], with its own
         copy of the models and a launcher thread of its own; k and slots apply per entry."""
         from .live import LiveSession
         return LiveSession(self, fps, streams, k, slots, devices)
 
-    def predict_clips(self, clips, fps, devices=None, cameras=False):
+    def predict_clips(self, clips, fps, devices=None, cameras=False, timestamps=None):
         """Many rallies in one call: returns [(spin, pos3d), ...], exactly [self.predict(c, fps) for c in clips] (same types, spin on
         the same device, same values bit for bit).  clips: list of clips, each a list of HWC uint8 BGR frames like predict takes, all
         of one frame size.
@@ -818,16 +885,26 @@ class TableTennisPipeline:
         calibrate_camera matrices, reproject(pos3d, Mint, Mext), the filtered ball detections the uplift used and the pixel error between
         the two; a clip whose calibration fails reports the message in camera.error instead of raising.  The keypoints and detections
         are the ones the pipeline computed anyway; per device one calibration over its clips and one reprojection launch are added, on
-        the device and stream of the uplift.  cameras=False launches and synchronises nothing of this."""
+        the device and stream of the uplift.  cameras=False launches and synchronises nothing of this.
+        timestamps: with fps=None, a list parallel to clips holding each clip's frame capture times as predict takes them; the results
+        are then [self.predict(c, None, timestamps=t) for c, t in zip(clips, timestamps)] bit for bit.  A wrong number of stamps, a
+        non-finite or a non-increasing one raises ValueError naming the clip, before any device work."""
+        check_time_source(fps, timestamps)
         clips = [list(c) for c in clips]
         for i, c in enumerate(clips):
             if len(c) < 3:
                 raise ValueError('clip %d: %d frames; a clip needs at least 3 (one (prev, cur, next) ball stack)' % (i, len(c)))
+        times = fps
+        if timestamps is not None:
+            timestamps = list(timestamps)
+            if len(timestamps) != len(clips):
+                raise ValueError('timestamps: %d entries for %d clips; give one list of stamps per clip' % (len(timestamps), len(clips)))
+            times = [check_timestamps(t, len(c), 'clip %d' % i) for i, (c, t) in enumerate(zip(clips, timestamps))]
         if devices is None:
             if not clips:
                 return []
             parts = self._parts()
-            packed, counts, kept = self._detect_clips(parts, clips, fps)
+            packed, counts, kept = self._detect_clips(parts, clips, times)
             counts = counts.cpu().tolist()
             self._check_counts(counts, 0)
             spin, pos = self._uplift_clips(parts, packed, counts)
@@ -850,7 +927,7 @@ class TableTennisPipeline:
             a, b = blocks[r]
             if a == b:
                 return parts, None, [], None
-            packed, counts, kept = self._detect_clips(parts, clips[a:b], fps)
+            packed, counts, kept = self._detect_clips(parts, clips[a:b], times if timestamps is None else times[a:b])
             return parts, packed, counts.cpu().tolist(), kept
 
         def uplift(r, parts, packed, counts, kept):
@@ -903,8 +980,9 @@ class TableTennisPipeline:
         cache[slot] = (key, tuple(parts))
         return cache[slot][1]
 
-    def _detect_clips(self, parts, clips, fps):
-        """Detectors, both filters and the trajectory packing of `clips` on the current device, a block of clips at a time.
+    def _detect_clips(self, parts, clips, times):
+        """Detectors, both filters and the trajectory packing of `clips` on the current device, a block of clips at a time.  times: the
+        fps, or a list of each clip's (n,) float64 frame stamps (check_timestamps).
         Returns the packed uplift inputs (ball, table, times, mask) of all clips, the (n,) int32 CUDA agreeing-detection counts and,
         per block, its filtered table keypoints (clips, 13, 3) and ball detections (rows of its clips in order, then unused capacity):
         what _with_cameras reads."""
@@ -920,12 +998,16 @@ class TableTennisPipeline:
                 frames, ready = frames[torch.tensor(order, device=dev)], None
             bfirst, boffs = clip_stack_plan(lengths, ball.frames_per_stack)
             tfirst, toffs = clip_stack_plan(lengths, table.frames_per_stack)
-            plan = torch.tensor(bfirst + boffs + tfirst + toffs, dtype=torch.int32).pin_memory().to(dev, non_blocking=True)
+            stamps = ball_row_stamps(times[a:b]) if isinstance(times, list) else None
+            plan, stamps_d = _upload_plan(bfirst + boffs + tfirst + toffs, stamps, dev)
             bfirst_d, boffs_d, tfirst_d, toffs_d = plan.split([len(bfirst), len(boffs), len(tfirst), len(toffs)])
             with torch.no_grad():
                 bpos = ball._run(frames, 1, len(bfirst), False, ready, first=(bfirst, bfirst_d))[0][:, 0]
                 bpos_aux = ball_aux._run(frames, 1, len(bfirst), False, None, first=(bfirst, bfirst_d))[0][:, 0]
-                ball_xy, _, times_ball, offsets = ops.filter_ball_clips(bpos, bpos_aux, boffs_d, float(fps))
+                if stamps is None:
+                    ball_xy, _, times_ball, offsets = ops.filter_ball_clips(bpos, bpos_aux, boffs_d, float(times))
+                else:
+                    ball_xy, _, times_ball, offsets = ops.filter_ball_clips_timed(bpos, bpos_aux, boffs_d, stamps_d)
                 tpos = table._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
                 tpos_aux = table_aux._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
             with _nvtx('ttk:filters_pack'):

@@ -12,6 +12,7 @@ goes on from there, so every stack of every stream is "first frame + 0, 1, 2" in
 entry is one ttk_preprocess_stacks_indexed call, as in predict_clips.
 
 The bookkeeping is kept in pure functions (push_plan, ready_stacks, check_live_args) so that it can be checked without a GPU."""
+import functools
 import itertools
 import numbers
 from concurrent.futures import ThreadPoolExecutor
@@ -20,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib, sharding
-from .interface import _Detector, _fingerprint, parse_devices
+from .interface import _Detector, _fingerprint, check_timestamps, parse_devices
 
 DEFAULT_K = 16          # ready stacks that launch a pass: _Detector.chunk, predict's pass size; 137-143 frames/s for k = 4..32 on
                         # WASB + HRNet (profiles/r06_live_timing.json), so no reason to give ViTPose's GEMMs fewer M tiles
@@ -126,6 +127,13 @@ class LiveSession:
     then starts a new rally; it does so also when end_rally raises: ValueError for a rally of fewer than 3 frames, predict's ValueError
     for 0 or 50 or more agreeing ball detections.
 
+    fps=None opens a timestamped session, for cameras whose frames are not 1 / fps apart (variable frame rate, dropped frames, or a
+    caller that skips frames to keep up): push(stream, frames, timestamps=...) then takes the capture time of each frame in seconds
+    (a number for a single frame), and end_rally returns exactly pipe.predict(the rally's frames, None, timestamps=their stamps).  Each
+    stamp must be finite and later than the stream's previous stamp in the open rally; the stamps are kept per stream on the host and
+    reset with the rally.  A wrong number of stamps, a bad stamp, stamps pushed to a session with fps or none to a timestamped session
+    raise ValueError before the push does anything.
+
     devices: None = one entry on the current device; push launches the passes on the caller's thread.  Otherwise a list of CUDA device
     indices, torch.device or 'cuda:N' strings, as predict_clips takes (a device may repeat): one entry per item, entry r serving
     streams sharding.shard_range(streams, r, len(devices)) -- contiguous blocks, the first streams % len(devices) entries one stream
@@ -172,6 +180,8 @@ class LiveSession:
         self._w = [0] * self.streams                        # next slot each stream writes
         self._n = [0] * self.streams                        # frames of each stream's open rally
         self._models = [None] * self.streams                # per open rally: (full fingerprint, weight tensors, quick key)
+        # fps=None: each stream's open rally's frame stamps, on the host (a wrap copies frames, not stamps)
+        self._stamps = [[] for _ in range(self.streams)] if fps is None else None
         self._stale = set()                                 # streams whose open rally was detected with replicas since rebuilt
         self._closed = False
 
@@ -181,12 +191,13 @@ class LiveSession:
         return {fps: [x for e in self._entries for x in e.pending[fps]] for fps in (BALL, TABLE)}
 
     # ---- public --------------------------------------------------------------------------------------
-    def push(self, stream, frames):
+    def push(self, stream, frames, timestamps=None):
         s = self._stream(stream)
         e = self._entry[s]
         if isinstance(frames, (np.ndarray, torch.Tensor)) and frames.ndim == 3:
             frames = [frames]
         frames = list(frames)
+        stamps = self._check_stamps(s, len(frames), timestamps)
         if not frames:
             return
         self._check_frames(frames)
@@ -197,6 +208,8 @@ class LiveSession:
                 self._wrap(s, *step[1:])
             else:
                 self._write(s, frames, *step[1:])
+                if stamps is not None:
+                    self._stamps[s] += stamps[step[2]:step[3]].tolist()
                 if len(e.pending[BALL]) >= self.k or len(e.pending[TABLE]) >= self.k:
                     self._launch(e)
 
@@ -208,7 +221,10 @@ class LiveSession:
             if n < 3:
                 raise ValueError('stream %d: a rally of %d frames; a rally needs at least 3 (one (prev, cur, next) ball stack)' % (s, n))
             self._launch(e, {s})
-            return self._run(e, self._finish, *((s, n, True) if cameras else (s, n)), wait=True)
+            finish = self._finish
+            if self._stamps is not None:
+                finish = functools.partial(self._finish, stamps=np.array(self._stamps[s], dtype=np.float64))
+            return self._run(e, finish, *((s, n, True) if cameras else (s, n)), wait=True)
         finally:
             self._reset(s)
 
@@ -267,6 +283,23 @@ class LiveSession:
         if self._pool is None:
             self.shape = shape
             self._pool = self._alloc_pool(shape)
+
+    def _check_stamps(self, s, count, timestamps):
+        """The float64 stamps of `count` frames pushed to stream s (None for a session with fps).  Raises ValueError, before any device
+        work, when a timestamped session gets no stamps or the wrong number, a non-finite one, one that does not increase, or one not
+        after the rally's previous frame, and when a session with fps gets stamps."""
+        if self._stamps is None:
+            if timestamps is not None:
+                raise ValueError('stream %d: this session runs at fps=%r and takes no timestamps; open it with fps=None to push them'
+                                 % (s, self.fps))
+            return None
+        if timestamps is None:
+            raise ValueError('stream %d: this session (fps=None) needs timestamps=, one capture time per frame' % s)
+        ts = check_timestamps([timestamps] if np.ndim(timestamps) == 0 else timestamps, count, 'stream %d' % s)     # (one frame, one stamp)
+        if count and self._n[s] and not ts[0] > self._stamps[s][-1]:
+            raise ValueError("stream %d: timestamp %r does not follow the rally's previous frame at %r; timestamps must increase strictly"
+                             % (s, float(ts[0]), self._stamps[s][-1]))
+        return ts
 
     def _check_models(self, s, full):
         parts = self.pipe._parts()
@@ -344,6 +377,8 @@ class LiveSession:
 
     def _reset(self, s):
         self._n[s], self._models[s] = 0, None
+        if self._stamps is not None:
+            self._stamps[s] = []
         self._stale.discard(s)
         e = self._entry[s]
         for fps in (BALL, TABLE):
@@ -485,10 +520,12 @@ class LiveSession:
         if e.copy is not None:
             torch.cuda.synchronize()
 
-    def _finish(self, s, n, cameras=False):
+    def _finish(self, s, n, cameras=False, stamps=None):
+        """stamps: the rally's n frame stamps (fps=None)."""
         e = self._entry[s]
         b, b_aux, t, t_aux = e.pos[s]
+        centre = None if stamps is None else stamps[1:n - 1]
         if e.launcher is None:
-            return self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, cameras=cameras)
-        out = self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, e.parts[4], cameras=cameras)
+            return self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, cameras=cameras, stamps=centre)
+        out = self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, e.parts[4], cameras=cameras, stamps=centre)
         return (out[0].to(self.pipe._home_device()),) + out[1:]

@@ -192,6 +192,41 @@ def filter_ball_clips(pos1, pos2, frame_offsets, fps, threshold=20.0):
     return xy, idx, times, offs
 
 
+def filter_ball_timed(pos1, pos2, stamps, threshold=20.0):
+    """filter_ball with each row's capture time instead of fps: stamps (T,) float64 CUDA, one per row of pos1.  A kept row t gets
+    time stamps[t] - stamps[0]; xy, idx and offsets are filter_ball's."""
+    _lib.require_device()
+    assert pos1.is_cuda and pos1.dtype == torch.float64 and pos1.shape == pos2.shape and pos1.dim() == 2 and pos1.shape[1] == 3
+    assert stamps.is_cuda and stamps.dtype == torch.float64 and tuple(stamps.shape) == (pos1.shape[0],)
+    pos1, pos2, stamps = pos1.contiguous(), pos2.contiguous(), stamps.contiguous()
+    T, dev = pos1.shape[0], pos1.device
+    xy = torch.empty((T, 2), dtype=torch.float64, device=dev)
+    idx = torch.empty((T,), dtype=torch.int64, device=dev)
+    times = torch.empty((T,), dtype=torch.float64, device=dev)
+    offs = torch.empty((2,), dtype=torch.int32, device=dev)
+    check(lib.ttk_filter_ball_timed(ptr(pos1), ptr(pos2), T, ptr(stamps), float(threshold), ptr(xy), ptr(idx), ptr(times), ptr(offs),
+                                    stream_ptr()))
+    return xy, idx, times, offs
+
+
+def filter_ball_clips_timed(pos1, pos2, frame_offsets, stamps, threshold=20.0):
+    """filter_ball_clips with each row's capture time instead of fps: stamps (sum T,) float64 CUDA in the layout of pos1.  A kept row
+    gets its stamp minus the stamp of its clip's first row; xy, idx and offsets are filter_ball_clips'."""
+    _lib.require_device()
+    assert pos1.is_cuda and pos1.dtype == torch.float64 and pos1.shape == pos2.shape and pos1.dim() == 2 and pos1.shape[1] == 3
+    assert frame_offsets.is_cuda and frame_offsets.dtype == torch.int32 and frame_offsets.dim() == 1
+    assert stamps.is_cuda and stamps.dtype == torch.float64 and tuple(stamps.shape) == (pos1.shape[0],)
+    pos1, pos2, frame_offsets, stamps = pos1.contiguous(), pos2.contiguous(), frame_offsets.contiguous(), stamps.contiguous()
+    T, dev, n = pos1.shape[0], pos1.device, frame_offsets.shape[0] - 1
+    xy = torch.empty((T, 2), dtype=torch.float64, device=dev)
+    idx = torch.empty((T,), dtype=torch.int64, device=dev)
+    times = torch.empty((T,), dtype=torch.float64, device=dev)
+    offs = torch.empty((n + 1,), dtype=torch.int32, device=dev)
+    check(lib.ttk_filter_ball_clips_timed(ptr(pos1), ptr(pos2), n, ptr(frame_offsets), T, ptr(stamps), float(threshold), ptr(xy),
+                                          ptr(idx), ptr(times), ptr(offs), stream_ptr()))
+    return xy, idx, times, offs
+
+
 def filter_table_clips(pos1, pos2, frame_offsets, agree=10.0, eps=10.0, min_samples=3):
     """filter_table over n clips of different lengths: pos1/pos2 (sum T, K, 3) float64 CUDA, the clips concatenated; frame_offsets
     (n+1,) int32 CUDA prefix sums.  Returns (n, K, 3) float64, each clip bit-identical to filter_table on that clip alone."""
