@@ -8,9 +8,14 @@ On one GPU: [pipe.predict(c, fps) for c in clips] against pipe.predict_clips(cli
 (those that exist) and over two replicas on GPU 0 (devices=[0, 0]).  Results of the two arms are compared bit for bit.  Writes one JSON file.
 --timestamps: instead, the rally workload on one GPU through predict_clips with fps against predict_clips with per-frame capture
 timestamps (fps=None, stamps (k - 1) / fps, so that both arms must return the same bits).
+--known-table: instead, the rally workload on one GPU through predict_clips with the table detected against predict_clips with each
+clip's own filtered keypoints given as table_keypoints (so that both arms must return the same bits).  --pipeline wasb-hrnet is the
+pipeline above; vitpose is ViTPose at 1152x640 (tf32x3) for all four detectors, each auxiliary sharing its main detector's weights
+(as tools/time_rally_cameras.py runs it).
 
     python tools/time_clips.py --out profiles/r05_clips_timing.json [--reps 5]
     python tools/time_clips.py --timestamps --out profiles/r09_timestamps_timing.json [--reps 9]
+    python tools/time_clips.py --known-table --pipeline vitpose --out known_table_vitpose.json [--reps 5]
 """
 import argparse
 import json
@@ -85,11 +90,35 @@ def time_timestamps(pipe, clips, reps):
             'fps_ms_all': t_fps, 'timestamps_ms_all': t_stamps}
 
 
+def time_known_table(pipe, clips, reps):
+    """predict_clips(clips, fps) against predict_clips(clips, fps, table_keypoints=each clip's own keypoints) on one GPU, arms
+    alternating."""
+    fps = 50.0
+    tables = [cam.keypoints for _, _, cam in pipe.predict_clips(clips, fps, cameras=True)]
+    detected = lambda: pipe.predict_clips(clips, fps)
+    known = lambda: pipe.predict_clips(clips, fps, table_keypoints=tables)
+    _, want = timed(detected)                                     # warm-up of both arms
+    _, got = timed(known)
+    t_detected, t_known = [], []
+    for _ in range(reps):
+        t_detected.append(timed(detected)[0])
+        t_known.append(timed(known)[0])
+    med_d, med_k = float(np.median(t_detected)), float(np.median(t_known))
+    return {'clips': len(clips), 'frames': sum(len(c) for c in clips), 'identical': same(got, want),
+            'visible_keypoints_per_clip': sorted({int(k[:, 2].sum()) for k in tables}),
+            'detected_ms': med_d, 'known_table_ms': med_k, 'detected_over_known': med_d / med_k,
+            'detected_ms_spread': [float(min(t_detected)), float(max(t_detected))],
+            'known_table_ms_spread': [float(min(t_known)), float(max(t_known))],
+            'detected_ms_all': t_detected, 'known_table_ms_all': t_known}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--out', required=True)
     ap.add_argument('--reps', type=int, default=5)
     ap.add_argument('--timestamps', action='store_true', help='time predict_clips with per-frame stamps against fps (rally workload)')
+    ap.add_argument('--known-table', action='store_true', help='time predict_clips with known tables against detected ones (rally workload)')
+    ap.add_argument('--pipeline', choices=('wasb-hrnet', 'vitpose'), default='wasb-hrnet', help='the pipeline of --known-table')
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit('time_clips.py measures on a GPU; none is visible')
@@ -106,6 +135,20 @@ def main():
     result = {'gpus': [l.strip() for l in q.strip().splitlines()], 'device_count': torch.cuda.device_count(), 'reps': args.reps,
               'pipeline': 'WASB main + aux at %dx%d (tf32), HRNet main + aux (tf32), uplift (tf32x3); 1080p numpy frames' % RES,
               'workloads': {}}
+    if args.known_table:
+        if args.pipeline == 'vitpose':
+            from time_live import VIT_RES, write_vitpose_checkpoints
+            write_vitpose_checkpoints(hub)
+            pipe = TableTennisPipeline(ball_model='vitpose', ball_model_aux='vitpose', table_model='vitpose', table_model_aux='vitpose')
+            result['pipeline'] = 'ViTPose main + aux (same weights) for ball and table at %dx%d (tf32x3), uplift (tf32x3); 1080p numpy frames' % VIT_RES
+        result['known_table'] = time_known_table(pipe, make_clips(workloads['rally'], pool), args.reps)
+        print('known_table', json.dumps({k: v for k, v in result['known_table'].items() if not k.endswith('_all')}), flush=True)
+        result['gpus_after'] = [l.strip() for l in subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader'],
+                                                                  capture_output=True, text=True).stdout.strip().splitlines()]
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, 'w') as f:
+            json.dump(result, f, indent=1)
+        return
     if args.timestamps:
         result['timestamps'] = time_timestamps(pipe, make_clips(workloads['rally'], pool), args.reps)
         print('timestamps', json.dumps({k: v for k, v in result['timestamps'].items() if not k.endswith('_all')}), flush=True)

@@ -11,6 +11,9 @@ With --devices N,M,...:
   launcher: (N = 1) devices=None against devices=[0] on one GPU: the max_fps arm for S = 1, 2, 4, with push p50 / p99.
   scaling : (N >= 2) devices=[0 .. N-1], one entry per GPU: the max_fps arm for S = 2, 4, 8, 16 cameras (S >= N), with end_rally median
             / p99.  An arm runs only where N GPUs are visible; the others, and S < N, are listed under 'skipped'.
+--known-table: instead, the cameras arm: at --fps (default 30 here) the most cameras, of 1 .. 8, whose pushes keep to the clock, with
+every stream's table set (LiveSession.set_table, the keypoints filtered from the pool's first 50 frames) against the tables detected,
+with push p50 / p99 and end_rally median / p99 of every trial.
 Pipelines (--pipeline): wasb-hrnet = WASB main + aux at 1280x704, HRNet main + aux (tf32), uplift (tf32x3) -- bench.py's pipeline leg;
 default = the pipeline's default composition, ViTPose main (1152x640, tf32x3) + WASB aux for the ball, ViTPose main + HRNet aux for the
 table.  The synthetic ViTPose and WASB ball detectors do not agree, so on `default` predict and end_rally refuse every rally with
@@ -18,6 +21,7 @@ ValueError after all detectors and filters have run (counted as 'refused'; laten
 
     python tools/time_live.py --out profiles/r06_live_timing.json
     python tools/time_live.py --out profiles/r07_live_devices_timing.json --pipeline default --devices 1,2,4,8
+    python tools/time_live.py --out profiles/r10_known_table_live.json --known-table [--pipeline default]
 """
 import argparse
 import json
@@ -113,13 +117,15 @@ def throughput(pipe, pool, k, rallies):
     return {'k': k, 'frames': rallies * RALLY, 'frames_per_s': rallies * RALLY / dt}
 
 
-def paced(pipe, pool, streams, fps, rallies, devices=None):
+def paced(pipe, pool, streams, fps, rallies, devices=None, table=None):
     """S cameras at fps, one frame each per tick, rally ends staggered; returns the push lags (s), the push durations (s), the
-    end_rally durations (s) and the number of rallies refused with ValueError."""
+    end_rally durations (s) and the number of rallies refused with ValueError.  table: every stream's known table, or None."""
     lags, durs, ends, refused = [], [], [], 0
     ticks = rallies * RALLY
     offset = [s * RALLY // streams for s in range(streams)]
     with pipe.live(fps, streams=streams, devices=devices) as live:
+        for s in range(streams):
+            live.set_table(s, table)
         t0 = time.perf_counter() + 0.05
         for t in range(ticks):
             due = t0 + t / fps
@@ -159,12 +165,31 @@ def max_fps(pipe, pool, streams, devices=None, label=''):
     return {'per_camera_fps': best, 'ladder': list(LADDER), 'trials': trials}
 
 
+def cameras_at(pipe, pool, fps, table, most=8):
+    """The most cameras (1 .. most) at fps that keep to the clock (95th percentile lag below one frame interval), every stream's
+    table set to `table` (None: detected)."""
+    best, trials = 0, []
+    for streams in range(1, most + 1):
+        lags, durs, ends, refused = paced(pipe, pool, streams, fps, 3, table=table)
+        ok = bool(np.percentile(lags, 95) < 1.0 / fps)
+        trials.append({'cameras': streams, 'sustained': ok, 'lag_ms_p50': float(np.median(lags) * 1e3),
+                       'lag_ms_p95': float(np.percentile(lags, 95) * 1e3), 'push_ms_p50': float(np.median(durs) * 1e3),
+                       'push_ms_p99': float(np.percentile(durs, 99) * 1e3), 'end_rally_ms_median': float(np.median(ends) * 1e3),
+                       'end_rally_ms_p99': float(np.percentile(ends, 99) * 1e3), 'refused_rallies': refused})
+        print('known' if table is not None else 'detected', json.dumps(trials[-1]), flush=True)
+        if not ok:
+            break
+        best = streams
+    return {'cameras': best, 'fps': fps, 'trials': trials}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--out', required=True)
-    ap.add_argument('--fps', type=float, default=60.0)
+    ap.add_argument('--fps', type=float, default=None, help='default 60, or 30 with --known-table')
     ap.add_argument('--rallies', type=int, default=10)
     ap.add_argument('--pipeline', choices=('wasb-hrnet', 'default'), default='wasb-hrnet')
+    ap.add_argument('--known-table', action='store_true', help='cameras at --fps with tables set against detected')
     ap.add_argument('--devices', default='', help='comma-separated GPU counts: 1 = the launcher arm, N >= 2 = the scaling arm on N GPUs')
     args = ap.parse_args()
     counts = [int(c) for c in args.devices.split(',') if c]
@@ -188,6 +213,23 @@ def main():
     pool = list(synthetic.frames_1080p(128, seed=11))
     result = {'gpus': [l.strip() for l in q.strip().splitlines()], 'default_k': DEFAULT_K, 'default_slots': DEFAULT_SLOTS,
               'pipeline': desc, 'pipeline_arg': args.pipeline}
+    if args.known_table:
+        frames = pool[:RALLY]
+        table = pipe.table_detector.filter_trajectory(pipe.table_detector.predict(frames, return_heatmaps=False)[0],
+                                                      pipe.table_detector_aux.predict(frames, return_heatmaps=False)[0])
+        fps = args.fps or 30.0
+        result['known_table'] = {'visible_keypoints': int(table[:, 2].sum())}
+        for label, t in (('detected', None), ('known', table)):           # warm-up of both arms: one camera, one rally
+            paced(pipe, pool, 1, fps, 1, table=t)
+        for label, t in (('detected', None), ('known', table)):
+            result['known_table'][label] = cameras_at(pipe, pool, fps, t)
+        result['gpus_after'] = [l.strip() for l in subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader'],
+                                                                  capture_output=True, text=True).stdout.strip().splitlines()]
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, 'w') as f:
+            json.dump(result, f, indent=1)
+        return
+    args.fps = args.fps or 60.0
     result['latency'] = latency(pipe, pool, args.fps, args.rallies)
     print('latency', json.dumps({k: v for k, v in result['latency'].items()}), flush=True)
     result['k'] = [throughput(pipe, pool, k, 4) for k in (4, 8, 16, 32)]

@@ -302,6 +302,37 @@ def check_timestamps(timestamps, n, what):
     return ts
 
 
+def check_table_keypoints(keypoints, what):
+    """A known table: (13, 3) (x, y, v) rows in image pixels, as filter_trajectory_table returns them and RallyCamera.keypoints holds
+    them (numpy, a nested list, or a torch CPU / CUDA tensor).  Every value finite, every v 0 or 1 (the uplift reads v as the keypoint
+    mask).  Returns a (13, 3) float64 array; raises ValueError naming `what` (the clip or stream)."""
+    if isinstance(keypoints, torch.Tensor):
+        keypoints = keypoints.detach().cpu().numpy()
+    try:
+        kp = np.array(keypoints, dtype=np.float64)
+    except (TypeError, ValueError) as e:
+        raise ValueError('%s: table keypoints must be numbers (%s)' % (what, e)) from None
+    if kp.shape != (13, 3):
+        raise ValueError('%s: table keypoints of shape %s; give (13, 3) rows of (x, y, v)' % (what, kp.shape))
+    bad = np.argwhere(~np.isfinite(kp))
+    if len(bad):
+        raise ValueError('%s: table keypoint %d holds %r; table keypoints must be finite' % (what, bad[0][0], float(kp[tuple(bad[0])])))
+    bad = np.flatnonzero((kp[:, 2] != KEYPOINT_VISIBLE) & (kp[:, 2] != KEYPOINT_INVISIBLE))
+    if len(bad):
+        raise ValueError('%s: table keypoint %d has visibility %r; v must be 0 or 1' % (what, bad[0], float(kp[bad[0], 2])))
+    return kp
+
+
+def select_stacks(first, offsets, clips):
+    """The stacks of the clips `clips` (indices, in order) out of a clip_stack_plan (first, offsets): their first frames, still in
+    the frames of every clip, and the prefix sums of their stack counts."""
+    sel, offs = [], [0]
+    for i in clips:
+        sel.extend(first[offsets[i]:offsets[i + 1]])
+        offs.append(offs[-1] + offsets[i + 1] - offsets[i])
+    return sel, offs
+
+
 def ball_row_stamps(stamps):
     """The stamps of the ball rows of clips whose frames have the stamps `stamps` (one (n,) float64 array per clip), in the layout of
     clip_stack_plan's ball stacks: row j of a clip is the stack centred on its frame j + 1, so the clip contributes stamps[1:n - 1]."""
@@ -312,6 +343,11 @@ def _upload_stamps(stamps, dev):
     """float64 host stamps as a tensor on dev, through pinned memory: the copy is queued behind the detectors on the current stream
     instead of waiting for them, as a copy from pageable memory would."""
     return torch.from_numpy(np.ascontiguousarray(stamps, dtype=np.float64)).pin_memory().to(dev, non_blocking=True)
+
+
+def _upload_tables(keypoints, dev):
+    """Known tables (a (13, 3) float64 array, or a list of them) as one tensor on dev, through pinned memory like _upload_stamps."""
+    return torch.from_numpy(np.ascontiguousarray(keypoints, dtype=np.float64)).pin_memory().to(dev, non_blocking=True)
 
 
 def _upload_plan(plan, stamps, dev):
@@ -732,10 +768,14 @@ def _rally_cameras(keypoints, det_xy, counts, positions):
     valid = torch.zeros((n,), dtype=torch.int32, device=dev)
     info = None
     if len(enough):
-        sel = torch.from_numpy(enough).to(dev)
-        samples = torch.from_numpy(ops.ransac_sample_table_cached(kp[enough])).to(dev)
-        mi, me, info = ops.calibrate_camera(keypoints[sel], samples, WIDTH, HEIGHT)
-        mint[sel], mext[sel] = mi, me
+        # the calibration is deterministic: each distinct keypoint array (a known table shared by many rallies) is calibrated once
+        distinct = {}
+        which = np.array([distinct.setdefault(kp[i].tobytes(), len(distinct)) for i in enough], dtype=np.int64)
+        first = enough[np.unique(which, return_index=True)[1]]
+        sel, which = torch.from_numpy(enough).to(dev), torch.from_numpy(which).to(dev)
+        samples = torch.from_numpy(ops.ransac_sample_table_cached(kp[first])).to(dev)
+        mi, me, info = ops.calibrate_camera(keypoints[torch.from_numpy(first).to(dev)], samples, WIDTH, HEIGHT)
+        mint[sel], mext[sel], info = mi[which], me[which], info[which]
         valid[sel] = ((info[:, 3] != 0) & (info[:, 0] != 0)).to(torch.int32)
     offsets = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
     points = torch.from_numpy(np.concatenate(positions).astype(np.float64)).to(dev)
@@ -807,19 +847,26 @@ class TableTennisPipeline:
         self.uplifting_model = UpliftingModel(dtype=dtype)
         self.KEYPOINT_VISIBLE = self.table_detector.KEYPOINT_VISIBLE
 
-    def predict(self, images, fps, timestamps=None):
+    def predict(self, images, fps, timestamps=None, table_keypoints=None):
         """interface.py:263-289.  Detections, both filters, the normalise/pad step and the transformer stay on the
         device: the only host visit is the final result (and T' for slicing it, as in the reference).
         timestamps: with fps=None, the capture time of each frame in seconds (finite, strictly increasing, any origin), for frames that
         are not 1 / fps apart (variable frame rate, dropped frames).  The stack centred on frame k then has the time
         timestamps[k] - timestamps[1] instead of (k - 1) / fps; with timestamps[k] = (k - 1) / fps the result is predict(images, fps)
         bit for bit.  Raises ValueError before any device work for a wrong number of stamps, a non-finite or a non-increasing one, and
-        when both fps and timestamps, or neither, are given."""
+        when both fps and timestamps, or neither, are given.
+        table_keypoints: the table of a camera that does not move, a (13, 3) array of (x, y, v) in image pixels (numpy, nested list or
+        torch tensor; as filter_trajectory_table returns it and RallyCamera.keypoints holds it).  Neither table detector then runs (half
+        the detector passes) and the uplift reads these keypoints in place of the filtered detections: the result is the reference's
+        predict with filter_trajectory_table(...) replaced by them, and with the clip's own filtered keypoints it is predict(images,
+        fps) bit for bit.  A shape other than (13, 3), a non-finite value or a v other than 0 or 1 raises ValueError before any device
+        work."""
         check_time_source(fps, timestamps)
         n = len(images)
         stamps = None if timestamps is None else check_timestamps(timestamps, n, 'timestamps')
-        # every frame crosses PCIe once: the four detector passes (ball / table, main / auxiliary) share the uploaded clip, and the
-        # first pass starts while later frames are still arriving
+        known = None if table_keypoints is None else check_table_keypoints(table_keypoints, 'table_keypoints')
+        # every frame crosses PCIe once: the detector passes (ball / table, main / auxiliary) share the uploaded clip, and the first
+        # pass starts while later frames are still arriving
         frames, order, ready = self.ball_detector._upload(list(images), self.device)
         if order != list(range(n)):
             torch.cuda.current_stream().wait_event(ready[-1][1])
@@ -827,18 +874,21 @@ class TableTennisPipeline:
         with torch.no_grad():
             ball_positions = self.ball_detector._run(frames, 1, n - 2, False, ready)[0][:, 0]       # sliding (prev, cur, next) window
             ball_positions_aux = self.ball_detector_aux._run(frames, 1, n - 2, False, None)[0][:, 0]
-            table_keypoints = self.table_detector._run(frames, 1, n, False, None)[0]
-            table_keypoints_aux = self.table_detector_aux._run(frames, 1, n, False, None)[0]
-        return self._tail(ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps,
-                          stamps=None if stamps is None else stamps[1:n - 1])
+            if known is None:
+                table_kp = self.table_detector._run(frames, 1, n, False, None)[0]
+                table_kp_aux = self.table_detector_aux._run(frames, 1, n, False, None)[0]
+                with _nvtx('ttk:filters_pack'):
+                    keypoints = ops.filter_table(table_kp, table_kp_aux)
+            else:
+                keypoints = _upload_tables(known, self.device)
+        return self._tail(ball_positions, ball_positions_aux, keypoints, fps, stamps=None if stamps is None else stamps[1:n - 1])
 
-    def _tail(self, ball_positions, ball_positions_aux, table_keypoints, table_keypoints_aux, fps, uplifting_model=None, cameras=False,
-              stamps=None):
-        """predict's steps after the four detectors, shared with LiveSession.end_rally: the ball filter, the table filters, the
-        trajectory packing, the uplifting transformer and the spin rotation.  Takes the (n - 2, 3) ball and (n, K, 3) table positions
-        of one clip on the device; returns predict's (spin, pos3d).  uplifting_model: a replica of self.uplifting_model to run instead
-        (on the positions' device).  cameras: return (spin, pos3d, RallyCamera) instead.  stamps: the (n - 2,) float64 host stamps of
-        the clip's centre frames (timestamps[1:n - 1]), used instead of fps."""
+    def _tail(self, ball_positions, ball_positions_aux, keypoints, fps, uplifting_model=None, cameras=False, stamps=None):
+        """predict's steps after the detectors and the table filter, shared with LiveSession.end_rally: the ball filter, the
+        trajectory packing, the uplifting transformer and the spin rotation.  Takes the (n - 2, 3) ball positions and the (13, 3)
+        float64 table keypoints (filtered, or known) of one clip on the device; returns predict's (spin, pos3d).  uplifting_model: a
+        replica of self.uplifting_model to run instead (on the positions' device).  cameras: return (spin, pos3d, RallyCamera)
+        instead.  stamps: the (n - 2,) float64 host stamps of the clip's centre frames (timestamps[1:n - 1]), used instead of fps."""
         up = self.uplifting_model if uplifting_model is None else uplifting_model
         if stamps is None:
             ball_xy, _, times_ball, offsets = ops.filter_ball(ball_positions, ball_positions_aux, float(fps))
@@ -846,15 +896,14 @@ class TableTennisPipeline:
             ball_xy, _, times_ball, offsets = ops.filter_ball_timed(ball_positions, ball_positions_aux,
                                                                     _upload_stamps(stamps, ball_positions.device))
         with _nvtx('ttk:filters_pack'):
-            filtered_table_keypoints = ops.filter_table(table_keypoints, table_keypoints_aux)
-            ball_coords, table_coords, times, mask = ops.trajectory_pack(ball_xy, times_ball, offsets, filtered_table_keypoints[None],
+            ball_coords, table_coords, times, mask = ops.trajectory_pack(ball_xy, times_ball, offsets, keypoints[None],
                                                                         SEQ_LEN, WIDTH, HEIGHT)
         with _nvtx('ttk:uplift'):
             spin, pos3d = up.predict_without_normalization(ball_coords, table_coords, mask, times)
         if not cameras:
             return spin, pos3d
         with _nvtx('ttk:cameras'):
-            return spin, pos3d, _rally_cameras(filtered_table_keypoints[None], ball_xy[:len(pos3d)], [len(pos3d)], [pos3d])[0]
+            return spin, pos3d, _rally_cameras(keypoints[None], ball_xy[:len(pos3d)], [len(pos3d)], [pos3d])[0]
 
     def live(self, fps, streams=1, k=None, slots=None, devices=None):
         """A LiveSession (upliftingtabletennis_b200/live.py) over `streams` cameras at `fps`: frames are pushed as they arrive, the
@@ -867,7 +916,7 @@ class TableTennisPipeline:
         from .live import LiveSession
         return LiveSession(self, fps, streams, k, slots, devices)
 
-    def predict_clips(self, clips, fps, devices=None, cameras=False, timestamps=None):
+    def predict_clips(self, clips, fps, devices=None, cameras=False, timestamps=None, table_keypoints=None):
         """Many rallies in one call: returns [(spin, pos3d), ...], exactly [self.predict(c, fps) for c in clips] (same types, spin on
         the same device, same values bit for bit).  clips: list of clips, each a list of HWC uint8 BGR frames like predict takes, all
         of one frame size.
@@ -888,7 +937,11 @@ class TableTennisPipeline:
         the device and stream of the uplift.  cameras=False launches and synchronises nothing of this.
         timestamps: with fps=None, a list parallel to clips holding each clip's frame capture times as predict takes them; the results
         are then [self.predict(c, None, timestamps=t) for c, t in zip(clips, timestamps)] bit for bit.  A wrong number of stamps, a
-        non-finite or a non-increasing one raises ValueError naming the clip, before any device work."""
+        non-finite or a non-increasing one raises ValueError naming the clip, before any device work.
+        table_keypoints: a list parallel to clips, each entry a known table as predict takes it, or None to detect that clip's table.
+        The table detectors then run over the clips whose entry is None only; each result is predict(c, fps, table_keypoints=k) bit
+        for bit (with devices, cameras and timestamps too), and with cameras=True its camera holds k.  A bad entry raises ValueError
+        naming the clip, before any device work."""
         check_time_source(fps, timestamps)
         clips = [list(c) for c in clips]
         for i, c in enumerate(clips):
@@ -900,11 +953,25 @@ class TableTennisPipeline:
             if len(timestamps) != len(clips):
                 raise ValueError('timestamps: %d entries for %d clips; give one list of stamps per clip' % (len(timestamps), len(clips)))
             times = [check_timestamps(t, len(c), 'clip %d' % i) for i, (c, t) in enumerate(zip(clips, timestamps))]
+        tables = None
+        if table_keypoints is not None:
+            table_keypoints = list(table_keypoints)
+            if len(table_keypoints) != len(clips):
+                raise ValueError('table_keypoints: %d entries for %d clips; give one (13, 3) array or None per clip'
+                                 % (len(table_keypoints), len(clips)))
+            tables = [None if k is None else check_table_keypoints(k, 'clip %d' % i) for i, k in enumerate(table_keypoints)]
+
+        def detect_block(parts, a, b):
+            t = times if timestamps is None else times[a:b]
+            if tables is None:
+                return self._detect_clips(parts, clips[a:b], t)
+            return self._detect_clips(parts, clips[a:b], t, tables[a:b])
+
         if devices is None:
             if not clips:
                 return []
             parts = self._parts()
-            packed, counts, kept = self._detect_clips(parts, clips, times)
+            packed, counts, kept = detect_block(parts, 0, len(clips))
             counts = counts.cpu().tolist()
             self._check_counts(counts, 0)
             spin, pos = self._uplift_clips(parts, packed, counts)
@@ -927,7 +994,7 @@ class TableTennisPipeline:
             a, b = blocks[r]
             if a == b:
                 return parts, None, [], None
-            packed, counts, kept = self._detect_clips(parts, clips[a:b], times if timestamps is None else times[a:b])
+            packed, counts, kept = detect_block(parts, a, b)
             return parts, packed, counts.cpu().tolist(), kept
 
         def uplift(r, parts, packed, counts, kept):
@@ -980,14 +1047,16 @@ class TableTennisPipeline:
         cache[slot] = (key, tuple(parts))
         return cache[slot][1]
 
-    def _detect_clips(self, parts, clips, times):
+    def _detect_clips(self, parts, clips, times, tables=None):
         """Detectors, both filters and the trajectory packing of `clips` on the current device, a block of clips at a time.  times: the
-        fps, or a list of each clip's (n,) float64 frame stamps (check_timestamps).
+        fps, or a list of each clip's (n,) float64 frame stamps (check_timestamps).  tables: None, or a list parallel to clips of
+        known (13, 3) float64 tables (check_table_keypoints) and None for the clips whose table is detected.
         Returns the packed uplift inputs (ball, table, times, mask) of all clips, the (n,) int32 CUDA agreeing-detection counts and,
-        per block, its filtered table keypoints (clips, 13, 3) and ball detections (rows of its clips in order, then unused capacity):
-        what _with_cameras reads."""
+        per block, its table keypoints (clips, 13, 3), filtered or known, and ball detections (rows of its clips in order, then unused
+        capacity): what _with_cameras reads."""
         ball, ball_aux, table, table_aux, _ = parts
         dev = torch.device('cuda', torch.cuda.current_device())
+        tables = [None] * len(clips) if tables is None else tables
         packed, counts, kept = [], [], []
         for a, b in clip_blocks([len(c) for c in clips], ball.segment):
             lengths = [len(c) for c in clips[a:b]]
@@ -996,8 +1065,10 @@ class TableTennisPipeline:
             if order != list(range(n)):
                 torch.cuda.current_stream().wait_event(ready[-1][1])
                 frames, ready = frames[torch.tensor(order, device=dev)], None
+            known = tables[a:b]
+            detect = [i for i, k in enumerate(known) if k is None]     # the block's clips whose table the table detectors find
             bfirst, boffs = clip_stack_plan(lengths, ball.frames_per_stack)
-            tfirst, toffs = clip_stack_plan(lengths, table.frames_per_stack)
+            tfirst, toffs = select_stacks(*clip_stack_plan(lengths, table.frames_per_stack), detect)
             stamps = ball_row_stamps(times[a:b]) if isinstance(times, list) else None
             plan, stamps_d = _upload_plan(bfirst + boffs + tfirst + toffs, stamps, dev)
             bfirst_d, boffs_d, tfirst_d, toffs_d = plan.split([len(bfirst), len(boffs), len(tfirst), len(toffs)])
@@ -1008,10 +1079,25 @@ class TableTennisPipeline:
                     ball_xy, _, times_ball, offsets = ops.filter_ball_clips(bpos, bpos_aux, boffs_d, float(times))
                 else:
                     ball_xy, _, times_ball, offsets = ops.filter_ball_clips_timed(bpos, bpos_aux, boffs_d, stamps_d)
-                tpos = table._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
-                tpos_aux = table_aux._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
+                if detect:
+                    tpos = table._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
+                    tpos_aux = table_aux._run(frames, 1, len(tfirst), False, None, first=(tfirst, tfirst_d))[0]
             with _nvtx('ttk:filters_pack'):
-                tab = ops.filter_table_clips(tpos, tpos_aux, toffs_d)
+                tab = ops.filter_table_clips(tpos, tpos_aux, toffs_d) if detect else None
+                if len(detect) < len(known):
+                    given = _upload_tables([k for k in known if k is not None], dev)
+                    if tab is None:
+                        tab = given
+                    else:           # the block's rows in clip order, from the filtered and the known tables
+                        rows, d, g = [], 0, 0
+                        for k in known:
+                            if k is None:
+                                rows.append(tab[d:d + 1])
+                                d += 1
+                            else:
+                                rows.append(given[g:g + 1])
+                                g += 1
+                        tab = torch.cat(rows)
                 packed.append(ops.trajectory_pack(ball_xy, times_ball, offsets, tab, SEQ_LEN, WIDTH, HEIGHT))
                 counts.append(offsets[1:] - offsets[:-1])
             kept.append((tab, ball_xy))

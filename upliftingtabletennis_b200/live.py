@@ -20,8 +20,8 @@ from concurrent.futures import ThreadPoolExecutor
 import numpy as np
 import torch
 
-from . import _lib, sharding
-from .interface import _Detector, _fingerprint, check_timestamps, parse_devices
+from . import _lib, ops, sharding
+from .interface import _Detector, _fingerprint, _upload_tables, check_table_keypoints, check_timestamps, parse_devices
 
 DEFAULT_K = 16          # ready stacks that launch a pass: _Detector.chunk, predict's pass size; 137-143 frames/s for k = 4..32 on
                         # WASB + HRNet (profiles/r06_live_timing.json), so no reason to give ViTPose's GEMMs fewer M tiles
@@ -134,6 +134,12 @@ class LiveSession:
     reset with the rally.  A wrong number of stamps, a bad stamp, stamps pushed to a session with fps or none to a timestamped session
     raise ValueError before the push does anything.
 
+    set_table(stream, keypoints) gives a stream whose camera does not move its table, a (13, 3) array as predict's table_keypoints
+    takes it (typically the RallyCamera.keypoints of an earlier rally's end_rally(stream, cameras=True)), or clears it with None.  It
+    applies from the stream's next rally until it is changed, and raises ValueError while the stream has an open rally.  While it is
+    set, the stream's pushes queue no table stacks (the table passes run over the other streams only) and end_rally returns exactly
+    pipe.predict(the rally's frames, fps, table_keypoints=keypoints), with the stamps in a timestamped session.
+
     devices: None = one entry on the current device; push launches the passes on the caller's thread.  Otherwise a list of CUDA device
     indices, torch.device or 'cuda:N' strings, as predict_clips takes (a device may repeat): one entry per item, entry r serving
     streams sharding.shard_range(streams, r, len(devices)) -- contiguous blocks, the first streams % len(devices) entries one stream
@@ -182,6 +188,7 @@ class LiveSession:
         self._models = [None] * self.streams                # per open rally: (full fingerprint, weight tensors, quick key)
         # fps=None: each stream's open rally's frame stamps, on the host (a wrap copies frames, not stamps)
         self._stamps = [[] for _ in range(self.streams)] if fps is None else None
+        self._tables = [None] * self.streams                # set_table: each stream's known (13, 3) float64 table, or None
         self._stale = set()                                 # streams whose open rally was detected with replicas since rebuilt
         self._closed = False
 
@@ -223,10 +230,24 @@ class LiveSession:
             self._launch(e, {s})
             finish = self._finish
             if self._stamps is not None:
-                finish = functools.partial(self._finish, stamps=np.array(self._stamps[s], dtype=np.float64))
+                finish = functools.partial(finish, stamps=np.array(self._stamps[s], dtype=np.float64))
+            if self._tables[s] is not None:
+                finish = functools.partial(finish, table=self._tables[s])
             return self._run(e, finish, *((s, n, True) if cameras else (s, n)), wait=True)
         finally:
             self._reset(s)
+
+    def set_table(self, stream, keypoints):
+        """The known table of `stream` from its next rally on, a (13, 3) (x, y, v) array as predict's table_keypoints takes it, or None
+        to detect the table again.  While it is set, the stream's frames go to the ball detectors only and end_rally returns
+        predict(the rally's frames, fps, table_keypoints=keypoints).  Raises ValueError while the stream has an open rally, and for
+        keypoints predict would refuse."""
+        s = self._stream(stream)
+        kp = None if keypoints is None else check_table_keypoints(keypoints, 'stream %d' % s)
+        if self._n[s]:
+            raise ValueError('stream %d: set_table with a rally of %d frames open; a table applies from the next rally, call it after '
+                             'end_rally' % (s, self._n[s]))
+        self._tables[s] = kp
 
     def close(self):
         if self._closed:
@@ -354,7 +375,7 @@ class LiveSession:
             self._hand_off(e, frames[a:b], base + slot)
         n0 = self._n[s]
         self._n[s], self._w[s] = n0 + b - a, slot + b - a
-        for fps in (BALL, TABLE):
+        for fps in (BALL, TABLE) if self._tables[s] is None else (BALL,):         # a known table needs no table stacks
             e.pending[fps] += [(s, j, base + f) for j, f in ready_stacks(n0, self._n[s], self._w[s], fps)]
 
     def _wrap(self, s, src, dst, m):
@@ -520,12 +541,14 @@ class LiveSession:
         if e.copy is not None:
             torch.cuda.synchronize()
 
-    def _finish(self, s, n, cameras=False, stamps=None):
-        """stamps: the rally's n frame stamps (fps=None)."""
+    def _finish(self, s, n, cameras=False, stamps=None, table=None):
+        """stamps: the rally's n frame stamps (fps=None).  table: the stream's known (13, 3) float64 table, copied to the entry's
+        device, or None: the table filter over the rally's table positions."""
         e = self._entry[s]
         b, b_aux, t, t_aux = e.pos[s]
         centre = None if stamps is None else stamps[1:n - 1]
+        keypoints = ops.filter_table(t[:n], t_aux[:n]) if table is None else _upload_tables(table, b.device)
         if e.launcher is None:
-            return self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, cameras=cameras, stamps=centre)
-        out = self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], t[:n], t_aux[:n], self.fps, e.parts[4], cameras=cameras, stamps=centre)
+            return self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], keypoints, self.fps, cameras=cameras, stamps=centre)
+        out = self.pipe._tail(b[:n - 2, 0], b_aux[:n - 2, 0], keypoints, self.fps, e.parts[4], cameras=cameras, stamps=centre)
         return (out[0].to(self.pipe._home_device()),) + out[1:]
